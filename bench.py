@@ -2,6 +2,7 @@
 """Headline benchmark: batched MARBLER env-steps/s on N B200s of one node (BASELINE.json `metric`).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scenario S] [--envs B]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one env step of every env of the batch (BASELINE.json configs[1]: PredatorCapturePrey-v0,
@@ -16,6 +17,10 @@ D2H obs/reward/done/message), wall clock with a synchronize on both sides.
 `--impl reference` times the CPU path: the C restatement of the reference (oracle/, kind "port" - the
 reference itself is Python that needs rps/cvxopt/gym, none of which exist on the GPU box) on all host
 threads.  The oracle is only ever the checker / the CPU baseline here, never the product path.
+`--dump-outputs DIR` writes what the last timed step returned to its caller (obs, reward, done, message; rank 0's
+shard) as DIR/<name>.npy in float32, so that two builds run with the same arguments can be compared output for
+output: reset seeds and actions are fixed, so the inputs are the same from run to run.  DIR/env_index.npy names the
+env of every row; above 64 MB in all, a fixed, seeded sample of envs is written instead of every env.
 """
 import argparse
 import json
@@ -45,7 +50,14 @@ def parse():
     ap.add_argument("--no-numa-bind", action="store_true", help="do not bind the process to the CPUs next to its GPU")
     ap.add_argument("--rollout", action="store_true",
                     help="also time the closed loop policy kernel -> step kernel (SURVEY 8f-1), random-init GRU agent")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm times a host-dependent sample of envs)")
+    return args
 
 
 def load_cfg(args):
@@ -249,6 +261,26 @@ def pcie_floor(env, world, barrier, reps=10):
                    "%d times back to back, all ranks at once; max over ranks" % reps}
 
 
+DUMP_LIMIT_BYTES = 64 * 1000 * 1000
+
+
+def dump_outputs(out_dir, outputs):
+    """outputs: name -> CUDA tensor with a leading env axis.  Writes each as out_dir/<name>.npy in float32 (done and
+    message are small integers, exact there) plus env_index.npy, the env of every row.  When everything would exceed
+    DUMP_LIMIT_BYTES, every array keeps the same fixed, seeded sample of envs."""
+    import numpy as np
+    B = next(iter(outputs.values())).shape[0]
+    per_env = 8 + sum(4 * t[0].numel() for t in outputs.values())      # 8: the float64 env index
+    budget = DUMP_LIMIT_BYTES - 4096                                      # .npy headers
+    index = np.arange(B)
+    if B * per_env > budget:
+        index = np.sort(np.random.RandomState(0).choice(B, budget // per_env, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy()[index].astype(np.float32))
+    np.save(os.path.join(out_dir, "env_index.npy"), index.astype(np.float64))
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -308,6 +340,8 @@ def run_ours(args):
         torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
     dev_ms_max = float(t.item())
     stats = sharding.summarize(sharding.allreduce_stats(env.stats))
+    if args.dump_outputs and rank == 0:                 # before the e2e leg below steps the env again
+        dump_outputs(args.dump_outputs, {"obs": env.obs, "reward": env.reward, "done": env.done, "message": env.message})
 
     # ---- end to end through the host API: pinned numpy actions -> H2D -> step -> D2H -> sync
     Ke = max(3, min(K, 50))

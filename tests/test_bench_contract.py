@@ -24,6 +24,38 @@ def test_reference_arm_prints_one_json_line():
     assert d["gpu_launches"] == 0 and d["vs_baseline"] is None and d["dtype"] == "f64" and d["data"] == "synthetic"
 
 
+def test_dump_outputs_is_float_and_a_fixed_sample_under_64_mb(tmp_path):
+    """bench.dump_outputs on a Warehouse-sized step (262,144 envs x 6 robots x 18 obs: 113 MB of obs alone): every
+    file float32 / float64, 64 MB at most in all, the same envs from run to run, rows taken from the envs named."""
+    import numpy as np
+    import torch
+    import bench
+    B, N, D = 262144, 6, 18
+    g = torch.Generator().manual_seed(0)
+    outputs = {"obs": torch.rand((B, N, D), generator=g), "reward": torch.rand((B, N), generator=g),
+               "done": torch.randint(0, 2, (B,), generator=g, dtype=torch.uint8),
+               "message": torch.randint(0, 4, (B,), generator=g, dtype=torch.uint8)}
+    runs = [tmp_path / "a", tmp_path / "b"]
+    for d in runs:
+        bench.dump_outputs(str(d), outputs)
+    files = sorted(os.listdir(runs[0]))
+    assert files == ["done.npy", "env_index.npy", "message.npy", "obs.npy", "reward.npy"]
+    assert sum(os.path.getsize(runs[0] / f) for f in files) <= bench.DUMP_LIMIT_BYTES
+    for f in files:
+        a, b = np.load(runs[0] / f), np.load(runs[1] / f)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b), f
+    index = np.load(runs[0] / "env_index.npy").astype(np.int64)
+    assert B // 2 < len(index) < B and (np.diff(index) > 0).all()
+    for name, t in outputs.items():
+        assert np.array_equal(np.load(runs[0] / (name + ".npy")), t.numpy()[index].astype(np.float32)), name
+
+
+def test_steps_below_one_are_refused():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True,
+                         text=True, timeout=120, cwd=ROOT)
+    assert out.returncode == 2 and "--steps" in out.stderr
+
+
 def test_reference_arm_other_ranks_exit_quietly():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2",

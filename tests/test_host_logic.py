@@ -118,16 +118,15 @@ def test_registry_keys_and_space_dims():
 
 
 def test_default_configs_equal_reference_yaml():
-    ref_root = "/root/reference/robotarium_gym/scenarios"
-    if not os.path.isdir(ref_root):
-        pytest.skip("reference tree not present on this machine")
-    import yaml
+    """Against the config each scenario's rollout fixture was made with: the reference's own config.yaml with the
+    overrides of oracle/ref_harness.py reference_config() (figures, gif, logging, real time and robotarium off) and a
+    seed of the fixture's own (oracle/gen_golden.py), so the seed is not compared."""
     from marbler_b200 import config
     for scn in config.SCENARIOS:
-        ref = yaml.safe_load(open(os.path.join(ref_root, scn, "config.yaml")))
+        ref = gu.Golden(scn + "_rollout").cfg
         mine = config.load_yaml(config.default_config_path(scn))
         for k, v in mine.items():
-            if k in ("show_figure_frequency", "save_gif", "real_time"):
+            if k in ("show_figure_frequency", "save_gif", "real_time", "seed"):
                 continue
             assert ref[k] == v, (scn, k)
 
