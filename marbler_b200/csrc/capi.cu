@@ -290,8 +290,7 @@ extern "C" int mrb_step_host(mrb_env *env, const int32_t *actions_host, float *o
     }
     // chunk size: multiple of 64 envs keeps every chunk's actions 16-byte aligned; >= 16,384 envs per chunk
     int64_t nchunks = B / 16384;          // measured on B200 / PCIe 5: 65,536 PCP envs 0.61 / 0.53 / 0.53 / 0.58 / 0.68 ms at 1 / 2 / 4 / 8 / 16 chunks (direct issue)
-    if (const char *ov = std::getenv("MRB_HOST_CHUNKS")) nchunks = std::atoi(ov);     // tuning knob
-    if (nchunks > 8 && !std::getenv("MRB_HOST_CHUNKS")) nchunks = 8;
+    if (nchunks > 8) nchunks = 8;
     nchunks = nchunks < 1 ? 1 : (nchunks > kPipeStreams ? kPipeStreams : nchunks);
     int64_t chunk = (B + nchunks - 1) / nchunks;
     chunk = (chunk + 63) / 64 * 64;

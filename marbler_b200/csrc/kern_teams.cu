@@ -6,8 +6,6 @@
 // 20: 29.0 vs 13.7; 16,384 envs: 24 robots 31.6 vs 12.5, 28: 56.6 vs 16.5; padded: 10 robots (on 12) 3.90 vs 2.97,
 // 18 (on 20) 12.6 vs 7.2, 23 (on 24) 22.3 vs 13.4; 20 robots padded variant 14.5 vs 13.7 folded.
 // Kernels exist for PredatorCapturePrey 8..32, Warehouse 8 and 12, Simple 8..16 (what their spawn grids hold).
-#include <cstdlib>
-
 #include "launchers.h"
 
 namespace mrb {
@@ -33,9 +31,8 @@ cudaError_t launch_qp_team_n_32(int N, int barrier_default, int64_t B, const dou
 
 cudaError_t launch_step_team(int scenario, const Params &p, const int32_t *actions, cudaStream_t s, bool *handled)
 {
-    static const bool padded_only = std::getenv("MRB_TEAM_PADDED") != nullptr;      // measurement aid: never the folded variant
     const int N = p.cfg.num_robots, size = (N + 3) & ~3;
-    const bool exact = size == N && !padded_only;
+    const bool exact = size == N;
     *handled = true;
     if (scenario == MRB_PCP) switch (size) {
     case 8: return launch_step_team_pcp_8(p, actions, s, exact);

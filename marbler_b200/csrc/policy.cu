@@ -74,11 +74,9 @@ __device__ __forceinline__ float rcp_(float x) { float y; asm("rcp.approx.ftz.f3
 __device__ __forceinline__ float sigmoidf_(float x) { return rcp_(1.f + ex2_(-1.4426950408889634f * x)); }
 __device__ __forceinline__ float tanhf_(float x) { return fmaf(2.f, rcp_(1.f + ex2_(-2.8853900817779268f * x)), -1.f); }
 
-#ifndef MRB_POLICY_MIN_BLOCKS
-#define MRB_POLICY_MIN_BLOCKS 4      // 128 registers, 16 warps per SM: measured 0.327 ms vs 0.344 (3) and 0.427 (2) for 262,144 agents
-#endif
+constexpr int kPolicyMinBlocks = 4;      // 128 registers, 16 warps per SM: measured 0.327 ms vs 0.344 (3) and 0.427 (2) for 262,144 agents
 template <int H, bool RNN>
-__global__ void __launch_bounds__(kPolicyWarps * 32, MRB_POLICY_MIN_BLOCKS)
+__global__ void __launch_bounds__(kPolicyWarps * 32, kPolicyMinBlocks)
 policy_act_kernel(const PolicyParams p, const float *obs, float *hidden, int32_t *__restrict__ actions,
                   float *__restrict__ q_out, const uint8_t *__restrict__ fresh)
 {
@@ -614,14 +612,3 @@ extern "C" int mrb_policy_act(mrb_policy *pol, int64_t num_envs, const float *ob
     count_launch();
     return MRB_OK;
 }
-
-#ifdef MRB_TC2_TRACE
-extern "C" int mrb_debug_tc2_trace(unsigned long long *out)
-{
-    return (int)cudaMemcpyFromSymbol(out, mrb::tc2::g_tc2_trace, sizeof(unsigned long long) * 256);
-}
-extern "C" int mrb_debug_tc2_trace2(unsigned long long *out)
-{
-    return (int)cudaMemcpyFromSymbol(out, mrb::tc2::g_tc2_trace2, sizeof(unsigned long long) * 256);
-}
-#endif

@@ -36,10 +36,7 @@ constexpr int kHalf = 64;                                  // hidden units per p
 constexpr int kHalfSlabBytes = kHalf * kH * 2;             // 16 KB
 constexpr int kSlabsPerTile = 12;                          // 2 passes x (W_ir, W_hr, W_iz, W_hz, W_in, W_hn)
 constexpr int kRingMax = 3;                               // weight-ring slots: 3 when they fit, else 2 (Params2::ring)
-#ifndef MRB_TC2_EPI_WARPS
-#define MRB_TC2_EPI_WARPS 8
-#endif
-constexpr int kStageWarps = 8, kEpiWarps = MRB_TC2_EPI_WARPS;    // kEpiWarps / 4 epilogue warps share a TMEM lane quarter
+constexpr int kStageWarps = 8, kEpiWarps = 8;             // kEpiWarps / 4 epilogue warps share a TMEM lane quarter
 constexpr int kColGroups = kEpiWarps / 4;                  // ... and split the 64 units of a pass between them
 constexpr int kUnitsPerWarp = kHalf / kColGroups;
 constexpr int kTileStride = 20;                            // floats per row of an epilogue exchange tile (16 + 4 pad)
@@ -50,11 +47,8 @@ constexpr int kTileStride = 20;                            // floats per row of 
 // epilogue warps rise to 128 (8 x 4096 + 4 x 1280 + 8 x 2816 = 60,416).
 constexpr int kMmaWarp = kEpiWarps, kLoadWarp = kEpiWarps + 1, kStageBase = kEpiWarps + 4;
 constexpr int kThreads2 = (kStageBase + kStageWarps) * 32;        // 640
-#ifndef MRB_TC2_SETMAXNREG
-#define MRB_TC2_SETMAXNREG 1
-#endif
-template <int R> __device__ __forceinline__ void reg_inc() { if (MRB_TC2_SETMAXNREG) asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(R)); }
-template <int R> __device__ __forceinline__ void reg_dec() { if (MRB_TC2_SETMAXNREG) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(R)); }
+template <int R> __device__ __forceinline__ void reg_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(R)); }
+template <int R> __device__ __forceinline__ void reg_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(R)); }
 constexpr int kMaxA = 8;                                  // fc2 runs on the CUDA cores of the epilogue warps
 
 struct Params2 {
@@ -132,31 +126,6 @@ __device__ __forceinline__ void mbar_wait_sleep(uint32_t bar, uint32_t parity)
         if (++spins > (1u << 20)) __trap();               // never hang the device on a protocol bug
     }
 }
-#ifdef MRB_TC2_TRACE
-__device__ unsigned long long g_tc2_trace[16][16];
-__device__ __forceinline__ void trace(int tile, int slot)
-{
-    if (blockIdx.x == 0 && tile < 16) {
-        unsigned long long t;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-        g_tc2_trace[tile][slot] = t;
-    }
-}
-#define TC2_TRACE(tile, slot) trace(tile, slot)
-__device__ unsigned long long g_tc2_trace2[16][16];
-__device__ __forceinline__ void trace2(int tile, int slot)
-{
-    if (blockIdx.x == 0 && tile < 16 && threadIdx.x == 0) {
-        unsigned long long t;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-        g_tc2_trace2[tile][slot] = t;
-    }
-}
-#define TC2_TRACE2(tile, slot) trace2(tile, slot)
-#else
-#define TC2_TRACE(tile, slot)
-#define TC2_TRACE2(tile, slot)
-#endif
 __device__ __forceinline__ void prefetch_l1(const void *ptr) { asm volatile("prefetch.global.L1 [%0];" ::"l"(ptr)); }
 __device__ __forceinline__ float round_f16(float v) { return __half2float(__float2half_rn(v)); }
 
@@ -254,14 +223,11 @@ policy_act_tc2_kernel(const Params2 p, const float *__restrict__ obs, float *hid
 #pragma unroll
                         for (int i = 0; i < 4; i++) ov[i] = *reinterpret_cast<const float4 *>(hidden + trow[i] * kH + ubn + 4 * tc4);
                     }
-                    if (gi == 0) TC2_TRACE2(n, 0);
                     if (G == 0) {
                         mbar_wait_sleep(tmem_full + 8 * pass, (uint32_t)(n & 1));
                         tc_fence_after();
-                        if (tid == 0) TC2_TRACE(n, 1 + 2 * pass);
                     }
                     __syncwarp();
-                    if (gi == 0) TC2_TRACE2(n, 1);
                     const uint32_t tb = lane_base + 256 * pass + kUnitsPerWarp * cq + 16 * G;
 #pragma unroll 1
                     for (int c = 0; c < 2; c++) {
@@ -275,7 +241,6 @@ policy_act_tc2_kernel(const Params2 p, const float *__restrict__ obs, float *hid
                         const float4 o0 = *reinterpret_cast<const float4 *>(mine), o1 = *reinterpret_cast<const float4 *>(mine + 4);
                         const float old[8] = {o0.x, o0.y, o0.z, o0.w, o1.x, o1.y, o1.z, o1.w};
                         tmem_ld_wait();
-                        if (gi == 0) TC2_TRACE2(n, 2 + 3 * c);
                         float hn[8];
 #pragma unroll
                         for (int i = 0; i < 8; i++) {
@@ -285,7 +250,6 @@ policy_act_tc2_kernel(const Params2 p, const float *__restrict__ obs, float *hid
                             const float nn = tanh_(ai[i] + b_ih[2 * kH + k] + r * (ah[i] + b_hh[2 * kH + k]));
                             hn[i] = (1.f - z) * nn + z * old[i];
                         }
-                        if (gi == 0) TC2_TRACE2(n, 3 + 3 * c);
                         *reinterpret_cast<float4 *>(mine) = make_float4(hn[0], hn[1], hn[2], hn[3]);
                         *reinterpret_cast<float4 *>(mine + 4) = make_float4(hn[4], hn[5], hn[6], hn[7]);
                         // fc2 partial sums (rnn_agent.py:28) with FP16-rounded operands, like the tensor-core kernels
@@ -302,11 +266,9 @@ policy_act_tc2_kernel(const Params2 p, const float *__restrict__ obs, float *hid
                                 qacc[a] = s;
                             }
                         }
-                        if (gi == 0) TC2_TRACE2(n, 4 + 3 * c);
                     }
                     if (G == kUnitsPerWarp / 16 - 1) {
                         tc_fence_before();
-                        if (tid == 0) TC2_TRACE(n, 2 + 2 * pass);
                         mbar_arrive(tmem_free + 8 * pass);  // this half may be overwritten by the next tile's pass
                     }
                     __syncwarp();
@@ -316,7 +278,6 @@ policy_act_tc2_kernel(const Params2 p, const float *__restrict__ obs, float *hid
                         if (tvalid[i])
                             *reinterpret_cast<float4 *>(hidden + trow[i] * kH + ub + 4 * tc4) =
                                 *reinterpret_cast<const float4 *>(tile + (8 * i + tr) * kTileStride + 4 * tc4);
-                    if (gi == 0) TC2_TRACE2(n, 8);
                 }
             }
             // the warps of a row add their parts of fc2 (fixed order), the first one picks the action; the partial sums
@@ -356,12 +317,10 @@ policy_act_tc2_kernel(const Params2 p, const float *__restrict__ obs, float *hid
                 const int b = n & 1;
                 mbar_wait(act_full + 8 * b, (uint32_t)((n >> 1) & 1));
                 tc_fence_after();
-                TC2_TRACE(n, 5);
                 const uint32_t xa = sbase + Smem2::act + b * Smem2::act_stride, ha = xa + kActBytes;
                 for (int pass = 0; pass < 2; pass++) {
                     mbar_wait(tmem_free + 8 * pass, (uint32_t)((n & 1) ^ 1));
                     tc_fence_after();
-                    TC2_TRACE(n, 6 + 2 * pass);
                     for (int g = 0; g < 6; g++, q++) {
                         const uint32_t slot = q % ring;
                         mbar_wait(slab_full + 8 * slot, (q / ring) & 1);
@@ -377,7 +336,6 @@ policy_act_tc2_kernel(const Params2 p, const float *__restrict__ obs, float *hid
                         tc_commit(slab_empty + 8 * slot);
                     }
                     tc_commit(tmem_full + 8 * pass);
-                    TC2_TRACE(n, 7 + 2 * pass);
                 }
                 tc_commit(act_free + 8 * b);                // both passes have read x and h of this buffer
             }
@@ -420,7 +378,6 @@ policy_act_tc2_kernel(const Params2 p, const float *__restrict__ obs, float *hid
             const bool valid = e < p.B;
             const int my_zero = (!valid || (fresh && fresh[e])) ? 1 : 0;
             const int64_t my_grow = (valid ? e : 0) * N + agent;
-            if (sw == 0 && lane == 0) TC2_TRACE(n, 10);
             // hidden state: one coalesced 512-byte row per load instruction, packed to FP16 as it arrives (this lane
             // keeps k = 4 lane .. 4 lane + 3 of each of the 16 rows)
             uint2 hp[16];
@@ -465,9 +422,7 @@ policy_act_tc2_kernel(const Params2 p, const float *__restrict__ obs, float *hid
                     af[ks][2] = *reinterpret_cast<const uint32_t *>(scr + g * KS + 16 * ks + 2 * tq + 8);
                     af[ks][3] = *reinterpret_cast<const uint32_t *>(scr + (g + 8) * KS + 16 * ks + 2 * tq + 8);
                 }
-            if (sw == 0 && lane == 0) TC2_TRACE(n, 11);
             mbar_wait_sleep(act_free + 8 * b, (uint32_t)(((n >> 1) & 1) ^ 1));
-            if (sw == 0 && lane == 0) TC2_TRACE(n, 12);
             uint8_t *xa = sm + Smem2::act + b * Smem2::act_stride, *ha = xa + kActBytes;
 #pragma unroll
             for (int r = 0; r < 16; r++) {
@@ -492,7 +447,6 @@ policy_act_tc2_kernel(const Params2 p, const float *__restrict__ obs, float *hid
                 *reinterpret_cast<uint32_t *>(xa + nt * kActLBO + r_hi) = h2(fmaxf(c[2], 0.f), fmaxf(c[3], 0.f));
             }
             fence_async_smem();                             // generic-proxy stores -> visible to the tensor core's async proxy
-            if (sw == 0 && lane == 0) TC2_TRACE(n, 13);
             mbar_arrive(act_full + 8 * b);
         }
     }

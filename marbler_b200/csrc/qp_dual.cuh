@@ -9,37 +9,21 @@
 // registers.  G G' is never stored: entry (c,d) is +-(a_c . a_d) when the two pairs share a robot.
 #pragma once
 #include "common.cuh"
-#include "qp_store.cuh"
 
 namespace mrb {
 
-// per-env vectors of the dual solver that may live in the shared store (bit i of VMASK <-> DualVec i); lengths m or n
-enum DualVec { DV_H = 0, DV_RZ, DV_T2, DV_Q, DV_RX, DV_CORR, DV_P, DV_D, DV_S, DV_Z, DV_AX, DV_AY, DV_X, DV_COUNT };
-
-// LS: 1 = the strictly-lower part of the m x m Cholesky factor lives in the shared store as well (the reciprocals
-// of its diagonal stay in registers).  TPB: threads per CTA (the interleave stride of the store).
-template <int N, int TPB = 1, unsigned VMASK = 0, int LS = 0>
+// Every vector of the solver, the factor included, is a register array: moving some of them to a shared-memory store
+// was measured slower for these team sizes (DESIGN.md section 4).
+template <int N>
 struct QpDual {
     static constexpr int n = 2 * N;
     static constexpr int m = N * (N - 1) / 2;
     static constexpr int MT = m * (m - 1) / 2;                 // strictly-lower entries
     __device__ static constexpr int low(int r, int c) { return r * (r - 1) / 2 + c; }   // r > c
 
-    __device__ static constexpr bool in_smem(int id) { return (VMASK >> id) & 1u; }
-    __device__ static constexpr int len(int id) { return (id == DV_Q || id == DV_RX || id == DV_X) ? n : m; }
-    __device__ static constexpr int offset(int id) { int k = 0; for (int b = 0; b < id; b++) k += in_smem(b) ? len(b) : 0; return k; }
-    static constexpr int kVecDoubles = offset(DV_COUNT);
-    static constexpr int kStoreDoubles = kVecDoubles + (LS ? MT : 0);      // doubles per thread
-    template <int ID> using Vec = MVec<len(ID), TPB, in_smem(ID)>;
-
-    Vec<DV_AX> ax;
-    Vec<DV_AY> ay;
-    MVec<MT, TPB, LS != 0> L;
+    double ax[m], ay[m];
+    double L[MT];
     double invd[m];
-    double *Vs;
-
-    __device__ __forceinline__ QpDual(double *Vs_ = nullptr)
-        : ax(Vs_, offset(DV_AX)), ay(Vs_, offset(DV_AY)), L(Vs_, kVecDoubles), Vs(Vs_) {}
 
     // sink(c, (G v)_c)
     template <typename V, typename F>
@@ -50,7 +34,7 @@ struct QpDual {
         for (int i = 0; i < N - 1; i++)
 #pragma unroll
             for (int j = i + 1; j < N; j++, c++)
-                sink(c, ax.get(c) * (v(2 * j) - v(2 * i)) + ay.get(c) * (v(2 * j + 1) - v(2 * i + 1)));
+                sink(c, ax[c] * (v(2 * j) - v(2 * i)) + ay[c] * (v(2 * j + 1) - v(2 * i + 1)));
     }
     // out += G' y
     template <typename F>
@@ -62,7 +46,7 @@ struct QpDual {
 #pragma unroll
             for (int j = i + 1; j < N; j++, c++) {
                 const double yc = y(c);
-                const double tx = ax.get(c) * yc, ty = ay.get(c) * yc;
+                const double tx = ax[c] * yc, ty = ay[c] * yc;
                 out[2 * i] -= tx; out[2 * i + 1] -= ty;
                 out[2 * j] += tx; out[2 * j + 1] += ty;
             }
@@ -75,7 +59,7 @@ struct QpDual {
         constexpr int sgn = (ci == ei) + (cj == ej) - (ci == ej) - (cj == ei);
         if constexpr (sgn == 0) return 0.0;
         else {
-            const double dot = fma(ax.get(C), ax.get(E), ay.get(C) * ay.get(E));
+            const double dot = fma(ax[C], ax[E], ay[C] * ay[E]);
             return sgn > 0 ? 0.5 * dot : -0.5 * dot;
         }
     }
@@ -91,18 +75,18 @@ struct QpDual {
     {
         static_for<0, m>([&](auto K_) {
             constexpr int k = decltype(K_)::value;
-            const double a = ax.get(k), b = ay.get(k);
+            const double a = ax[k], b = ay[k];
             double dk = fma(a, a, b * b) + d(k);                                    // 1/2 |g_k|^2 = |a_k|^2
 #pragma unroll
-            for (int j = 0; j < k; j++) { const double l = L.get(low(k, j)); dk = fma(-l, l, dk); }
+            for (int j = 0; j < k; j++) { const double l = L[low(k, j)]; dk = fma(-l, l, dk); }
             const double r = fast_rsqrt(dk);
             invd[k] = r;
             static_for<k + 1, m>([&](auto I_) {
                 constexpr int i = decltype(I_)::value;
                 double v = gram<i, k>();
 #pragma unroll
-                for (int j = 0; j < k; j++) v = fma(-L.get(low(i, j)), L.get(low(k, j)), v);
-                L.set(low(i, k), v * r);
+                for (int j = 0; j < k; j++) v = fma(-L[low(i, j)], L[low(k, j)], v);
+                L[low(i, k)] = v * r;
             });
         });
     }
@@ -113,7 +97,7 @@ struct QpDual {
             constexpr int i = decltype(I)::value;
             double v = b[i];
 #pragma unroll
-            for (int k = 0; k < i; k++) v = fma(-L.get(low(i, k)), b[k], v);
+            for (int k = 0; k < i; k++) v = fma(-L[low(i, k)], b[k], v);
             b[i] = v * invd[i];
         });
         // backward sweep in row order: once x_i is known every earlier row receives -L_ik x_i
@@ -122,15 +106,14 @@ struct QpDual {
             const double xi = b[i] * invd[i];
             b[i] = xi;
 #pragma unroll
-            for (int k = 0; k < i; k++) b[k] = fma(-L.get(low(i, k)), xi, b[k]);
+            for (int k = 0; k < i; k++) b[k] = fma(-L[low(i, k)], xi, b[k]);
         });
     }
 
     __device__ __forceinline__ int run(const double (&xix)[N], const double (&xiy)[N], double (&ux)[N],
                                        double (&uy)[N], bool barrier_default)
     {
-        Vec<DV_Q> q(Vs, offset(DV_Q));
-        Vec<DV_X> x(Vs, offset(DV_X));
+        double q[n], x[n];
 #pragma unroll
         for (int i = 0; i < N; i++) {          // A.8: pre-clip columns of dxi to norm 0.2, f = -2 dxi
             const double n2 = ux[i] * ux[i] + uy[i] * uy[i];
@@ -138,18 +121,10 @@ struct QpDual {
                 const double sc = kQpMagnitudeLimit / sqrt(n2);
                 ux[i] *= sc; uy[i] *= sc;
             }
-            q.set(2 * i, -2.0 * ux[i]);
-            q.set(2 * i + 1, -2.0 * uy[i]);
+            q[2 * i] = -2.0 * ux[i];
+            q[2 * i + 1] = -2.0 * uy[i];
         }
-        Vec<DV_H> h(Vs, offset(DV_H));
-        Vec<DV_S> s(Vs, offset(DV_S));
-        Vec<DV_Z> z(Vs, offset(DV_Z));
-        Vec<DV_RZ> rz(Vs, offset(DV_RZ));
-        Vec<DV_RX> rxs(Vs, offset(DV_RX));
-        Vec<DV_T2> t2(Vs, offset(DV_T2));
-        Vec<DV_D> dd(Vs, offset(DV_D));
-        Vec<DV_CORR> corr(Vs, offset(DV_CORR));
-        Vec<DV_P> pp(Vs, offset(DV_P));
+        double h[m], s[m], z[m], rz[m], rxs[n], t2[m], dd[m], corr[m], pp[m];
 
         const double r2 = barrier_default ? 0.17 * 0.17 : 0.2 * 0.2;
         double hh = 0.0, qq = 0.0;
@@ -163,8 +138,8 @@ struct QpDual {
                     const double hv = (ex * ex + ey * ey) - r2;
                     const double gain = barrier_default ? 100.0 : (hv >= 0.0 ? 100.0 : 1e6);
                     const double hc = gain * (hv * hv * hv);
-                    h.set(c, hc);
-                    ax.set(c, 2.0 * ex); ay.set(c, 2.0 * ey);
+                    h[c] = hc;
+                    ax[c] = 2.0 * ex; ay[c] = 2.0 * ey;
                     hh = fma(hc, hc, hh);
                 }
         }
@@ -172,7 +147,7 @@ struct QpDual {
             double q0 = 0.0, q1 = 0.0;
 #pragma unroll
             for (int a = 0; a < n; a += 2) {
-                const double qa = q.get(a), qb = q.get(a + 1);
+                const double qa = q[a], qb = q[a + 1];
                 q0 = fma(qa, qa, q0); q1 = fma(qb, qb, q1);
             }
             qq = q0 + q1;
@@ -183,20 +158,20 @@ struct QpDual {
         // ---- default starting point [P G'; G -I][x; z] = [-q; h]:  (1/2 GG' + I) z = -h - 1/2 G q,  x = -1/2 (q + G'z)
         factor([](int) { return 1.0; });
         double tv[m];
-        G_mul([&](int a) { return q.get(a); }, [&](int c, double g) { tv[c] = -h.get(c) - 0.5 * g; });
+        G_mul([&](int a) { return q[a]; }, [&](int c, double g) { tv[c] = -h[c] - 0.5 * g; });
         solve(tv);
         {
             double xa[n];
 #pragma unroll
-            for (int a = 0; a < n; a++) xa[a] = q.get(a);
+            for (int a = 0; a < n; a++) xa[a] = q[a];
             GT_acc([&](int c) { return tv[c]; }, xa);
 #pragma unroll
-            for (int a = 0; a < n; a++) x.set(a, xa[a] * -0.5);
+            for (int a = 0; a < n; a++) x[a] = xa[a] * -0.5;
         }
         double ss = 0.0, ts = -INFINITY, tz = -INFINITY;
-        G_mul([&](int a) { return x.get(a); }, [&](int c, double g) {       // z = Gx - h as cvxopt forms it
-            const double zc = g - h.get(c);
-            z.set(c, zc);
+        G_mul([&](int a) { return x[a]; }, [&](int c, double g) {       // z = Gx - h as cvxopt forms it
+            const double zc = g - h[c];
+            z[c] = zc;
             ss = fma(zc, zc, ss);
             ts = dmax(zc, ts);
             tz = dmax(-zc, tz);
@@ -206,11 +181,11 @@ struct QpDual {
         double gap = 0.0;
 #pragma unroll
         for (int c = 0; c < m; c++) {
-            const double z0 = z.get(c);
+            const double z0 = z[c];
             double sc = -z0, zc = z0;
             if (do_s) sc += 1.0 + ts;
             if (do_z) zc += 1.0 + tz;
-            s.set(c, sc); z.set(c, zc);
+            s[c] = sc; z[c] = zc;
             gap = fma(sc, zc, gap);
         }
 
@@ -221,23 +196,23 @@ struct QpDual {
             double xq = 0.0, xrx = 0.0, xq1 = 0.0, xrx1 = 0.0;
 #pragma unroll
             for (int a = 0; a < n; a += 2) {
-                const double xa = x.get(a), qa = q.get(a), xb = x.get(a + 1), qb = q.get(a + 1);
+                const double xa = x[a], qa = q[a], xb = x[a + 1], qb = q[a + 1];
                 rx[a] = fma(2.0, xa, qa);
                 rx[a + 1] = fma(2.0, xb, qb);
                 xrx = fma(xa, rx[a], xrx); xrx1 = fma(xb, rx[a + 1], xrx1);
                 xq = fma(xa, qa, xq); xq1 = fma(xb, qb, xq1);
             }
             const double f0 = 0.5 * ((xrx + xrx1) + (xq + xq1));
-            GT_acc([&](int c) { return z.get(c); }, rx);
+            GT_acc([&](int c) { return z[c]; }, rx);
             double resx = 0.0, resx1 = 0.0, resz = 0.0, resz1 = 0.0, zrz = 0.0, zrz1 = 0.0;
 #pragma unroll
             for (int a = 0; a < n; a += 2) { resx = fma(rx[a], rx[a], resx); resx1 = fma(rx[a + 1], rx[a + 1], resx1); }
             resx += resx1;
-            G_mul([&](int a) { return x.get(a); }, [&](int c, double g) {
-                const double r = g + (s.get(c) - h.get(c));
-                rz.set(c, r);
-                if (c & 1) { resz1 = fma(r, r, resz1); zrz1 = fma(z.get(c), r, zrz1); }
-                else { resz = fma(r, r, resz); zrz = fma(z.get(c), r, zrz); }
+            G_mul([&](int a) { return x[a]; }, [&](int c, double g) {
+                const double r = g + (s[c] - h[c]);
+                rz[c] = r;
+                if (c & 1) { resz1 = fma(r, r, resz1); zrz1 = fma(z[c], r, zrz1); }
+                else { resz = fma(r, r, resz); zrz = fma(z[c], r, zrz); }
             });
             resz += resz1; zrz += zrz1;
             const double pcost = f0, dcost = f0 + zrz - gap;
@@ -249,30 +224,30 @@ struct QpDual {
             if ((resz <= feas_z2 && resx <= feas_x2 && gap_ok) || iters == 50) break;
 
             // 1/s and 1/z are recomputed where they are used (same function of the same input: identical bits)
-            auto inv_s = [&](int c) { return fast_rcp1(s.get(c)); };
-            auto inv_z = [&](int c) { return fast_rcp1(z.get(c)); };
+            auto inv_s = [&](int c) { return fast_rcp1(s[c]); };
+            auto inv_z = [&](int c) { return fast_rcp1(z[c]); };
 #pragma unroll
-            for (int c = 0; c < m; c++) dd.set(c, s.get(c) * inv_z(c));           // D = s/z
-            factor([&](int c) { return dd.get(c); });
+            for (int c = 0; c < m; c++) dd[c] = s[c] * inv_z(c);           // D = s/z
+            factor([&](int c) { return dd[c]; });
             // base right-hand side shared by predictor and corrector: rz - 1/2 G rx - s
-            G_mul([&](int a) { return rx[a]; }, [&](int c, double g) { t2.set(c, rz.get(c) - 0.5 * g - s.get(c)); });
+            G_mul([&](int a) { return rx[a]; }, [&](int c, double g) { t2[c] = rz[c] - 0.5 * g - s[c]; });
 #pragma unroll
-            for (int a = 0; a < n; a++) rxs.set(a, rx[a]);                          // rx is needed again after the solves
+            for (int a = 0; a < n; a++) rxs[a] = rx[a];                          // rx is needed again after the solves
             // predictor (rc = -s.z)
             double dz[m];
 #pragma unroll
-            for (int c = 0; c < m; c++) dz[c] = t2.get(c);
+            for (int c = 0; c < m; c++) dz[c] = t2[c];
             solve(dz);
             double dsdz = 0.0, dsdz1 = 0.0, tmax;
             double cand[m];
 #pragma unroll
             for (int c = 0; c < m; c++) {
-                const double sc = s.get(c);
-                const double dsc = -sc - dd.get(c) * dz[c];
+                const double sc = s[c];
+                const double dsc = -sc - dd[c] * dz[c];
                 const double p = dsc * dz[c];
                 if (c & 1) dsdz1 += p; else dsdz += p;
                 cand[c] = dmax(-dsc * inv_s(c), -dz[c] * inv_z(c));
-                pp.set(c, p);                                  // keep only the Mehrotra correction term
+                pp[c] = p;                                  // keep only the Mehrotra correction term
             }
             dsdz += dsdz1;
             tmax = dmax(tree_max(cand), 0.0);
@@ -282,14 +257,14 @@ struct QpDual {
             // corrector (rc = -s.z - ds_aff.dz_aff + sigma mu)
 #pragma unroll
             for (int c = 0; c < m; c++) {
-                const double cr = (sigmamu - pp.get(c)) * inv_z(c);        // (rc + s.z)/z
-                corr.set(c, cr);
-                dz[c] = t2.get(c) + cr;
+                const double cr = (sigmamu - pp[c]) * inv_z(c);        // (rc + s.z)/z
+                corr[c] = cr;
+                dz[c] = t2[c] + cr;
             }
             solve(dz);
 #pragma unroll
             for (int c = 0; c < m; c++) {
-                const double dsc = corr.get(c) - s.get(c) - dd.get(c) * dz[c];
+                const double dsc = corr[c] - s[c] - dd[c] * dz[c];
                 cand[c] = dmax(-dsc * inv_s(c), -dz[c] * inv_z(c));
             }
             tmax = dmax(tree_max(cand), 0.0);
@@ -297,27 +272,27 @@ struct QpDual {
             // dx = -1/2 (rx + G'dz)
             double rx2[n];
 #pragma unroll
-            for (int a = 0; a < n; a++) rx2[a] = rxs.get(a);
+            for (int a = 0; a < n; a++) rx2[a] = rxs[a];
             GT_acc([&](int c) { return dz[c]; }, rx2);
             const double hstep = -0.5 * step;
 #pragma unroll
-            for (int a = 0; a < n; a++) x.set(a, fma(hstep, rx2[a], x.get(a)));
+            for (int a = 0; a < n; a++) x[a] = fma(hstep, rx2[a], x[a]);
             gap = 0.0;
             double gap1 = 0.0;
 #pragma unroll
             for (int c = 0; c < m; c++) {
-                const double s0 = s.get(c);
-                const double dsc = corr.get(c) - s0 - dd.get(c) * dz[c];
-                const double sc = fma(step, dsc, s0), zc = fma(step, dz[c], z.get(c));
-                s.set(c, sc); z.set(c, zc);
+                const double s0 = s[c];
+                const double dsc = corr[c] - s0 - dd[c] * dz[c];
+                const double sc = fma(step, dsc, s0), zc = fma(step, dz[c], z[c]);
+                s[c] = sc; z[c] = zc;
                 if (c & 1) gap1 = fma(sc, zc, gap1); else gap = fma(sc, zc, gap);
             }
             gap += gap1;
         }
 #pragma unroll
         for (int i = 0; i < N; i++) {
-            ux[i] = x.get(2 * i);
-            uy[i] = x.get(2 * i + 1);
+            ux[i] = x[2 * i];
+            uy[i] = x[2 * i + 1];
         }
         return iters;
     }

@@ -1,4 +1,4 @@
-// Barrier-certificate QP, one env per thread, everything in registers (small teams).
+// Barrier-certificate QP, one env per thread, primal normal equations (teams of 5 and 6 robots).
 //
 // Replaces rps create_single_integrator_barrier_certificate{,2} -> cvxopt.solvers.qp (called at
 // /root/reference/robotarium_gym/utilities/controller.py:23; SURVEY.md App. A.8 / A.9).
@@ -14,81 +14,68 @@
 //   graph Laplacian of 2x2 blocks  w_c a_c a_c'  -> packed lower-triangular Cholesky, no pivoting.
 #pragma once
 #include "common.cuh"
-#include "qp_store.cuh"
 
 namespace mrb {
 
-// Storage of the factor.  The 2N x 2N Cholesky factor is kept as N x N blocks of 2 x 2 (one block per robot
-// pair, [e0 e1; e2 e3] = rows 2a, 2a+1 x columns 2b, 2b+1).  The diagonal blocks live in registers as
-// (1/l11, 1/l22, l21).  The strictly-lower blocks of the first RS block rows live in SHARED memory, two 128-bit
-// words per block, interleaved over the threads of the CTA (word w of thread t at Ls[w * TPB + t]: conflict-free);
-// block rows >= RS stay in registers.  With everything in registers (RS = 0) a 6-robot team needs ~350 live
-// doubles per env and the kernel spills ~1.9 KB per thread to local memory; the factor is the one large array
-// whose accesses are few enough per flop (each block is read once per triangular solve, and the block-row
-// factorisation below reads 20 blocks and writes 15) to sit behind the 128 B/clk shared-memory pipe.
-//
-// The per-constraint vectors of the iteration (m = N(N-1)/2 numbers each) follow the same rule: the ones in
-// kVecMask (bit order: VecId) live in shared memory, one double per (vector, constraint) interleaved over the
-// threads like the factor; the others are register arrays.
-enum VecId { V_H = 0, V_RZ, V_T2, V_SINV, V_ZINV, V_DS, V_DZ, V_S, V_Z, V_W, V_AX, V_AY, V_COUNT };
+// Storage.  Registers cap the number of resident warps, and these kernels are bound by dependent-issue latency, i.e.
+// by how many warps an SM sub-partition can switch between (DESIGN.md section 4).  The 2N x 2N Cholesky factor is kept
+// as N x N blocks of 2 x 2 (one block per robot pair, [e0 e1; e2 e3] = rows 2a, 2a+1 x columns 2b, 2b+1).  The
+// diagonal blocks live in registers as (1/l11, 1/l22, l21).  The strictly-lower blocks live in SHARED memory, two
+// 128-bit words per block, interleaved over the threads of the CTA (word w of thread t at Ls[w * TPB + t]:
+// conflict-free).  With everything in registers a 6-robot team needs ~350 live doubles per env and the kernel spills
+// ~1.9 KB per thread to local memory; the factor is the one large array whose accesses are few enough per flop (each
+// block is read once per triangular solve, and the block-row factorisation below reads 20 blocks and writes 15) to
+// sit behind the 128 B/clk shared-memory pipe.  Two per-constraint vectors (m = N(N-1)/2 numbers each), h and rz,
+// live in the same store, one double per constraint interleaved over the threads like the factor; the other vectors
+// are register arrays.
 
-// MRB_QP_RECOMPUTE: 1 = 1/s and 1/z are recomputed where they are used (same function of the same input: identical
-// bits) and the corrector's (ds, dz) are recomputed in the update pass instead of being stored: two SFU seeds and
-// ~10 flops per constraint buy four fewer per-constraint vectors to keep on chip.
-#ifndef MRB_QP_RECOMPUTE
-#define MRB_QP_RECOMPUTE 1
-#endif
-#ifndef MRB_QP_RECOMPUTE_INV          // 0: keep 1/s and 1/z as stored vectors even when (ds, dz) are recomputed
-#define MRB_QP_RECOMPUTE_INV MRB_QP_RECOMPUTE
-#endif
+// One per-env vector in the shared store: element c of this thread's vector at base[c * TPB].
+template <int TPB>
+struct SharedCol {
+    double *base;
+    // volatile: without it the compiler merges the repeated loads of one iteration into a single early load and
+    // keeps the value live (then spills it to local memory) -- the opposite of what this store is for
+    __device__ __forceinline__ double get(int c) const { return reinterpret_cast<const volatile double *>(base)[c * TPB]; }
+    __device__ __forceinline__ void set(int c, double v) { reinterpret_cast<volatile double *>(base)[c * TPB] = v; }
+};
+__device__ __forceinline__ void lds_block(uint32_t addr, uint32_t stride, double (&o)[4])
+{
+    asm volatile("ld.volatile.shared.v2.f64 {%0, %1}, [%2];" : "=d"(o[0]), "=d"(o[1]) : "r"(addr));
+    asm volatile("ld.volatile.shared.v2.f64 {%0, %1}, [%2];" : "=d"(o[2]), "=d"(o[3]) : "r"(addr + stride));
+}
+__device__ __forceinline__ void sts_block(uint32_t addr, uint32_t stride, const double (&o)[4])
+{
+    asm volatile("st.volatile.shared.v2.f64 [%0], {%1, %2};" ::"r"(addr), "d"(o[0]), "d"(o[1]));
+    asm volatile("st.volatile.shared.v2.f64 [%0], {%1, %2};" ::"r"(addr + stride), "d"(o[2]), "d"(o[3]));
+}
 
-template <int N, int RS_, int TPB, unsigned VMASK = 0>
+// TPB: threads per CTA (the interleave stride of the shared store)
+template <int N, int TPB>
 struct QpThread {
     static constexpr int n = 2 * N;
     static constexpr int m = N * (N - 1) / 2;
-    static constexpr int RS = RS_ > N ? N : RS_;
-    static constexpr int MM = m > 0 ? m : 1;
     __device__ static constexpr int lowidx(int a, int b) { return a * (a - 1) / 2 + b; }        // a > b
-    static constexpr int kSmemBlocks = RS * (RS - 1) / 2;
-    static constexpr int kSmemWords = 2 * kSmemBlocks;            // double2 words per thread
-    static constexpr int kRegBlocks = m - kSmemBlocks;
+    static constexpr int kSmemWords = 2 * m;                      // factor: double2 words per thread (m blocks)
+    static constexpr int kVecDoubles = 2 * m;                     // h, rz: doubles per thread
     __device__ static constexpr int pair(int i, int j) { return i * (2 * N - i - 1) / 2 + (j - i - 1); }   // i < j
 
-    __device__ static constexpr bool in_smem(int id) { return (VMASK >> id) & 1u; }
-    __device__ static constexpr int slot(int id) { int k = 0; for (int b = 0; b < id; b++) k += (VMASK >> b) & 1u; return k; }
-    static constexpr int kSmemVecs = slot(V_COUNT);
-    static constexpr int kVecDoubles = kSmemVecs * MM;          // doubles per thread in the vector store
-    template <int ID> using Vec = MVec<MM, TPB, in_smem(ID)>;
-
-    Vec<V_AX> ax;
-    Vec<V_AY> ay;
-    double Lr[kRegBlocks > 0 ? kRegBlocks : 1][4];
+    double ax[m], ay[m];
     double invd[n], l21[N];
     uint32_t Ls;                 // shared-window address of this thread's first factor word
-    double *Vs;
+    double *Vs;                  // this thread's first vector double
 
     template <int A, int B>
     __device__ __forceinline__ void load_blk(double (&o)[4]) const
     {
-        if constexpr (A < RS) {
-            lds_block(Ls + (2 * lowidx(A, B)) * TPB * 16, TPB * 16, o);
-        } else {
-#pragma unroll
-            for (int e = 0; e < 4; e++) o[e] = Lr[lowidx(A, B) - kSmemBlocks][e];
-        }
+        lds_block(Ls + (2 * lowidx(A, B)) * TPB * 16, TPB * 16, o);
     }
     template <int A, int B>
     __device__ __forceinline__ void store_blk(const double (&o)[4])
     {
-        if constexpr (A < RS) {
-            sts_block(Ls + (2 * lowidx(A, B)) * TPB * 16, TPB * 16, o);
-        } else {
-#pragma unroll
-            for (int e = 0; e < 4; e++) Lr[lowidx(A, B) - kSmemBlocks][e] = o[e];
-        }
+        sts_block(Ls + (2 * lowidx(A, B)) * TPB * 16, TPB * 16, o);
     }
 
-    __device__ __forceinline__ QpThread(double2 *Ls_, double *Vs_) : ax(Vs_, slot(V_AX) * MM), ay(Vs_, slot(V_AY) * MM), Ls((uint32_t)__cvta_generic_to_shared(Ls_)), Vs(Vs_) {}
+    __device__ __forceinline__ QpThread(double2 *Ls_, double *Vs_) : Ls((uint32_t)__cvta_generic_to_shared(Ls_)), Vs(Vs_) {}
 
     // sink(c, (G v)_c) for every constraint c
     template <typename F>
@@ -99,7 +86,7 @@ struct QpThread {
         for (int i = 0; i < N - 1; i++)
 #pragma unroll
             for (int j = i + 1; j < N; j++, c++)
-                sink(c, ax.get(c) * (v[2 * j] - v[2 * i]) + ay.get(c) * (v[2 * j + 1] - v[2 * i + 1]));
+                sink(c, ax[c] * (v[2 * j] - v[2 * i]) + ay[c] * (v[2 * j + 1] - v[2 * i + 1]));
     }
     // out += G' y,  y given as a function of the constraint index
     template <typename F>
@@ -111,7 +98,7 @@ struct QpThread {
 #pragma unroll
             for (int j = i + 1; j < N; j++, c++) {
                 const double yc = y(c);
-                const double tx = ax.get(c) * yc, ty = ay.get(c) * yc;
+                const double tx = ax[c] * yc, ty = ay[c] * yc;
                 out[2 * i] -= tx; out[2 * i + 1] -= ty;
                 out[2 * j] += tx; out[2 * j + 1] += ty;
             }
@@ -131,7 +118,7 @@ struct QpThread {
             for (int i = 0; i < N - 1; i++)
 #pragma unroll
                 for (int j = i + 1; j < N; j++, c++) {
-                    const double wc = w(c), ac = ax.get(c), bc = ay.get(c);
+                    const double wc = w(c), ac = ax[c], bc = ay[c];
                     const double wx = wc * ac, wy = wc * bc;
                     const double pxx = wx * ac, pxy = wx * bc, pyy = wy * bc;
                     dxx[i] += pxx; dxy[i] += pxy; dyy[i] += pyy;
@@ -144,7 +131,7 @@ struct QpThread {
             static_for<0, a>([&](auto B_) {
                 constexpr int b = decltype(B_)::value;
                 constexpr int c = pair(b, a);
-                const double wc = w(c), ac = ax.get(c), bc = ay.get(c);
+                const double wc = w(c), ac = ax[c], bc = ay[c];
                 const double wx = wc * ac, wy = wc * bc;
                 double s0 = -wx * ac, s1 = -wx * bc, s2 = s1, s3 = -wy * bc;
                 static_for<0, b>([&](auto C_) {
@@ -227,18 +214,8 @@ struct QpThread {
             q[2 * i] = -2.0 * ux[i];
             q[2 * i + 1] = -2.0 * uy[i];
         }
-        if (m == 0) return 0;                  // single robot: u = dxi
-
-        Vec<V_H> h(Vs, slot(V_H) * MM);
-        Vec<V_S> s(Vs, slot(V_S) * MM);
-        Vec<V_Z> z(Vs, slot(V_Z) * MM);
-        Vec<V_RZ> rz(Vs, slot(V_RZ) * MM);
-        Vec<V_T2> t2(Vs, slot(V_T2) * MM);
-        Vec<V_W> w(Vs, slot(V_W) * MM);
-        Vec<V_SINV> sinv(Vs, slot(V_SINV) * MM);
-        Vec<V_ZINV> zinv(Vs, slot(V_ZINV) * MM);
-        Vec<V_DS> ds(Vs, slot(V_DS) * MM);
-        Vec<V_DZ> dz(Vs, slot(V_DZ) * MM);
+        SharedCol<TPB> h{Vs}, rz{Vs + (size_t)m * TPB};
+        double s[m], z[m], t2[m], w[m];
 
         const double r2 = barrier_default ? 0.17 * 0.17 : 0.2 * 0.2;
         double hh = 0.0, qq = 0.0;
@@ -253,7 +230,7 @@ struct QpThread {
                     double gain = barrier_default ? 100.0 : (hv >= 0.0 ? 100.0 : 1e6);
                     const double hc = gain * (hv * hv * hv);
                     h.set(c, hc);
-                    ax.set(c, 2.0 * ex); ay.set(c, 2.0 * ey);
+                    ax[c] = 2.0 * ex; ay[c] = 2.0 * ey;
                     hh += hc * hc;
                 }
 #pragma unroll
@@ -270,7 +247,7 @@ struct QpThread {
         double ss = 0.0, ts = -INFINITY, tz = -INFINITY;
         G_mul(x, [&](int c, double gx) {
             const double zc = gx - h.get(c);
-            z.set(c, zc);
+            z[c] = zc;
             ss += zc * zc;
             ts = dmax(zc, ts);                // max(-s) = max(z)
             tz = dmax(-zc, tz);
@@ -281,11 +258,11 @@ struct QpThread {
         double gap = 0.0;
 #pragma unroll
         for (int c = 0; c < m; c++) {
-            const double z0 = z.get(c);
+            const double z0 = z[c];
             double sc = -z0, zc = z0;
             if (do_s) sc += s_shift;
             if (do_z) zc += z_shift;
-            s.set(c, sc); z.set(c, zc);
+            s[c] = sc; z[c] = zc;
             gap += sc * zc;
         }
 
@@ -301,16 +278,16 @@ struct QpThread {
                 xq += x[a] * q[a];
             }
             const double f0 = 0.5 * (xrx + xq);
-            GT_acc([&](int c) { return z.get(c); }, rx);
+            GT_acc([&](int c) { return z[c]; }, rx);
             double resx = 0.0, resx1 = 0.0, resz = 0.0, resz1 = 0.0, zrz = 0.0, zrz1 = 0.0;      // sums in two halves
 #pragma unroll
             for (int a = 0; a < n; a += 2) { resx = fma(rx[a], rx[a], resx); resx1 = fma(rx[a + 1], rx[a + 1], resx1); }
             resx += resx1;
             G_mul(x, [&](int c, double gx) {
-                const double r = gx + (s.get(c) - h.get(c));
+                const double r = gx + (s[c] - h.get(c));
                 rz.set(c, r);
-                if (c & 1) { resz1 = fma(r, r, resz1); zrz1 = fma(z.get(c), r, zrz1); }
-                else { resz = fma(r, r, resz); zrz = fma(z.get(c), r, zrz); }
+                if (c & 1) { resz1 = fma(r, r, resz1); zrz1 = fma(z[c], r, zrz1); }
+                else { resz = fma(r, r, resz); zrz = fma(z[c], r, zrz); }
             });
             resz += resz1; zrz += zrz1;
             const double pcost = f0, dcost = f0 + zrz - gap;
@@ -321,14 +298,13 @@ struct QpThread {
 
             // w = z/s ; K = 2I + G' diag(w) G
 #pragma unroll
-            for (int c = 0; c < m; c++) {
-                const double si = fast_rcp1(s.get(c)), zc = z.get(c);
-                if (!MRB_QP_RECOMPUTE_INV) { sinv.set(c, si); zinv.set(c, fast_rcp1(zc)); }
-                w.set(c, zc * si);
-            }
-            auto inv_s = [&](int c) { return MRB_QP_RECOMPUTE_INV ? fast_rcp1(s.get(c)) : sinv.get(c); };
-            auto inv_z = [&](int c) { return MRB_QP_RECOMPUTE_INV ? fast_rcp1(z.get(c)) : zinv.get(c); };
-            factor([&](int c) { return w.get(c); });
+            for (int c = 0; c < m; c++) w[c] = z[c] * fast_rcp1(s[c]);
+            // 1/s and 1/z are recomputed where they are used (same function of the same input: identical bits), and the
+            // corrector's (ds, dz) are recomputed in the update pass instead of being stored: two SFU seeds and ~10 flops
+            // per constraint buy four fewer per-constraint vectors to keep on chip
+            auto inv_s = [&](int c) { return fast_rcp1(s[c]); };
+            auto inv_z = [&](int c) { return fast_rcp1(z[c]); };
+            factor([&](int c) { return w[c]; });
 
             // predictor (rc = -s.z):                 K dx = -rx - G'(w.rz - z)
             // corrector (rc = -s.z - ds_aff.dz_aff + sigma mu):  K dx = -rx - G'(w.rz - z + t2),  t2 = (rc + s.z)/s
@@ -340,15 +316,15 @@ struct QpThread {
             double tm[4];
 #pragma unroll
             for (int a = 0; a < n; a++) dx[a] = -rx[a];
-            GT_acc([&](int c) { return z.get(c) - w.get(c) * rz.get(c); }, dx);
+            GT_acc([&](int c) { return z[c] - w[c] * rz.get(c); }, dx);
             solve(dx);
             double dsdz = 0.0, dsdz1 = 0.0;
             tm[0] = tm[1] = tm[2] = tm[3] = 0.0;
             G_mul(dx, [&](int c, double gd) {
                 const double dsc = -rz.get(c) - gd;
-                const double dzc = -z.get(c) - w.get(c) * dsc;
+                const double dzc = -z[c] - w[c] * dsc;
                 const double pr = dsc * dzc;                 // Mehrotra correction term
-                t2.set(c, pr);
+                t2[c] = pr;
                 if (c & 1) dsdz1 += pr; else dsdz += pr;
                 tm[c & 3] = dmax(dmax(-dsc * inv_s(c), -dzc * inv_z(c)), tm[c & 3]);
             });
@@ -358,44 +334,34 @@ struct QpThread {
             double sg = dmin(dmax(1.0 - step + dsdz * fast_rcp(gap) * (step * step), 0.0), 1.0);
             const double sigmamu = sg * sg * sg * (gap / m);
 #pragma unroll
-            for (int c = 0; c < m; c++) t2.set(c, (sigmamu - t2.get(c)) * inv_s(c));         // (rc + s.z)/s
+            for (int c = 0; c < m; c++) t2[c] = (sigmamu - t2[c]) * inv_s(c);         // (rc + s.z)/s
 #pragma unroll
             for (int a = 0; a < n; a++) dx[a] = -rx[a];
-            GT_acc([&](int c) { return z.get(c) - w.get(c) * rz.get(c) - t2.get(c); }, dx);   // -(rc + z.rz)/s
+            GT_acc([&](int c) { return z[c] - w[c] * rz.get(c) - t2[c]; }, dx);   // -(rc + z.rz)/s
             solve(dx);
             tm[0] = tm[1] = tm[2] = tm[3] = 0.0;
             G_mul(dx, [&](int c, double gd) {
                 const double dsc = -rz.get(c) - gd;
-                const double dzc = fma(-w.get(c), dsc, t2.get(c) - z.get(c));                 // (rc - z.ds)/s
-                if (!MRB_QP_RECOMPUTE) { ds.set(c, dsc); dz.set(c, dzc); }
+                const double dzc = fma(-w[c], dsc, t2[c] - z[c]);                 // (rc - z.ds)/s
                 tm[c & 3] = dmax(dmax(-dsc * inv_s(c), -dzc * inv_z(c)), tm[c & 3]);
             });
             tmax = dmax(dmax(tm[0], tm[1]), dmax(tm[2], tm[3]));
             step = tmax <= 0.99 ? 1.0 : 0.99 * fast_rcp(tmax);
             gap = 0.0;
             double gap1 = 0.0;
-            if (MRB_QP_RECOMPUTE) {
-                // the same expressions again; dx is laundered so that the compiler does not keep the first pass's
-                // 2m results live across the step-length reduction
+            // the same expressions again; dx is laundered so that the compiler does not keep the first pass's
+            // 2m results live across the step-length reduction
 #pragma unroll
-                for (int a = 0; a < n; a++) asm volatile("" : "+d"(dx[a]));
-                G_mul(dx, [&](int c, double gd) {
-                    const double dsc = -rz.get(c) - gd;
-                    const double zc0 = z.get(c);
-                    const double dzc = fma(-w.get(c), dsc, t2.get(c) - zc0);
-                    const double sc = fma(step, dsc, s.get(c)), zc = fma(step, dzc, zc0);
-                    s.set(c, sc); z.set(c, zc);
-                    if (c & 1) gap1 = fma(sc, zc, gap1); else gap = fma(sc, zc, gap);
-                });
-                gap += gap1;
-            } else {
-#pragma unroll
-                for (int c = 0; c < m; c++) {
-                    const double sc = fma(step, ds.get(c), s.get(c)), zc = fma(step, dz.get(c), z.get(c));
-                    s.set(c, sc); z.set(c, zc);
-                    gap = fma(sc, zc, gap);
-                }
-            }
+            for (int a = 0; a < n; a++) asm volatile("" : "+d"(dx[a]));
+            G_mul(dx, [&](int c, double gd) {
+                const double dsc = -rz.get(c) - gd;
+                const double zc0 = z[c];
+                const double dzc = fma(-w[c], dsc, t2[c] - zc0);
+                const double sc = fma(step, dsc, s[c]), zc = fma(step, dzc, zc0);
+                s[c] = sc; z[c] = zc;
+                if (c & 1) gap1 = fma(sc, zc, gap1); else gap = fma(sc, zc, gap);
+            });
+            gap += gap1;
 #pragma unroll
             for (int a = 0; a < n; a++) x[a] += step * dx[a];
         }

@@ -25,9 +25,7 @@ template <int SCN>
 inline cudaError_t launch_step_generic(const Params &p, const int32_t *actions, cudaStream_t s, bool *launched)
 {
     *launched = true;
-    static const bool force_warp = std::getenv("MRB_FORCE_WARP") != nullptr;      // measurement aid
-    // (ignored for ArcticTransport, which only exists on the thread kernel)
-    if (!force_warp || SCN == MRB_ARCTIC) switch (p.cfg.num_robots) {
+    switch (p.cfg.num_robots) {
     case 2: if (SCN != MRB_MATERIAL) return launch_thread<SCN, (SCN != MRB_MATERIAL ? 2 : 4)>(p, actions, s); break;
     case 3: if (SCN != MRB_MATERIAL) return launch_thread<SCN, (SCN != MRB_MATERIAL ? 3 : 4)>(p, actions, s); break;
     case 4: return launch_thread<SCN, 4>(p, actions, s);

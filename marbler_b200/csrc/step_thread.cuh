@@ -9,93 +9,50 @@
 #include "common.cuh"
 #include "qp_thread.cuh"
 #include "qp_dual.cuh"
-#include <type_traits>
 
 namespace mrb {
 
-#ifndef MRB_THREADS_PER_BLOCK
-#define MRB_THREADS_PER_BLOCK 64
-#endif
-#ifndef MRB_MIN_BLOCKS
-#define MRB_MIN_BLOCKS 4
-#endif
-// teams of 5 and 6 robots: the CTA shape is set by the shared-memory QP store (see below), not by registers
-#ifndef MRB_THREADS_PER_BLOCK_PRIMAL
-#define MRB_THREADS_PER_BLOCK_PRIMAL 256     // one 8-warp CTA per SM: its warps run the 12 k-instruction body in step and share the instruction fetches
-#endif
-#ifndef MRB_MIN_BLOCKS_PRIMAL
-#define MRB_MIN_BLOCKS_PRIMAL 1
-#endif
+// CTA shape, from the measurements in DESIGN.md section 4.  Teams of up to 4 robots (dual QP, everything in registers):
+// 255 registers and 64-thread CTAs, 4 per SM (32- and 128-thread CTAs measured the same, every lower register cap
+// slower).  Teams of 5 and 6 robots (primal QP): the shape is set by the shared-memory QP store, not by registers --
+// one 8-warp CTA per SM, whose warps run the 12 k-instruction body in step and share the instruction fetches.
 template <int N>
 struct ThreadShape {
-    static constexpr bool kPrimal = !(N >= 2 && N <= 4);
-    static constexpr int kThreads = kPrimal ? MRB_THREADS_PER_BLOCK_PRIMAL : MRB_THREADS_PER_BLOCK;
-    static constexpr int kMinBlocks = kPrimal ? MRB_MIN_BLOCKS_PRIMAL : MRB_MIN_BLOCKS;
+    static constexpr bool kPrimal = !(N >= 2 && N <= 4);     // up to 4 robots the dual Newton system is the smaller one (m <= 6 < 2N)
+    static constexpr int kThreads = kPrimal ? 256 : 64;
+    static constexpr int kMinBlocks = kPrimal ? 1 : 4;
 };
 
-// Teams of 5 and 6 robots (primal QP, qp_thread.cuh): which parts of the per-env QP state live in shared memory
-// instead of registers -- the leading MRB_QP_SMEM_ROWS block rows of the factor and the per-constraint vectors in
-// MRB_QP_SMEM_VECS (bits: VecId).  Defaults from the measurements in DESIGN.md section 4.
-#ifndef MRB_QP_SMEM_ROWS
-#define MRB_QP_SMEM_ROWS 6
-#endif
-#ifndef MRB_QP_SMEM_VECS
-#define MRB_QP_SMEM_VECS 0x03      // h, rz
-#endif
-
-// Teams of up to 4 robots (dual QP, qp_dual.cuh): the same choice -- MRB_QPD_SMEM_VECS (bits: DualVec) and
-// MRB_QPD_SMEM_L (the factor) -- together with the CTA shape MRB_THREADS_PER_BLOCK / MRB_MIN_BLOCKS.
-#ifndef MRB_QPD_SMEM_VECS
-#define MRB_QPD_SMEM_VECS 0
-#endif
-#ifndef MRB_QPD_SMEM_L
-#define MRB_QPD_SMEM_L 0
-#endif
-
-#ifndef MRB_PARK_DUAL
-#define MRB_PARK_DUAL 1            // park the outer state around the solve for teams of up to 4 robots too (measured: 0.159 -> 0.154 ms, PCP 65,536 envs)
-#endif
-
-// up to 4 robots the constraint-space (dual) Newton system is the smaller one (m <= 6 < 2N)
-template <int N>
-using QpForTeam = std::conditional_t<(N >= 2 && N <= 4), QpDual<N, ThreadShape<N>::kThreads, MRB_QPD_SMEM_VECS, MRB_QPD_SMEM_L>,
-                                     QpThread<N, MRB_QP_SMEM_ROWS, ThreadShape<N>::kThreads, MRB_QP_SMEM_VECS>>;
-
-// per-CTA shared store of the QP: [factor words (double2, primal only) | vectors (double)], interleaved over threads
-template <int N>
+// Per-CTA shared store of the primal QP (qp_thread.cuh): [factor words (double2) | h, rz (double)], interleaved over
+// the threads.  The dual QP has none: its teams launch with 0 bytes of dynamic shared memory.
+template <int N, bool = ThreadShape<N>::kPrimal>
 struct QpStore {
-    static constexpr bool kPrimal = !(N >= 2 && N <= 4);
-    __host__ __device__ static constexpr int factor_words()
-    {
-        if constexpr (kPrimal) return QpForTeam<N>::kSmemWords;
-        else return 0;
-    }
-    __host__ __device__ static constexpr int words()
-    {
-        if constexpr (kPrimal) return QpForTeam<N>::kSmemWords + (QpForTeam<N>::kVecDoubles + 1) / 2;
-        else return (QpForTeam<N>::kStoreDoubles + 1) / 2;
-    }
-    static constexpr size_t kBytes = (size_t)words() * ThreadShape<N>::kThreads * sizeof(double2);
+    static constexpr size_t kBytes = 0;
+};
+template <int N>
+struct QpStore<N, true> {
+    using Qp = QpThread<N, ThreadShape<N>::kThreads>;
+    static constexpr size_t kBytes = (size_t)(Qp::kSmemWords + Qp::kVecDoubles / 2) * ThreadShape<N>::kThreads * sizeof(double2);
     double2 *Ls;
     double *Vs;
-    __device__ __forceinline__ QpStore() : Ls(nullptr), Vs(nullptr)
+    __device__ __forceinline__ QpStore()
     {
-        if constexpr (words() > 0) {
-            extern __shared__ double2 store[];           // words() * threads per CTA, sized by the launcher
-            Ls = store + threadIdx.x;
-            Vs = reinterpret_cast<double *>(store + factor_words() * ThreadShape<N>::kThreads) + threadIdx.x;
-        }
+        extern __shared__ double2 store[];           // kBytes, sized by the launcher
+        Ls = store + threadIdx.x;
+        Vs = reinterpret_cast<double *>(store + Qp::kSmemWords * ThreadShape<N>::kThreads) + threadIdx.x;
     }
 };
+static_assert(QpStore<5>::kBytes == 122880 && QpStore<6>::kBytes == 184320, "primal QP store: 120 / 180 KB per CTA");
+
 template <int N>
 __device__ __forceinline__ int qp_run(const double (&xix)[N], const double (&xiy)[N], double (&ux)[N], double (&uy)[N],
                                       bool barrier_default, const QpStore<N> &st)
 {
-    if constexpr (N >= 2 && N <= 4) {
-        QpForTeam<N> qp(st.Vs);
+    if constexpr (ThreadShape<N>::kPrimal) {
+        typename QpStore<N>::Qp qp(st.Ls, st.Vs);
         return qp.run(xix, xiy, ux, uy, barrier_default);
     } else {
-        QpForTeam<N> qp(st.Ls, st.Vs);
+        QpDual<N> qp;
         return qp.run(xix, xiy, ux, uy, barrier_default);
     }
 }
@@ -287,7 +244,7 @@ step_thread_kernel(const __grid_constant__ Params p, const int32_t *__restrict__
     int32_t *si = p.buf.state_i32 + env;
     int32_t *sci = si + kCommonRowsI32 * S;
     double *scf = sf + (5 * N + 1) * S;
-    const QpStore<N> qp_store;
+    const QpStore<N> qp_smem;
 
     double px[N], py[N], th[N], qx[N], qy[N];
     int act[N];
@@ -363,26 +320,22 @@ step_thread_kernel(const __grid_constant__ Params p, const int32_t *__restrict__
             // loop even as a stand-alone kernel), and whatever else is live across the call makes that worse - measured
             // 205 local loads + 117 stores per iteration here against 110 + 69 alone.  So everything that is only needed
             // AFTER the solve is parked in local memory by hand (one store and one load per value and controller
-            // evaluation); volatile, so that the compiler cannot keep register copies alive across the solve.
-            constexpr bool kPark = ThreadShape<N>::kPrimal || MRB_PARK_DUAL;
-            volatile double park[kPark ? 8 * N : 1];
-            volatile int park_act[kPark ? N : 1];
-            if constexpr (kPark) {
+            // evaluation); volatile, so that the compiler cannot keep register copies alive across the solve.  Teams of
+            // up to 4 robots park too (measured: 0.159 -> 0.154 ms, PCP 65,536 envs).
+            volatile double park[8 * N];
+            volatile int park_act[N];
 #pragma unroll
-                for (int i = 0; i < N; i++) {
-                    park[i] = px[i]; park[N + i] = py[i]; park[2 * N + i] = th[i]; park[3 * N + i] = gx[i];
-                    park[4 * N + i] = gy[i]; park[5 * N + i] = dist[i]; park[6 * N + i] = cs[i]; park[7 * N + i] = sn[i];
-                    park_act[i] = act[i];
-                }
+            for (int i = 0; i < N; i++) {
+                park[i] = px[i]; park[N + i] = py[i]; park[2 * N + i] = th[i]; park[3 * N + i] = gx[i];
+                park[4 * N + i] = gy[i]; park[5 * N + i] = dist[i]; park[6 * N + i] = cs[i]; park[7 * N + i] = sn[i];
+                park_act[i] = act[i];
             }
-            const int it = qp_run<N>(xix, xiy, ux, uy, c.barrier_default != 0, qp_store);   // controller.py:23
-            if constexpr (kPark) {
+            const int it = qp_run<N>(xix, xiy, ux, uy, c.barrier_default != 0, qp_smem);    // controller.py:23
 #pragma unroll
-                for (int i = 0; i < N; i++) {
-                    px[i] = park[i]; py[i] = park[N + i]; th[i] = park[2 * N + i]; gx[i] = park[3 * N + i];
-                    gy[i] = park[4 * N + i]; dist[i] = park[5 * N + i]; cs[i] = park[6 * N + i]; sn[i] = park[7 * N + i];
-                    act[i] = park_act[i];
-                }
+            for (int i = 0; i < N; i++) {
+                px[i] = park[i]; py[i] = park[N + i]; th[i] = park[2 * N + i]; gx[i] = park[3 * N + i];
+                gy[i] = park[4 * N + i]; dist[i] = park[5 * N + i]; cs[i] = park[6 * N + i]; sn[i] = park[7 * N + i];
+                act[i] = park_act[i];
             }
             n_it += it;
             n_stall += it >= 25;

@@ -13,13 +13,8 @@
 
 namespace mrb {
 
-#ifndef MRB_WARPS_PER_BLOCK
-#define MRB_WARPS_PER_BLOCK 4
-#endif
-constexpr int kWarpsPerBlock = MRB_WARPS_PER_BLOCK;
-#ifndef MRB_WARP_MIN_BLOCKS
-#define MRB_WARP_MIN_BLOCKS 3      // 168 registers, 12 warps per SM (the per-constraint vectors that used to force 255 registers are recomputed or read back from the workspace)
-#endif
+constexpr int kWarpsPerBlock = 4;
+constexpr int kWarpMinBlocks = 3;      // 168 registers, 12 warps per SM (the per-constraint vectors that used to force 255 registers are recomputed or read back from the workspace)
 constexpr unsigned kFull = 0xffffffffu;
 
 __device__ __forceinline__ double warp_sum(double v)
@@ -68,13 +63,11 @@ __host__ __device__ constexpr size_t warp_workspace_doubles(int N)
 __host__ __device__ constexpr int team_ppl(int N) { return (N * (N - 1) / 2 + 31) / 32; }
 // (register file: 168 registers at 12 warps; small teams need fewer -- measured, 65,536 envs: 8 robots 6.54 ms at 12 warps,
 // 5.91 at 16, 5.78 at 20; 12 robots 11.30 / 10.99 / 10.99; 16 robots 17.85 / 17.21 / 18.18)
-#ifndef MRB_TEAM_WARPS_CAP
-#define MRB_TEAM_WARPS_CAP(N) ((N) <= 8 ? 20 : (N) <= 16 ? 16 : 12)
-#endif
 __host__ __device__ constexpr int team_warps(int N)
 {
     const int fit = (int)((227 * 1024) / (warp_workspace_doubles(N) * sizeof(double)));
-    return fit < MRB_TEAM_WARPS_CAP(N) ? fit : MRB_TEAM_WARPS_CAP(N);
+    const int cap = N <= 8 ? 20 : N <= 16 ? 16 : 12;
+    return fit < cap ? fit : cap;
 }
 
 // NC: compile-time size of the Newton system in robots, a multiple of 4 (0 = run-time team size, 2 x 2-block code).  The
@@ -668,7 +661,7 @@ struct QpWarp {
 // 14 k-instruction body roughly in step and share the instruction fetches (21.8 vs 22.5 ms per 32,768 envs); the generic
 // path keeps 4-warp CTAs because the workspace of a 32-robot team would not fit twelve times.
 template <int SCN, int PPL, int NC = 0, int WPB = kWarpsPerBlock, bool EXACT = true>
-__global__ void __launch_bounds__(WPB * 32, NC == 0 ? MRB_WARP_MIN_BLOCKS : 1)
+__global__ void __launch_bounds__(WPB * 32, NC == 0 ? kWarpMinBlocks : 1)
 step_warp_kernel(const __grid_constant__ Params p, const int32_t *__restrict__ actions)
 {
     extern __shared__ __align__(16) double smem[];
@@ -1027,7 +1020,7 @@ inline cudaError_t launch_step_warp(const Params &p, const int32_t *actions, cud
 
 // ---- barrier QP alone, one problem per warp
 template <int PPL, int NC = 0, bool EXACT = true>
-__global__ void __launch_bounds__(kWarpsPerBlock * 32, MRB_WARP_MIN_BLOCKS)
+__global__ void __launch_bounds__(kWarpsPerBlock * 32, kWarpMinBlocks)
 qp_warp_kernel(int N_, int64_t B, int barrier_default, const double *__restrict__ dxi, const double *__restrict__ xi,
                double *__restrict__ u, int32_t *__restrict__ iters)
 {
