@@ -206,7 +206,8 @@ const char *mrb_policy_last_error(const mrb_policy *policy);
 /* obs f32 [B][N][D], hidden f32 [B][N][H] (in/out), actions i32 [B][N] (out), q f32 [B][N][n_actions] (out,
  * may be NULL), fresh u8 [B] (may be NULL): envs flagged != 0 start a new episode - their hidden state and
  * observation are taken as zero (run_env re-zeroes hs and feeds reset()'s all-zero obs, misc.py:156,219).
- * All device pointers; stream-ordered, no synchronisation. */
+ * All device pointers; stream-ordered, no synchronisation.  hidden must be 16-byte aligned (MRB_E_ARG otherwise):
+ * the kernels access it as float4; a contiguous view that starts a multiple of 4 floats into an allocation is. */
 int mrb_policy_act(mrb_policy *policy, int64_t num_envs, const float *obs, float *hidden, int32_t *actions,
                    float *q, const uint8_t *fresh, void *cuda_stream);
 

@@ -555,7 +555,10 @@ extern "C" int mrb_policy_act(mrb_policy *pol, int64_t num_envs, const float *ob
                               float *q, const uint8_t *fresh, void *stream)
 {
     if (!pol || !obs || !hidden || !actions || num_envs < 1) return pfail(pol, MRB_E_ARG, "mrb_policy_act: bad argument");
-    if (((uintptr_t)hidden & 7) != 0) return pfail(pol, MRB_E_ARG, "mrb_policy_act: hidden must be 8-byte aligned");
+    // the tcgen05 kernel moves hidden rows as float4 (the mma.sync kernel as float2): one rule for every path, so that a
+    // buffer that works with one model works with all of them
+    if (((uintptr_t)hidden & 15) != 0)
+        return pfail(pol, MRB_E_ARG, "mrb_policy_act: hidden must be 16-byte aligned (its kernels access it as float4)");
     cudaError_t st = cudaSetDevice(pol->device);
     if (st != cudaSuccess) return pfail(pol, MRB_E_CUDA, cudaGetErrorString(st));
     PolicyParams p = pol->p;
