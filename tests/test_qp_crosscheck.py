@@ -14,46 +14,11 @@ import sys
 
 import numpy as np
 import pytest
-from scipy.optimize import nnls
 
 import golden_util as gu
+from qp_util import _exact, _problem
 
 SHIMS = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "shims")
-
-
-def _problem(dxi, xi, default):
-    """rps create_single_integrator_barrier_certificate{,2} (SURVEY App. A.8): min |u - dxi|^2  s.t.  A u <= b."""
-    N = dxi.shape[1]
-    dxi = dxi.copy()
-    nrm = np.linalg.norm(dxi, axis=0)
-    big = nrm > 0.2
-    dxi[:, big] *= 0.2 / nrm[big]
-    r2 = 0.17 ** 2 if default else 0.2 ** 2
-    rows, b = [], []
-    for i in range(N - 1):
-        for j in range(i + 1, N):
-            e = xi[:, i] - xi[:, j]
-            h = e @ e - r2
-            a = np.zeros(2 * N)
-            a[2 * i:2 * i + 2], a[2 * j:2 * j + 2] = -2 * e, 2 * e
-            rows.append(a)
-            b.append((100.0 if (default or h >= 0) else 1e6) * h ** 3)
-    return dxi.reshape(-1, order="F"), np.array(rows), np.array(b)
-
-
-def _exact(d, A, b):
-    """Least-distance problem by Lawson-Hanson: min |u - d|  s.t.  A u <= b   <=>   NNLS on the dual."""
-    # u = d - A' lam / 1 with lam >= 0 minimising |A' lam - ... |: solve  min_{lam>=0} |[A'; (b - A d)'] lam + [0; 1]|  (LDP)
-    c = b - A @ d                                   # constraints in shifted variable y = u - d:  A y <= c
-    E = np.vstack([-A.T, -c[None, :]])
-    f = np.zeros(E.shape[0])
-    f[-1] = 1.0
-    lam, _ = nnls(E, f, maxiter=20 * E.shape[1] + 1000)
-    r = E @ lam - f
-    if abs(r[-1]) < 1e-14:                          # y = 0 is optimal only when d itself is feasible
-        return d.copy()
-    y = -r[:-1] / r[-1]
-    return d + y
 
 
 @pytest.mark.parametrize("N", sorted(gu.qp_vectors().keys()))

@@ -15,6 +15,8 @@ import numpy as np
 import pytest
 import torch
 
+from qp_util import _hard_layouts
+
 pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -52,20 +54,6 @@ def _both(lib, dxi, xi, default):
     assert st == 0, "CUDA error %d" % st
     out = lambda u: u.cpu().numpy().transpose(2, 0, 1)
     return out(u_ref), it_ref.cpu().numpy(), out(u_new), it_new.cpu().numpy()
-
-
-def _hard_layouts(rng, B, N):
-    xi = np.stack([rng.uniform(-1.5, 1.5, (B, N)), rng.uniform(-0.9, 0.9, (B, N))], axis=1)
-    for b in range(B):
-        k = b % 3
-        if k == 0:                                   # a pair inside the safety radius (0.17 / 0.2)
-            i, j = rng.choice(N, 2, replace=False)
-            xi[b][:, j] = xi[b][:, i] + rng.uniform(-0.14, 0.14, 2)
-        elif k == 1:                                 # near-coincident robots
-            i, j = rng.choice(N, 2, replace=False)
-            xi[b][:, j] = xi[b][:, i] + rng.uniform(-1e-3, 1e-3, 2)
-    dxi = rng.uniform(-0.3, 0.3, (B, 2, N))
-    return dxi, xi
 
 
 def _pcp_layouts(rng, B, steps):
