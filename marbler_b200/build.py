@@ -52,7 +52,10 @@ def build(force=False, verbose=False):
     if verbose:
         for _, log in results:
             print(log)
-    res = subprocess.run([nvcc, "-shared", "-o", LIB_PATH] + [o for o, _ in results], capture_output=True, text=True)
+    # --no-undefined: a launcher that launchers.h declares and no unit instantiates fails the link instead of leaving an
+    # undefined symbol in the library
+    res = subprocess.run([nvcc, "-shared", "-Xlinker", "--no-undefined", "-o", LIB_PATH] + [o for o, _ in results],
+                         capture_output=True, text=True)
     if res.returncode != 0:
         raise RuntimeError("marbler_b200: link failed\n" + res.stdout + res.stderr)
     return LIB_PATH

@@ -187,18 +187,15 @@ static int step_range(mrb_env *env, const int32_t *actions, int64_t lo, int64_t 
     p.env_lo = lo;
     p.env_hi = hi;
     if (hout) p.hout = *hout;
-    // teams of up to 6 robots: one env per thread (registers); larger teams: one env per warp
-    bool launched = false;
     cudaError_t st;
     switch (p.cfg.scenario) {
-    case MRB_PCP: st = launch_step_pcp(p, actions, s, &launched); break;
-    case MRB_WAREHOUSE: st = launch_step_warehouse(p, actions, s, &launched); break;
-    case MRB_MATERIAL: st = launch_step_material(p, actions, s, &launched); break;
-    case MRB_ARCTIC: st = launch_step_arctic(p, actions, s, &launched); break;
-    default: st = launch_step_simple(p, actions, s, &launched); break;
+    case MRB_PCP: st = launch_step<MRB_PCP>(p, actions, s); break;
+    case MRB_WAREHOUSE: st = launch_step<MRB_WAREHOUSE>(p, actions, s); break;
+    case MRB_MATERIAL: st = launch_step<MRB_MATERIAL>(p, actions, s); break;
+    case MRB_ARCTIC: st = launch_step<MRB_ARCTIC>(p, actions, s); break;
+    default: st = launch_step<MRB_SIMPLE>(p, actions, s); break;
     }
     if (st != cudaSuccess) return cuda_fail(env, st, "step kernel launch");
-    if (!launched) return fail(env, MRB_E_UNSUPPORTED, "mrb_step: no kernel for this (scenario, num_robots)");
     g_launches++;
     if ((st = cudaGetLastError()) != cudaSuccess) return cuda_fail(env, st, "step kernel launch");
     return MRB_OK;

@@ -67,9 +67,13 @@ cudaError_t launch_barrier_qp(int N, int barrier_default, int64_t B, const doubl
     case 4: return launch_qp_thread<4>(B, barrier_default, dxi, xi, u, iters, s);
     case 5: return launch_qp_thread<5>(B, barrier_default, dxi, xi, u, iters, s);
     case 6: return launch_qp_thread<6>(B, barrier_default, dxi, xi, u, iters, s);
-    default: return launch_qp_warp(N, barrier_default, B, dxi, xi, u, iters, s);
+    default: break;
     }
-    return cudaGetLastError();
+    // one robot (no pair constraint) and MRB_WARP_GENERIC: the run-time team size kernel; 7..32 robots: the tensor-core
+    // kernels of the PredatorCapturePrey team units
+    if (N >= 7 && team_size(N) <= team_kernel_max(MRB_PCP) && !warp_generic())
+        return with_team_size<team_kernel_max(MRB_PCP)>(N, [&](auto nc) { return launch_qp_team<nc>(N, barrier_default, B, dxi, xi, u, iters, s); });
+    return with_runtime_ppl(N, [&](auto ppl) { return launch_qp_warp_ppl<ppl>(N, barrier_default, B, dxi, xi, u, iters, s); });
 }
 
 }  // namespace mrb

@@ -1,8 +1,4 @@
-#include "step_dispatch.cuh"
+#include "step_warp.cuh"
 namespace mrb {
-cudaError_t launch_step_arctic(const Params &p, const int32_t *actions, cudaStream_t s, bool *launched)
-{
-    *launched = p.cfg.num_robots == 4;          // the scenario is defined for exactly 4 robots
-    return *launched ? launch_thread<MRB_ARCTIC, 4>(p, actions, s) : cudaSuccess;
-}
+template cudaError_t launch_step<MRB_ARCTIC>(const Params &, const int32_t *, cudaStream_t);
 }  // namespace mrb

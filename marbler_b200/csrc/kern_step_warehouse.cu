@@ -1,7 +1,4 @@
-#include "step_dispatch.cuh"
+#include "step_warp.cuh"
 namespace mrb {
-cudaError_t launch_step_warehouse(const Params &p, const int32_t *actions, cudaStream_t s, bool *launched)
-{
-    return launch_step_generic<MRB_WAREHOUSE>(p, actions, s, launched);
-}
+template cudaError_t launch_step<MRB_WAREHOUSE>(const Params &, const int32_t *, cudaStream_t);
 }  // namespace mrb

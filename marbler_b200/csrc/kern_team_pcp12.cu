@@ -1,5 +1,5 @@
-#define MRB_TEAM_SCN MRB_PCP
-#define MRB_TEAM_TAG pcp
-#define MRB_TEAM_N 12
-#define MRB_TEAM_WITH_QP
-#include "kern_team.inc.h"
+#include "kern_team.cuh"
+namespace mrb {
+template cudaError_t launch_step_team<MRB_PCP, 12>(const Params &, const int32_t *, cudaStream_t, bool);
+template cudaError_t launch_qp_team<12>(int, int, int64_t, const double *, const double *, double *, int32_t *, cudaStream_t);
+}  // namespace mrb

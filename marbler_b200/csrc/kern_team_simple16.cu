@@ -1,4 +1,4 @@
-#define MRB_TEAM_SCN MRB_SIMPLE
-#define MRB_TEAM_TAG simple
-#define MRB_TEAM_N 16
-#include "kern_team.inc.h"
+#include "kern_team.cuh"
+namespace mrb {
+template cudaError_t launch_step_team<MRB_SIMPLE, 16>(const Params &, const int32_t *, cudaStream_t, bool);
+}  // namespace mrb

@@ -1,19 +1,26 @@
-// Launch entry points, one translation unit per scenario so that the library builds in parallel.
+// Launch entry points.  The step kernels are spread over translation units so that the library builds in parallel: one
+// per scenario (kern_step_<scenario>.cu) and one per scenario and compile-time team size (kern_team_<scenario><n>.cu).
 #pragma once
 #include "common.cuh"
 
 namespace mrb {
-// *launched = false when no kernel exists for (scenario, num_robots)
-cudaError_t launch_step_pcp(const Params &p, const int32_t *actions, cudaStream_t s, bool *launched);
-cudaError_t launch_step_warehouse(const Params &p, const int32_t *actions, cudaStream_t s, bool *launched);
-cudaError_t launch_step_material(const Params &p, const int32_t *actions, cudaStream_t s, bool *launched);
-cudaError_t launch_step_arctic(const Params &p, const int32_t *actions, cudaStream_t s, bool *launched);
-cudaError_t launch_step_simple(const Params &p, const int32_t *actions, cudaStream_t s, bool *launched);
-// team sizes that have a kernel of their own (compile-time team size, tensor-core solver; kern_team_*.cu + kern_teams.cu):
-// *handled = false when (scenario, num_robots) has none and the caller falls back to the run-time team size kernels
-cudaError_t launch_step_team(int scenario, const Params &p, const int32_t *actions, cudaStream_t s, bool *handled);
-cudaError_t launch_qp_team(int N, int barrier_default, int64_t B, const double *dxi, const double *xi, double *u, int32_t *iters,
-                           cudaStream_t s, bool *handled);
+// kern_team_<scenario><n>.cu exists for n = 8, 12, ..., team_kernel_max(scenario); 0 = none. The PredatorCapturePrey
+// units also carry the QP-alone kernels of mrb_barrier_qp.
+constexpr int team_kernel_max(int scn) { return scn == MRB_PCP ? 32 : scn == MRB_WAREHOUSE ? 12 : scn == MRB_SIMPLE ? 16 : 0; }
+template <int SCN, int NC> cudaError_t launch_step_team(const Params &, const int32_t *, cudaStream_t, bool exact);
+template <int NC> cudaError_t launch_qp_team(int N, int barrier_default, int64_t B, const double *, const double *, double *, int32_t *, cudaStream_t);
+
+// the compile-time team size a team of N robots runs on: N rounded up to a multiple of four
+constexpr int team_size(int N) { return (N + 3) & ~3; }
+// launch(std::integral_constant<int, team_size(N)>()) if team_size(N) is one of 8, 12, ..., MAX
+template <int MAX, int NC = 8, typename F>
+cudaError_t with_team_size(int N, F &&launch)
+{
+    if constexpr (NC > MAX) return cudaErrorNotSupported;
+    else return team_size(N) == NC ? launch(std::integral_constant<int, NC>()) : with_team_size<MAX, NC + 4>(N, launch);
+}
+
+template <int SCN> cudaError_t launch_step(const Params &p, const int32_t *actions, cudaStream_t s);   // kern_step_<scenario>.cu
 cudaError_t launch_reset(const Params &p, const uint8_t *mask, cudaStream_t s);
 cudaError_t launch_barrier_qp(int N, int barrier_default, int64_t B, const double *dxi, const double *xi, double *u,
                               int32_t *iters, cudaStream_t s);

@@ -772,4 +772,18 @@ step_thread_kernel(const __grid_constant__ Params p, const int32_t *__restrict__
     if (done && c.auto_reset) reset_env<SCN>(p, env, episode);
 }
 
+template <int SCN, int N>
+inline cudaError_t launch_thread(const Params &p, const int32_t *actions, cudaStream_t s)
+{
+    constexpr int tpb = ThreadShape<N>::kThreads;
+    const unsigned grid = (unsigned)((p.env_hi - p.env_lo + tpb - 1) / tpb);
+    constexpr size_t smem = QpStore<N>::kBytes;
+    if (smem > 48 * 1024) {
+        const cudaError_t attr = cudaFuncSetAttribute(step_thread_kernel<SCN, N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (attr != cudaSuccess) return attr;
+    }
+    step_thread_kernel<SCN, N><<<grid, tpb, smem, s>>>(p, actions);
+    return cudaGetLastError();
+}
+
 }  // namespace mrb

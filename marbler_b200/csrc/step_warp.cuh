@@ -10,6 +10,7 @@
 
 #include "common.cuh"
 #include "launchers.h"
+#include "step_thread.cuh"     // ObsRow, reset_env, launch_thread
 
 namespace mrb {
 
@@ -984,7 +985,22 @@ step_warp_kernel(const __grid_constant__ Params p, const int32_t *__restrict__ a
     if (done && c.auto_reset && lane == 0) reset_env<SCN>(p, env, si[2 * S]);
 }
 
-inline int pairs_per_lane(int N) { return (N * (N - 1) / 2 + 31) / 32; }
+// MRB_WARP_GENERIC (any value): every team of 7 or more robots runs on the run-time team size kernels, the reference of
+// the tensor-core kernels.  Read on every launch: tests switch it within one process.
+inline bool warp_generic() { return std::getenv("MRB_WARP_GENERIC") != nullptr; }
+
+// launch(std::integral_constant<int, PPL>()) with the pair slots per lane of N robots rounded up to an instantiated width
+template <typename F>
+cudaError_t with_runtime_ppl(int N, F &&launch)
+{
+    const int ppl = team_ppl(N);
+    if (ppl <= 1) return launch(std::integral_constant<int, 1>());
+    if (ppl <= 2) return launch(std::integral_constant<int, 2>());
+    if (ppl <= 4) return launch(std::integral_constant<int, 4>());
+    if (ppl <= 6) return launch(std::integral_constant<int, 6>());
+    if (ppl <= 8) return launch(std::integral_constant<int, 8>());
+    return launch(std::integral_constant<int, 16>());
+}
 
 template <int SCN, int PPL, int NC = 0, bool EXACT = true>
 inline cudaError_t launch_step_warp_ppl(const Params &p, const int32_t *actions, cudaStream_t s)
@@ -998,24 +1014,29 @@ inline cudaError_t launch_step_warp_ppl(const Params &p, const int32_t *actions,
     return cudaSuccess;
 }
 
+// Teams of 2..6 robots: one env per thread; 7..32 robots: one env per warp, on the kernel of the scenario's compile-time
+// team size (kern_team_*.cu, tensor-core solver; measured against the run-time size in DESIGN.md section 4) where there
+// is one, else on the run-time team size kernel.  Explicitly instantiated in kern_step_<scenario>.cu.
 template <int SCN>
-inline cudaError_t launch_step_warp(const Params &p, const int32_t *actions, cudaStream_t s)
+cudaError_t launch_step(const Params &p, const int32_t *actions, cudaStream_t s)
 {
-    // ArcticTransport (exactly 4 robots, per-terrain step sizes, grid observations) exists on the thread kernel only
-    if (SCN == MRB_ARCTIC) return cudaErrorNotSupported;
-    // team sizes with a kernel of their own (kern_team_*.cu): the tensor-core solver
-    if (!std::getenv("MRB_WARP_GENERIC")) {
-        bool handled = false;
-        const cudaError_t st = launch_step_team(SCN, p, actions, s, &handled);
-        if (handled) return st;
+    const int N = p.cfg.num_robots;
+    if constexpr (SCN == MRB_ARCTIC) {           // per-terrain step sizes and grid observations, for exactly 4 robots
+        return N == 4 ? launch_thread<SCN, 4>(p, actions, s) : cudaErrorNotSupported;
+    } else {
+        switch (N) {
+        case 2: if constexpr (SCN != MRB_MATERIAL) return launch_thread<SCN, 2>(p, actions, s); break;   // MaterialTransport: 4 or more
+        case 3: if constexpr (SCN != MRB_MATERIAL) return launch_thread<SCN, 3>(p, actions, s); break;
+        case 4: return launch_thread<SCN, 4>(p, actions, s);
+        case 5: return launch_thread<SCN, 5>(p, actions, s);
+        case 6: return launch_thread<SCN, 6>(p, actions, s);
+        default:
+            if (team_size(N) <= team_kernel_max(SCN) && !warp_generic())
+                return with_team_size<team_kernel_max(SCN)>(N, [&](auto nc) { return launch_step_team<SCN, nc>(p, actions, s, N == nc); });
+            return with_runtime_ppl(N, [&](auto ppl) { return launch_step_warp_ppl<SCN, ppl>(p, actions, s); });
+        }
+        return cudaErrorNotSupported;
     }
-    const int ppl = pairs_per_lane(p.cfg.num_robots);
-    if (ppl <= 1) return launch_step_warp_ppl<SCN, 1>(p, actions, s);
-    if (ppl <= 2) return launch_step_warp_ppl<SCN, 2>(p, actions, s);
-    if (ppl <= 4) return launch_step_warp_ppl<SCN, 4>(p, actions, s);
-    if (ppl <= 6) return launch_step_warp_ppl<SCN, 6>(p, actions, s);
-    if (ppl <= 8) return launch_step_warp_ppl<SCN, 8>(p, actions, s);
-    return launch_step_warp_ppl<SCN, 16>(p, actions, s);
 }
 
 // ---- barrier QP alone, one problem per warp
@@ -1045,21 +1066,6 @@ inline cudaError_t launch_qp_warp_ppl(int N, int bd, int64_t B, const double *dx
     if (st != cudaSuccess) return st;
     qp_warp_kernel<PPL, NC, EXACT><<<(unsigned)((B + kWarpsPerBlock - 1) / kWarpsPerBlock), kWarpsPerBlock * 32, smem, s>>>(N, B, bd, dxi, xi, u, iters);
     return cudaSuccess;
-}
-inline cudaError_t launch_qp_warp(int N, int bd, int64_t B, const double *dxi, const double *xi, double *u, int32_t *iters, cudaStream_t s)
-{
-    if (!std::getenv("MRB_WARP_GENERIC")) {             // team sizes with the tensor-core solver (kern_team_*.cu)
-        bool handled = false;
-        const cudaError_t st = launch_qp_team(N, bd, B, dxi, xi, u, iters, s, &handled);
-        if (handled) return st;
-    }
-    const int ppl = pairs_per_lane(N);
-    if (ppl <= 1) return launch_qp_warp_ppl<1>(N, bd, B, dxi, xi, u, iters, s);
-    if (ppl <= 2) return launch_qp_warp_ppl<2>(N, bd, B, dxi, xi, u, iters, s);
-    if (ppl <= 4) return launch_qp_warp_ppl<4>(N, bd, B, dxi, xi, u, iters, s);
-    if (ppl <= 6) return launch_qp_warp_ppl<6>(N, bd, B, dxi, xi, u, iters, s);
-    if (ppl <= 8) return launch_qp_warp_ppl<8>(N, bd, B, dxi, xi, u, iters, s);
-    return launch_qp_warp_ppl<16>(N, bd, B, dxi, xi, u, iters, s);
 }
 
 }  // namespace mrb

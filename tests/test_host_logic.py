@@ -178,27 +178,22 @@ def test_spawn_grid_division_trick_is_exact():
             assert (cell * inv) >> 16 == cell // yr, (cell, yr)
 
 
-def test_every_team_kernel_is_dispatched():
-    """csrc/kern_team_<scenario><size>.cu (one kernel per scenario and size of the Newton system, FP64 tensor-core solver)
-    and the dispatch table csrc/kern_teams.cu are maintained by hand: every unit must be reachable, every case must exist,
-    sizes are multiples of four, and PredatorCapturePrey units carry the QP-alone kernel mrb_barrier_qp uses."""
+def test_team_kernel_table_matches_the_units():
+    """csrc/launchers.h states which (scenario, size of the Newton system) has a kernel with the FP64 tensor-core solver:
+    n = 8, 12, ..., team_kernel_max(scenario).  The units kern_team_<scenario><n>.cu must be exactly those, each must
+    instantiate the step launcher of its size, and each PredatorCapturePrey unit also the QP-alone launcher mrb_barrier_qp
+    uses."""
     import glob
     import re
     csrc = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "marbler_b200", "csrc")
-    table = open(os.path.join(csrc, "kern_teams.cu")).read()
-    units = sorted(glob.glob(os.path.join(csrc, "kern_team_*.cu")))
-    assert len(units) >= 12
-    seen = set()
-    for u in units:
-        src = open(u).read()
-        tag = re.search(r"#define MRB_TEAM_TAG (\w+)", src).group(1)
-        n = int(re.search(r"#define MRB_TEAM_N (\d+)", src).group(1))
-        scn = re.search(r"#define MRB_TEAM_SCN (\w+)", src).group(1)
-        assert n % 4 == 0 and 8 <= n <= 32, u
-        assert os.path.basename(u) == "kern_team_%s%d.cu" % (tag, n)
-        assert re.search(r"if \(scenario == %s\) switch \(size\) \{[^}]*case %d: return launch_step_team_%s_%d\(" % (scn, n, tag, n), table), u
-        if "MRB_TEAM_WITH_QP" in src:
-            assert scn == "MRB_PCP" and "case %d: return launch_qp_team_n_%d(" % (n, n) in table, u
-        seen.add((tag, n))
-    for tag, n in re.findall(r"return launch_step_team_(\w+)_(\d+)\(", table):
-        assert (tag, int(n)) in seen, (tag, n)
+    table = re.search(r"constexpr int team_kernel_max\(int scn\) \{ return (.*?); \}", open(os.path.join(csrc, "launchers.h")).read()).group(1)
+    tags = {"MRB_PCP": "pcp", "MRB_WAREHOUSE": "warehouse", "MRB_SIMPLE": "simple"}
+    maxima = {scn: int(n) for scn, n in re.findall(r"scn == (\w+) \? (\d+)", table)}
+    assert table.endswith(": 0") and set(maxima) == set(tags) and all(8 <= top <= 32 for top in maxima.values()), table
+    want = {(scn, n) for scn, top in maxima.items() for n in range(8, top + 1, 4)}
+    units = {os.path.basename(u): u for u in glob.glob(os.path.join(csrc, "kern_team_*.cu"))}
+    assert set(units) == {"kern_team_%s%d.cu" % (tags[scn], n) for scn, n in want}, sorted(units)
+    for scn, n in want:
+        src = open(units["kern_team_%s%d.cu" % (tags[scn], n)]).read()
+        assert "template cudaError_t launch_step_team<%s, %d>(" % (scn, n) in src, (scn, n)
+        assert ("template cudaError_t launch_qp_team<%d>(" % n in src) == (scn == "MRB_PCP"), (scn, n)

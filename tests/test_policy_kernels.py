@@ -27,6 +27,7 @@ import pytest
 import torch
 
 import golden_util as gu
+from trace_util import kernels_launched
 
 POLICY = os.path.join(gu.GOLDEN, "policy")
 FIXTURES = ["ArcticTransport_qmix_ns", "MaterialTransport_mappo_ns", "PredatorCapturePrey_vdn"]
@@ -169,17 +170,8 @@ def make_policy(sd, shape, accurate):
     return Policy(sd, shape["N"], shape["D"], obs_agent_id=shape["agent_id"], device="cuda:0", accurate=accurate)
 
 
-def kernels_launched(fn):
-    """Names of the CUDA kernels `fn` launches (profiler trace)."""
-    from torch.profiler import ProfilerActivity, profile
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        fn()
-        torch.cuda.synchronize()
-    return [e.name for e in prof.events() if "policy_act" in e.name]
-
-
 def assert_ran_on(kernel, fn):
-    names = kernels_launched(fn)
+    names = kernels_launched(fn, "policy_act")
     assert len(names) == 1 and KERNEL_NAME[kernel] in names[0], (kernel, names)
 
 
