@@ -17,7 +17,7 @@
 extern "C" {
 #endif
 
-#define MRB_ABI_VERSION 2
+#define MRB_ABI_VERSION 3
 #define MRB_MAX_ROBOTS 32
 #define MRB_MAX_PREY 32
 
@@ -210,6 +210,34 @@ const char *mrb_policy_last_error(const mrb_policy *policy);
  * the kernels access it as float4; a contiguous view that starts a multiple of 4 floats into an allocation is. */
 int mrb_policy_act(mrb_policy *policy, int64_t num_envs, const float *obs, float *hidden, int32_t *actions,
                    float *q, const uint8_t *fresh, void *cuda_stream);
+
+/* ---- exploratory action selection (training-time data collection).  EPyMARL, which trains the reference's
+ * checkpoints, does not act greedily while it collects data: QMIX / VDN / IQL use EpsilonGreedyActionSelector with a
+ * linear DecayThenFlatSchedule, MAPPO / IPPO use SoftPoliciesSelector.  mrb_select_actions restates both over the
+ * output of mrb_policy_act, one thread per (env, agent) row.
+ *   MRB_SELECT_EPSILON_GREEDY: actions (in/out) holds the greedy actions on entry (q is not read and may be NULL);
+ *     eps(t) = max(eps_finish, eps_start - (eps_start - eps_finish) * t / anneal_time) in double; a row explores iff
+ *     w0 < (eps >= 1 ? 2^32 : floor(eps * 2^32)), and then takes action (w1 * n_actions) >> 32.
+ *   MRB_SELECT_SOFTMAX: q f32 [B][N][n_actions] (in), actions (out): u = ((w2 >> 5) * 2^26 + (w3 >> 6)) / 2^53;
+ *     in double, e_a = exp(q_a - max q), S = sum of e_a in index order; the action is the first a whose running sum
+ *     exceeds u * S (the last a with e_a > 0 if rounding leaves none).
+ * w0..w3 is one Philox4x32-10 block: key (seed lo, seed hi), counter (gid lo, gid hi, (uint32) t, 0x80000000 | agent),
+ * gid = env_id0 + env.  t = *step, a device int64 that the call reads and then advances by one on the same stream
+ * (a one-thread kernel after the selection kernel: two launches), so every replay of a captured CUDA graph moves the
+ * schedule on.  The Philox counter takes t modulo 2^32: draws repeat after 2^32 steps of one counter. */
+enum { MRB_SELECT_EPSILON_GREEDY = 1, MRB_SELECT_SOFTMAX = 2 };
+typedef struct mrb_select_desc {
+    int32_t struct_size;        /* sizeof(mrb_select_desc): ABI check */
+    int32_t mode;               /* MRB_SELECT_* */
+    uint64_t seed;
+    int64_t env_id0;            /* global id of env 0 of this batch (sharding) */
+    double eps_start, eps_finish;   /* epsilon-greedy: DecayThenFlatSchedule, linear; both in [0, 1] */
+    int64_t anneal_time;        /* in steps of *step; >= 1 */
+} mrb_select_desc;
+/* errors through mrb_last_error(NULL); every argument is checked before the device is touched */
+int mrb_select_actions(int device, int64_t num_envs, int32_t n_agents, int32_t n_actions,
+                       const mrb_select_desc *desc, int64_t *step, const float *q, int32_t *actions,
+                       void *cuda_stream);
 
 /* FP64 roofline denominator, measured: runs a kernel of independent DFMA chains (8 per thread, one 1,024-thread
  * CTA per SM) for about `milliseconds` on `device`, timed with CUDA events, and returns the rate of the best launch

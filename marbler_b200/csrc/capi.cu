@@ -335,3 +335,28 @@ extern "C" int mrb_barrier_qp(int device, int32_t N, int32_t barrier_default, in
     if ((st = cudaGetLastError()) != cudaSuccess) return cuda_fail(nullptr, st, "qp kernel launch");
     return MRB_OK;
 }
+
+extern "C" int mrb_select_actions(int device, int64_t num_envs, int32_t n_agents, int32_t n_actions,
+                                  const mrb_select_desc *desc, int64_t *step, const float *q, int32_t *actions,
+                                  void *stream)
+{
+    if (!desc || !step || !actions) return fail(nullptr, MRB_E_ARG, "mrb_select_actions: desc, step and actions are required");
+    if (desc->struct_size != (int32_t)sizeof(mrb_select_desc))
+        return fail(nullptr, MRB_E_ARG, "mrb_select_actions: mrb_select_desc.struct_size does not match this library (ABI mismatch)");
+    if (desc->mode != MRB_SELECT_EPSILON_GREEDY && desc->mode != MRB_SELECT_SOFTMAX)
+        return fail(nullptr, MRB_E_ARG, "mrb_select_actions: unknown mode");
+    if (num_envs < 1 || n_agents < 1 || n_actions < 1)
+        return fail(nullptr, MRB_E_ARG, "mrb_select_actions: num_envs, n_agents and n_actions must be >= 1");
+    if (num_envs > ((int64_t)1 << 39) / n_agents)        // one 256-thread CTA per 256 rows: at most 2^31 CTAs
+        return fail(nullptr, MRB_E_ARG, "mrb_select_actions: num_envs * n_agents must be <= 2^39");
+    if (!(desc->eps_start >= 0.0 && desc->eps_start <= 1.0 && desc->eps_finish >= 0.0 && desc->eps_finish <= 1.0))
+        return fail(nullptr, MRB_E_ARG, "mrb_select_actions: eps_start and eps_finish must be in [0, 1]");
+    if (desc->anneal_time < 1) return fail(nullptr, MRB_E_ARG, "mrb_select_actions: anneal_time must be >= 1");
+    if (desc->mode == MRB_SELECT_SOFTMAX && !q) return fail(nullptr, MRB_E_ARG, "mrb_select_actions: softmax needs q");
+    cudaError_t st = cudaSetDevice(device);
+    if (st != cudaSuccess) return cuda_fail(nullptr, st, "cudaSetDevice");
+    st = launch_select_actions(num_envs, n_agents, n_actions, *desc, step, q, actions, (cudaStream_t)stream);
+    if (st != cudaSuccess) return cuda_fail(nullptr, st, "select kernel launch");
+    g_launches += 2;
+    return MRB_OK;
+}

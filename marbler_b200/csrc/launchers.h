@@ -24,4 +24,7 @@ template <int SCN> cudaError_t launch_step(const Params &p, const int32_t *actio
 cudaError_t launch_reset(const Params &p, const uint8_t *mask, cudaStream_t s);
 cudaError_t launch_barrier_qp(int N, int barrier_default, int64_t B, const double *dxi, const double *xi, double *u,
                               int32_t *iters, cudaStream_t s);
+// explore.cu: the selection kernel, then a one-thread kernel that advances *step
+cudaError_t launch_select_actions(int64_t num_envs, int32_t n_agents, int32_t n_actions, const mrb_select_desc &desc,
+                                  int64_t *step, const float *q, int32_t *actions, cudaStream_t s);
 }  // namespace mrb

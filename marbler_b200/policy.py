@@ -91,9 +91,11 @@ class Policy(object):
         """rnn_agent.py:17-19 init_hidden: zeros, one row per agent."""
         return torch.zeros((num_envs, self.n_agents, self.hidden_dim), dtype=torch.float32, device=self.device)
 
-    def act(self, obs, hidden, actions=None, q=None, fresh=None):
+    def act(self, obs, hidden, actions=None, q=None, fresh=None, explore=None):
         """obs f32 [B,N,D], hidden f32 [B,N,H] (updated in place) -> actions i32 [B,N] (greedy).  `fresh` u8 [B]:
-        envs that start an episode (zero hidden state and observation).  Stream-ordered, no synchronisation."""
+        envs that start an episode (zero hidden state and observation).  `explore`: an `Exploration` that then
+        replaces the greedy actions (softmax reads q, allocated here when not given).  Stream-ordered, no
+        synchronisation."""
         B = obs.shape[0]
         assert obs.is_cuda and obs.dtype == torch.float32 and obs.is_contiguous() and tuple(obs.shape) == (B, self.n_agents, self.obs_dim)
         assert hidden.dtype == torch.float32 and hidden.is_contiguous() and tuple(hidden.shape) == (B, self.n_agents, self.hidden_dim)
@@ -101,25 +103,96 @@ class Policy(object):
             actions = torch.empty((B, self.n_agents), dtype=torch.int32, device=self.device)
         if fresh is not None:
             assert fresh.dtype == torch.uint8 and fresh.is_contiguous() and fresh.shape == (B,)
+        if explore is not None and explore.mode == "softmax" and q is None:
+            q = torch.empty((B, self.n_agents, self.n_actions), dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.device):
             _lib.check_policy(self.lib.mrb_policy_act(
                 self.handle, B, _ptr(obs), _ptr(hidden), _ptr(actions), _ptr(q), _ptr(fresh),
                 C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)), self.handle)
+        if explore is not None:
+            explore.select(actions, q, n_actions=self.n_actions)
         return actions
+
+
+class Exploration(object):
+    """EPyMARL's exploratory action selectors on the device (mrb_select_actions, csrc/explore.cu).
+
+    mode "epsilon_greedy" is EpsilonGreedyActionSelector (QMIX, VDN, IQL) with its linear DecayThenFlatSchedule:
+    eps(t) = max(eps_finish, eps_start - (eps_start - eps_finish) * t / anneal_time); each (env, agent) row keeps its
+    greedy action or, with probability eps, takes one uniformly over all actions (MARBLER has no unavailable actions).
+    mode "softmax" is SoftPoliciesSelector (MAPPO, IPPO): a draw from softmax(q).  The defaults are EPyMARL's.
+
+    `step` is the schedule's counter t: an int64 CUDA tensor [1] that every `select` reads and then advances by one
+    on the stream, so a captured CUDA graph moves it on at every replay.  EPyMARL's t_env counts env steps over the
+    whole batch (it advances by the number of envs per step), so its `epsilon_anneal_time` is `anneal_time` times the
+    batch size B here: anneal_time = epsilon_anneal_time / B.
+
+    Every draw is a function of (seed, global env id, t, agent) alone (Philox; the exact contract is in
+    include/marbler_b200.h): envs sharded over several devices draw what one device would have drawn when each
+    shard passes the global id of its first env as `env_id0` (None: 0, or the env's own under `Rollout`)."""
+
+    MODES = {"epsilon_greedy": _lib.SELECT_EPSILON_GREEDY, "softmax": _lib.SELECT_SOFTMAX}
+
+    def __init__(self, mode, seed=0, env_id0=None, eps_start=1.0, eps_finish=0.05, anneal_time=50000, device=None):
+        if mode not in self.MODES:
+            raise ValueError("Exploration mode must be one of %s, not %r" % (sorted(self.MODES), mode))
+        if not torch.cuda.is_available():
+            raise RuntimeError("marbler_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback")
+        self.lib = _lib.load()
+        self.mode, self.seed, self.env_id0 = mode, int(seed) & (2 ** 64 - 1), env_id0
+        self.eps_start, self.eps_finish, self.anneal_time = float(eps_start), float(eps_finish), int(anneal_time)
+        dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        self.device = torch.device("cuda", dev.index if dev.index is not None else torch.cuda.current_device())
+        self.step = torch.zeros((1,), dtype=torch.int64, device=self.device)
+
+    def select(self, actions, q=None, n_actions=None):
+        """actions i32 [B,N] on the device: the greedy actions on entry (epsilon_greedy, which needs `n_actions`)
+        or output only (softmax, which reads q f32 [B,N,A]).  Advances `step` by one.  Stream-ordered."""
+        B, N = actions.shape
+        assert actions.dtype == torch.int32 and actions.is_contiguous() and actions.device == self.device
+        if q is not None:
+            assert q.dtype == torch.float32 and q.is_contiguous() and tuple(q.shape[:2]) == (B, N) and q.device == self.device
+            n_actions = q.shape[2] if n_actions is None else n_actions
+            assert q.shape[2] == n_actions
+        if n_actions is None:
+            raise ValueError("Exploration.select: pass n_actions (or q)")
+        d = _lib.SelectDesc(C.sizeof(_lib.SelectDesc), self.MODES[self.mode], self.seed, int(self.env_id0 or 0),
+                            self.eps_start, self.eps_finish, self.anneal_time)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.mrb_select_actions(
+                self.device.index, B, N, int(n_actions), C.byref(d), _ptr(self.step), _ptr(q), _ptr(actions),
+                C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)))
+        return actions
+
+    def epsilon(self):
+        """eps(t) of the current counter, computed on the host (synchronises; for logging)."""
+        t = int(self.step.item())
+        return max(self.eps_finish, self.eps_start - (self.eps_start - self.eps_finish) * t / self.anneal_time)
 
 
 class Rollout(object):
     """run_env's loop for a whole batch, on the device: act -> step -> act -> ...  (misc.py:155-187).
 
     The env auto-resets finished envs inside the step kernel; their `done` flag doubles as the next step's
-    `fresh` mask (zero hidden state, zero observation - what run_env feeds after env.reset())."""
+    `fresh` mask (zero hidden state, zero observation - what run_env feeds after env.reset()).
 
-    def __init__(self, vec_env, policy, use_graph=True, steps_per_graph=8):
+    `explore`: an `Exploration` that selects the actions of every step after the policy (its counter advances inside
+    the captured graph too, and `reset` does not rewind it: the schedule runs across episodes).  When its `env_id0` is
+    None it takes the env's own, so that the ranks of a sharded run draw distinct streams."""
+
+    def __init__(self, vec_env, policy, use_graph=True, steps_per_graph=8, explore=None):
         assert vec_env.N == policy.n_agents and vec_env.D == policy.obs_dim and vec_env.device == policy.device
         assert vec_env.n_actions == policy.n_actions, "policy and scenario disagree on the number of actions"
         self.env, self.policy = vec_env, policy
         self.hidden = policy.init_hidden(vec_env.B)
         self.actions = torch.zeros((vec_env.B, vec_env.N), dtype=torch.int32, device=vec_env.device)
+        self.explore, self.q = explore, None
+        if explore is not None:
+            assert explore.device == vec_env.device
+            if explore.env_id0 is None:
+                explore.env_id0 = vec_env.env_id0
+            if explore.mode == "softmax":
+                self.q = torch.zeros((vec_env.B, vec_env.N, policy.n_actions), dtype=torch.float32, device=vec_env.device)
         self.use_graph, self.steps_per_graph = use_graph, int(steps_per_graph)
         self._graph = None
 
@@ -129,11 +202,11 @@ class Rollout(object):
         self.hidden.zero_()
 
     def _one(self):
-        self.policy.act(self.env.obs, self.hidden, actions=self.actions, fresh=self.env.done)
+        self.policy.act(self.env.obs, self.hidden, actions=self.actions, q=self.q, fresh=self.env.done, explore=self.explore)
         self.env.step(self.actions)
 
     def run(self, steps):
-        """Advance every env by `steps` env steps (2 kernels per step, no host synchronisation)."""
+        """Advance every env by `steps` env steps (2 kernels per step, 4 with `explore`; no host synchronisation)."""
         k = self.steps_per_graph
         if self.use_graph:
             if self._graph is None and steps > k:
