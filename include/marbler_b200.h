@@ -17,7 +17,7 @@
 extern "C" {
 #endif
 
-#define MRB_ABI_VERSION 3
+#define MRB_ABI_VERSION 4
 #define MRB_MAX_ROBOTS 32
 #define MRB_MAX_PREY 32
 
@@ -238,6 +238,57 @@ typedef struct mrb_select_desc {
 int mrb_select_actions(int device, int64_t num_envs, int32_t n_agents, int32_t n_actions,
                        const mrb_select_desc *desc, int64_t *step, const float *q, int32_t *actions,
                        void *cuda_stream);
+
+/* ---- episode recording (training-time data collection).  EPyMARL's ParallelRunner.run fills an EpisodeBatch one
+ * step at a time; mrb_record_begin / mrb_record_step write the same fields straight into caller-owned device tensors,
+ * after every mrb_step, in one launch per step (EPyMARL is not vendored in the reference, so the contract is restated
+ * here).  B envs (the env handle's), episode limit T (EPyMARL's time_limit), N agents, D = mrb_obs_dim, A =
+ * mrb_num_actions, W = obs_width >= D (the declared observation width; columns D .. W-1 are zero, as the adapter's
+ * padding).  Every field has T + 1 rows per env (max_seq_length = episode_limit + 1), all contiguous, row-major:
+ *   obs f32 [B][T+1][N][W] | state f32 [B][T+1][N*W]: the same memory as obs (state = concat(obs)), state == obs |
+ *   actions i64 [B][T+1][N] | actions_onehot f32 [B][T+1][N][A] | avail_actions i32 [B][T+1][N][A] |
+ *   reward f32 [B][T+1] | terminated u8 [B][T+1] | filled i64 [B][T+1] | cursor i32 [B].
+ * Every env records exactly one episode, starting at row 0 (ParallelRunner.reset):
+ *   row 0: obs 0 (the reset observation), avail_actions 1, filled 1.
+ *   step t (the t-th mrb_record_step since mrb_record_begin), for every env that has not terminated yet:
+ *     actions[t] = the actions sent to the env (after exploration), actions_onehot[t] their one-hot encoding,
+ *     reward[t] = the float32 sum of the N agent rewards in agent index order,
+ *     terminated[t] = done || t + 1 >= T (truncation is stored as terminal: the gym wrapper reports no
+ *     episode_limit info), obs[t+1] = the env's obs buffer after the step (the terminal observation of an env that
+ *     has just finished), avail_actions[t+1] = 1, filled[t+1] = 1; the env is inactive from then on if terminated.
+ *   every other element is 0, including actions, actions_onehot, reward and terminated of the terminal row and all
+ *   the rows after it.
+ * Each element is written exactly once per collection: mrb_record_begin writes row 0 of obs / avail_actions / filled
+ * and row T of actions / actions_onehot / reward / terminated; step t writes row t of the latter four and row t + 1 of
+ * the former three for every env, active or not (zeros for an inactive one), so after mrb_record_begin and T calls of
+ * mrb_record_step every row has been written and the tensors need no zeroing.  cursor[b] is the recorder's position:
+ * t while env b is active, ~t (= -t - 1) once it has terminated, t = the calls since mrb_record_begin; a call at
+ * t >= T writes nothing.  Each env's cursor is read and written by that env's own thread of one launch.
+ * Accesses are scalar and of the elements' own widths (no vector accesses): every pointer must be aligned to its
+ * element size (8 bytes for actions and filled, 4 for the others), MRB_E_ARG otherwise. */
+typedef struct mrb_episode_batch {
+    int32_t struct_size;        /* sizeof(mrb_episode_batch): ABI check */
+    int32_t episode_limit;      /* T: 1 .. 2^30 */
+    int32_t obs_width;          /* W: D .. 65,536 */
+    int32_t reserved0;
+    float *obs;
+    float *state;               /* == obs */
+    int64_t *actions;
+    float *actions_onehot;
+    int32_t *avail_actions;
+    float *reward;
+    uint8_t *terminated;
+    int64_t *filled;
+    int32_t *cursor;
+} mrb_episode_batch;
+/* Brings the batch to its row-0 state (see above) and sets every cursor to 0.  One launch, stream-ordered.  Errors
+ * through mrb_last_error(env) (mrb_last_error(NULL) when env is NULL); every argument is checked before the device is
+ * touched: NULL pointers, struct_size, episode_limit, obs_width and alignment -> MRB_E_ARG, an env without buffers
+ * (mrb_bind) -> MRB_E_STATE. */
+int mrb_record_begin(mrb_env *env, const mrb_episode_batch *batch, void *cuda_stream);
+/* Records the step that mrb_step just took with `actions` (device i32 [B][N], 4-byte aligned): reads the bound obs,
+ * reward and done buffers.  One launch, stream-ordered, never synchronises; checks as mrb_record_begin. */
+int mrb_record_step(mrb_env *env, const mrb_episode_batch *batch, const int32_t *actions, void *cuda_stream);
 
 /* FP64 roofline denominator, measured: runs a kernel of independent DFMA chains (8 per thread, one 1,024-thread
  * CTA per SM) for about `milliseconds` on `device`, timed with CUDA events, and returns the rate of the best launch

@@ -5,14 +5,14 @@ import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MARBLER_B200_LIB") or os.path.join(HERE, "libmarbler_b200.so")
-ABI_VERSION = 3
+ABI_VERSION = 4
 NUM_STATS = 16
 STAT_NAMES = ("episodes", "return_sum", "length_sum", "collisions", "boundary_exits", "scenario_metric",
               "env_steps", "qp_solves", "qp_iterations", "timeouts", "qp_stalls", "substeps", "qp_iterations_warp")
 SYMBOLS = ("mrb_version", "mrb_create", "mrb_destroy", "mrb_last_error", "mrb_state_rows", "mrb_obs_dim",
            "mrb_num_actions", "mrb_bind", "mrb_reset", "mrb_step", "mrb_step_host", "mrb_barrier_qp",
            "mrb_get_state", "mrb_set_state", "mrb_fp64_peak", "mrb_launch_count", "mrb_policy_create", "mrb_policy_destroy", "mrb_policy_last_error", "mrb_policy_act",
-           "mrb_select_actions")
+           "mrb_select_actions", "mrb_record_begin", "mrb_record_step")
 
 
 class Spawn(C.Structure):
@@ -76,6 +76,12 @@ class SelectDesc(C.Structure):
                 ("eps_start", C.c_double), ("eps_finish", C.c_double), ("anneal_time", C.c_int64)]
 
 
+class EpisodeBatchDesc(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ("struct_size", "episode_limit", "obs_width", "reserved0")] + \
+        [(n, C.c_void_p) for n in ("obs", "state", "actions", "actions_onehot", "avail_actions", "reward", "terminated",
+                                   "filled", "cursor")]
+
+
 _lib = None
 
 
@@ -111,6 +117,8 @@ def load():
         "mrb_policy_last_error": ([vp], C.c_char_p),
         "mrb_policy_act": ([vp, i64, vp, vp, vp, vp, vp, vp], C.c_int),
         "mrb_select_actions": ([C.c_int, i64, i32, i32, C.POINTER(SelectDesc), vp, vp, vp, vp], C.c_int),
+        "mrb_record_begin": ([vp, C.POINTER(EpisodeBatchDesc), vp], C.c_int),
+        "mrb_record_step": ([vp, C.POINTER(EpisodeBatchDesc), vp, vp], C.c_int),
     }
     for name, (args, res) in sig.items():
         f = getattr(L, name)

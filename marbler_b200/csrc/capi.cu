@@ -140,6 +140,8 @@ extern "C" int mrb_destroy(mrb_env *env)
     return MRB_OK;
 }
 
+static int num_actions_of(const mrb_config &c) { return c.scenario == MRB_MATERIAL ? 20 : 5; }
+
 extern "C" int mrb_state_rows(const mrb_env *env, int32_t *rf, int32_t *ri)
 {
     if (!env || !rf || !ri) return MRB_E_ARG;
@@ -150,7 +152,7 @@ extern "C" int mrb_obs_dim(const mrb_env *env) { return env ? env->p.obs_dim : M
 extern "C" int mrb_num_actions(const mrb_env *env)
 {
     if (!env) return MRB_E_ARG;
-    return env->p.cfg.scenario == MRB_MATERIAL ? 20 : 5;     // spaces.Discrete(20) MaterialTransport.py:80, Discrete(5) elsewhere
+    return num_actions_of(env->p.cfg);     // spaces.Discrete(20) MaterialTransport.py:80, Discrete(5) elsewhere
 }
 
 extern "C" int mrb_bind(mrb_env *env, const mrb_buffers *b)
@@ -359,4 +361,54 @@ extern "C" int mrb_select_actions(int device, int64_t num_envs, int32_t n_agents
     if (st != cudaSuccess) return cuda_fail(nullptr, st, "select kernel launch");
     g_launches += 2;
     return MRB_OK;
+}
+
+// Everything mrb_record_begin / mrb_record_step check before they touch the device.
+static int check_episode_batch(mrb_env *env, const mrb_episode_batch *b, const char *fn)
+{
+    const std::string f(fn);
+    if (!env) return fail(nullptr, MRB_E_ARG, f + ": env is NULL");
+    if (!b) return fail(env, MRB_E_ARG, f + ": batch is NULL");
+    if (b->struct_size != (int32_t)sizeof(mrb_episode_batch))
+        return fail(env, MRB_E_ARG, f + ": mrb_episode_batch.struct_size does not match this library (ABI mismatch)");
+    if (!b->obs || !b->state || !b->actions || !b->actions_onehot || !b->avail_actions || !b->reward || !b->terminated ||
+        !b->filled || !b->cursor)
+        return fail(env, MRB_E_ARG, f + ": every pointer of mrb_episode_batch is required");
+    if (b->state != b->obs) return fail(env, MRB_E_ARG, f + ": state must be obs (state = concat(obs), the same memory)");
+    if (b->episode_limit < 1 || b->episode_limit > (1 << 30))
+        return fail(env, MRB_E_ARG, f + ": episode_limit must be in [1, 2^30]");
+    if (b->obs_width < env->p.obs_dim || b->obs_width > 65536)
+        return fail(env, MRB_E_ARG, f + ": obs_width must be in [obs_dim, 65536]");
+    // the kernel's accesses are scalar, each at its element's width
+    if ((((uintptr_t)b->actions | (uintptr_t)b->filled) & 7) ||
+        (((uintptr_t)b->obs | (uintptr_t)b->actions_onehot | (uintptr_t)b->avail_actions | (uintptr_t)b->reward |
+          (uintptr_t)b->cursor) & 3))
+        return fail(env, MRB_E_ARG, f + ": actions and filled must be 8-byte aligned, obs, actions_onehot, avail_actions, "
+                                        "reward and cursor 4-byte aligned");
+    if (!env->bound) return fail(env, MRB_E_STATE, f + ": call mrb_bind first");
+    return MRB_OK;
+}
+
+static int record(mrb_env *env, const mrb_episode_batch *b, bool begin, const int32_t *actions, void *stream)
+{
+    cudaError_t st = cudaSetDevice(env->device);
+    if (st != cudaSuccess) return cuda_fail(env, st, "cudaSetDevice");
+    if ((st = launch_record(env->p, num_actions_of(env->p.cfg), *b, begin, actions, (cudaStream_t)stream)) != cudaSuccess)
+        return cuda_fail(env, st, "record kernel launch");
+    g_launches++;
+    return MRB_OK;
+}
+
+extern "C" int mrb_record_begin(mrb_env *env, const mrb_episode_batch *batch, void *stream)
+{
+    const int rc = check_episode_batch(env, batch, "mrb_record_begin");
+    return rc != MRB_OK ? rc : record(env, batch, true, nullptr, stream);
+}
+
+extern "C" int mrb_record_step(mrb_env *env, const mrb_episode_batch *batch, const int32_t *actions, void *stream)
+{
+    int rc = check_episode_batch(env, batch, "mrb_record_step");
+    if (rc != MRB_OK) return rc;
+    if (!actions || ((uintptr_t)actions & 3)) return fail(env, MRB_E_ARG, "mrb_record_step: actions must be a 4-byte aligned device pointer");
+    return record(env, batch, false, actions, stream);
 }

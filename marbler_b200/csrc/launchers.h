@@ -27,4 +27,7 @@ cudaError_t launch_barrier_qp(int N, int barrier_default, int64_t B, const doubl
 // explore.cu: the selection kernel, then a one-thread kernel that advances *step
 cudaError_t launch_select_actions(int64_t num_envs, int32_t n_agents, int32_t n_actions, const mrb_select_desc &desc,
                                   int64_t *step, const float *q, int32_t *actions, cudaStream_t s);
+// record.cu: mrb_record_begin (begin, actions unused) and mrb_record_step, one launch each
+cudaError_t launch_record(const Params &p, int n_actions, const mrb_episode_batch &batch, bool begin,
+                          const int32_t *actions, cudaStream_t s);
 }  // namespace mrb

@@ -16,6 +16,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from .config import obs_space_dim
 
 
 def _ptr(t):
@@ -170,6 +171,64 @@ class Exploration(object):
         return max(self.eps_finish, self.eps_start - (self.eps_start - self.eps_finish) * t / self.anneal_time)
 
 
+class EpisodeBatch(object):
+    """EPyMARL's EpisodeBatch for one runner batch of `vec_env`, filled on the device (mrb_record_begin /
+    mrb_record_step, csrc/record.cu; the exact contract is in include/marbler_b200.h).
+
+    Each env records one episode from row 0, as ParallelRunner.reset() and run() do: row 0 holds the zero reset
+    observation.  Step t writes into row t the actions sent, the team reward (float32 sum over agents in index order)
+    and terminated (the env's own done or the time limit: truncation counts as terminal, since the gym wrapper reports
+    no episode_limit info), and into row t + 1 the observation after the step.  `filled` marks rows 0 .. terminal; every
+    other element is zero, the actions of the terminal row included (ParallelRunner also selects an action there,
+    which the learners' masks drop).  `obs_width` (default: the declared observation width, what
+    `GymmaVecEnv.get_obs_size()` returns) pads each agent's observation with zeros.
+
+    `data` is EPyMARL's scheme: obs [B,T+1,N,W] f32, state [B,T+1,N*W] (a view of obs), actions [B,T+1,N,1] i64,
+    actions_onehot [B,T+1,N,A] f32, avail_actions [B,T+1,N,A] i32, reward / terminated / filled [B,T+1,1] as f32 /
+    u8 / i64.  `cursor` [B] is the recorder's per-env position."""
+
+    def __init__(self, vec_env, episode_limit, obs_width=None):
+        self.env, self.lib = vec_env, _lib.load()
+        B, N, A, dev = vec_env.B, vec_env.N, vec_env.n_actions, vec_env.device
+        self.episode_limit = T = int(episode_limit)
+        self.obs_width = W = obs_space_dim(vec_env.scenario, vec_env.cfg, vec_env.c) if obs_width is None else int(obs_width)
+        self.obs = torch.zeros((B, T + 1, N, W), dtype=torch.float32, device=dev)
+        self.actions = torch.zeros((B, T + 1, N, 1), dtype=torch.int64, device=dev)
+        self.actions_onehot = torch.zeros((B, T + 1, N, A), dtype=torch.float32, device=dev)
+        self.avail_actions = torch.zeros((B, T + 1, N, A), dtype=torch.int32, device=dev)
+        self.reward = torch.zeros((B, T + 1, 1), dtype=torch.float32, device=dev)
+        self.terminated = torch.zeros((B, T + 1, 1), dtype=torch.uint8, device=dev)
+        self.filled = torch.zeros((B, T + 1, 1), dtype=torch.int64, device=dev)
+        self.cursor = torch.zeros((B,), dtype=torch.int32, device=dev)
+        self.desc = _lib.EpisodeBatchDesc(C.sizeof(_lib.EpisodeBatchDesc), T, W, 0, *[t.data_ptr() for t in (
+            self.obs, self.obs, self.actions, self.actions_onehot, self.avail_actions, self.reward, self.terminated,
+            self.filled, self.cursor)])
+
+    @property
+    def data(self):
+        B, R, N, W = self.obs.shape
+        return {"obs": self.obs, "state": self.obs.view(B, R, N * W), "actions": self.actions,
+                "actions_onehot": self.actions_onehot, "avail_actions": self.avail_actions, "reward": self.reward,
+                "terminated": self.terminated, "filled": self.filled}
+
+    def _stream(self):
+        return C.c_void_p(torch.cuda.current_stream(self.env.device).cuda_stream)
+
+    def begin(self):
+        """Row 0 of every env (and the zero row T of actions, reward and terminated); cursors to 0.  One launch."""
+        with torch.cuda.device(self.env.device):
+            _lib.check(self.lib.mrb_record_begin(self.env.handle, C.byref(self.desc), self._stream()), self.env.handle)
+
+    def record(self, actions):
+        """Record the step the env just took with `actions` (i32 [B,N] on the device).  One launch, stream-ordered;
+        after `episode_limit` calls further ones write nothing."""
+        assert actions.dtype == torch.int32 and actions.is_contiguous() and actions.device == self.env.device
+        assert tuple(actions.shape) == (self.env.B, self.env.N)
+        with torch.cuda.device(self.env.device):
+            _lib.check(self.lib.mrb_record_step(self.env.handle, C.byref(self.desc), _ptr(actions), self._stream()),
+                       self.env.handle)
+
+
 class Rollout(object):
     """run_env's loop for a whole batch, on the device: act -> step -> act -> ...  (misc.py:155-187).
 
@@ -178,9 +237,12 @@ class Rollout(object):
 
     `explore`: an `Exploration` that selects the actions of every step after the policy (its counter advances inside
     the captured graph too, and `reset` does not rewind it: the schedule runs across episodes).  When its `env_id0` is
-    None it takes the env's own, so that the ranks of a sharded run draw distinct streams."""
+    None it takes the env's own, so that the ranks of a sharded run draw distinct streams.
 
-    def __init__(self, vec_env, policy, use_graph=True, steps_per_graph=8, explore=None):
+    `record`: an `EpisodeBatch` of the same env that records every step after it is taken (one more launch per step,
+    captured in the graph too); `collect()` then fills it with one runner batch."""
+
+    def __init__(self, vec_env, policy, use_graph=True, steps_per_graph=8, explore=None, record=None):
         assert vec_env.N == policy.n_agents and vec_env.D == policy.obs_dim and vec_env.device == policy.device
         assert vec_env.n_actions == policy.n_actions, "policy and scenario disagree on the number of actions"
         self.env, self.policy = vec_env, policy
@@ -193,6 +255,8 @@ class Rollout(object):
                 explore.env_id0 = vec_env.env_id0
             if explore.mode == "softmax":
                 self.q = torch.zeros((vec_env.B, vec_env.N, policy.n_actions), dtype=torch.float32, device=vec_env.device)
+        assert record is None or record.env is vec_env, "the EpisodeBatch must belong to the rollout's env"
+        self.record = record
         self.use_graph, self.steps_per_graph = use_graph, int(steps_per_graph)
         self._graph = None
 
@@ -204,9 +268,23 @@ class Rollout(object):
     def _one(self):
         self.policy.act(self.env.obs, self.hidden, actions=self.actions, q=self.q, fresh=self.env.done, explore=self.explore)
         self.env.step(self.actions)
+        if self.record is not None:
+            self.record.record(self.actions)
+
+    def collect(self):
+        """One EPyMARL runner batch into `record`: mrb_record_begin, `reset()`, then exactly episode_limit env steps,
+        so every env records one episode and the result is the same with or without the graph (the auto-resets of
+        envs that finish early included).  No host synchronisation.  Returns `record.data`."""
+        if self.record is None:
+            raise ValueError("Rollout.collect needs record=EpisodeBatch(...)")
+        self.record.begin()
+        self.reset()
+        self.run(self.record.episode_limit)
+        return self.record.data
 
     def run(self, steps):
-        """Advance every env by `steps` env steps (2 kernels per step, 4 with `explore`; no host synchronisation)."""
+        """Advance every env by `steps` env steps (2 kernels per step, 4 with `explore`, one more with `record`; no
+        host synchronisation)."""
         k = self.steps_per_graph
         if self.use_graph:
             if self._graph is None and steps > k:
