@@ -17,7 +17,7 @@
 extern "C" {
 #endif
 
-#define MRB_ABI_VERSION 4
+#define MRB_ABI_VERSION 5
 #define MRB_MAX_ROBOTS 32
 #define MRB_MAX_PREY 32
 
@@ -198,9 +198,20 @@ typedef struct mrb_policy_desc {
 typedef struct mrb_policy mrb_policy;
 /* weights: HOST float32, (non_shared ? n_agents : 1) sets back to back, each set in state_dict order and
  * torch layout ([out][in] row-major): fc1.weight, fc1.bias, then rnn.weight_ih [3H][H], rnn.weight_hh [3H][H],
- * rnn.bias_ih, rnn.bias_hh (use_rnn) or rnn.weight [H][H], rnn.bias (otherwise), then fc2.weight, fc2.bias. */
+ * rnn.bias_ih, rnn.bias_hh (use_rnn) or rnn.weight [H][H], rnn.bias (otherwise), then fc2.weight, fc2.bias.
+ * Synchronous: uploads the weights to a temporary device buffer and builds the policy's images from it with the
+ * kernel mrb_policy_load launches, on the legacy default stream. */
 int mrb_policy_create(const mrb_policy_desc *desc, int device, const float *weights, int64_t num_weights,
                       mrb_policy **out);
+/* Replace the weights of `policy` in place (EPyMARL's mac.load_state: the collecting policy follows the learner).
+ * weights: DEVICE float32 on the policy's device, num_weights = the count mrb_policy_create took, same order.  Rebuilds
+ * every image the policy holds on cuda_stream: one launch, no allocation, no host copy, no synchronisation; capturable
+ * in a CUDA graph.  Graphs that captured mrb_policy_act on this policy stay valid and see the new weights at their next
+ * replay.  Ordered after the work already on cuda_stream; the caller orders other streams (e.g. a learner's) before it,
+ * and keeps `weights` unchanged until the launch has run.  Every argument is checked before the device is touched: a
+ * NULL policy or weights, another count, weights that are not 4-byte aligned or not device memory of the policy's
+ * device (cudaPointerGetAttributes) -> MRB_E_ARG, and the policy's images are untouched. */
+int mrb_policy_load(mrb_policy *policy, const float *weights, int64_t num_weights, void *cuda_stream);
 int mrb_policy_destroy(mrb_policy *policy);
 const char *mrb_policy_last_error(const mrb_policy *policy);
 /* obs f32 [B][N][D], hidden f32 [B][N][H] (in/out), actions i32 [B][N] (out), q f32 [B][N][n_actions] (out,

@@ -5,14 +5,14 @@ import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MARBLER_B200_LIB") or os.path.join(HERE, "libmarbler_b200.so")
-ABI_VERSION = 4
+ABI_VERSION = 5
 NUM_STATS = 16
 STAT_NAMES = ("episodes", "return_sum", "length_sum", "collisions", "boundary_exits", "scenario_metric",
               "env_steps", "qp_solves", "qp_iterations", "timeouts", "qp_stalls", "substeps", "qp_iterations_warp")
 SYMBOLS = ("mrb_version", "mrb_create", "mrb_destroy", "mrb_last_error", "mrb_state_rows", "mrb_obs_dim",
            "mrb_num_actions", "mrb_bind", "mrb_reset", "mrb_step", "mrb_step_host", "mrb_barrier_qp",
            "mrb_get_state", "mrb_set_state", "mrb_fp64_peak", "mrb_launch_count", "mrb_policy_create", "mrb_policy_destroy", "mrb_policy_last_error", "mrb_policy_act",
-           "mrb_select_actions", "mrb_record_begin", "mrb_record_step")
+           "mrb_policy_load", "mrb_select_actions", "mrb_record_begin", "mrb_record_step")
 
 
 class Spawn(C.Structure):
@@ -116,6 +116,7 @@ def load():
         "mrb_policy_destroy": ([vp], C.c_int),
         "mrb_policy_last_error": ([vp], C.c_char_p),
         "mrb_policy_act": ([vp, i64, vp, vp, vp, vp, vp, vp], C.c_int),
+        "mrb_policy_load": ([vp, vp, i64, vp], C.c_int),
         "mrb_select_actions": ([C.c_int, i64, i32, i32, C.POINTER(SelectDesc), vp, vp, vp, vp], C.c_int),
         "mrb_record_begin": ([vp, C.POINTER(EpisodeBatchDesc), vp], C.c_int),
         "mrb_record_step": ([vp, C.POINTER(EpisodeBatchDesc), vp, vp], C.c_int),

@@ -216,4 +216,21 @@ __device__ __forceinline__ double tree_max(double (&v)[M])
     return v[0];
 }
 
+// ---- one weight set of mrb_policy_create / mrb_policy_load: state_dict order, torch layout ([out][in] row-major)
+// (include/marbler_b200.h).  Without a GRU, wih / bih are rnn.weight / rnn.bias and whh / bhh are unused.
+__host__ __device__ inline int64_t weight_set_floats(int H, int Din, int A, bool rnn)
+{
+    return (int64_t)H * Din + H + (rnn ? 2LL * 3 * H * H + 2 * 3 * H : (int64_t)H * H + H) + (int64_t)A * H + A;
+}
+struct WeightSet {
+    const float *fc1w, *fc1b, *wih, *whh, *bih, *bhh, *fc2w, *fc2b;
+    __host__ __device__ WeightSet(const float *w, int H, int Din, int A, bool rnn)
+    {
+        fc1w = w; fc1b = fc1w + (size_t)H * Din; wih = fc1b + H;
+        if (rnn) { whh = wih + (size_t)3 * H * H; bih = whh + (size_t)3 * H * H; bhh = bih + 3 * H; fc2w = bhh + 3 * H; }
+        else { whh = nullptr; bih = wih + (size_t)H * H; bhh = nullptr; fc2w = bih + H; }
+        fc2b = fc2w + (size_t)A * H;
+    }
+};
+
 }  // namespace mrb

@@ -12,8 +12,8 @@
 // shared-memory loads, profiles/r01_ncu_policy_tf32.txt).  The activations never leave registers: the
 // accumulator fragments of two adjacent 16x8 output tiles ARE the A fragment of the next layer's 16x16
 // k-tile (no shuffles), the hidden state is loaded once as A fragments, and fc2 is accumulated as the GRU
-// produces h'.  Weights are rounded to FP16 and laid out in fragment order ONCE on the host
-// (mrb_policy_create), so staging them is a linear cp.async copy and every B fragment pair is a single
+// produces h'.  Weights are rounded to FP16 and laid out in fragment order once, on the device (policy_pack_kernel, at
+// mrb_policy_create and mrb_policy_load), so staging them is a linear cp.async copy and every B fragment pair is a single
 // conflict-free 128-bit shared load; the GRU weights (6 H^2 halves, 197 KB for H = 128) stream through a
 // double-buffered 2 x 12.3 KB window, one 8-unit column tile at a time.
 #include <cmath>
@@ -21,7 +21,6 @@
 #include <cstring>
 #include <new>
 #include <string>
-#include <vector>
 
 #include <cuda_fp16.h>
 
@@ -283,6 +282,88 @@ policy_act_kernel(const PolicyParams p, const float *obs, float *hidden, int32_t
     }
 }
 
+// ---- weight images, built on the device from the state_dict-order weights (mrb_policy_create, mrb_policy_load)
+//
+// B fragment word of W' (W torch layout [out][in]; rows >= rows_valid and columns >= cols_valid read as zero) for 8-column
+// tile j, 16-wide k-step s, lane (g, t): half 0 is b0 = {W[r][16s+2t], W[r][16s+2t+1]}, half 1 is b1 = the same 8 columns
+// on, r = row0 + 8j + g, each pair rounded to FP16 and packed low | high
+__device__ __forceinline__ uint32_t frag_word(const float *W, int ld, int row0, int rows_valid, int cols_valid, int j, int s,
+                                              int lane, int half)
+{
+    const int r = 8 * j + (lane >> 2), k = 16 * s + 2 * (lane & 3) + 8 * half;
+    auto at = [&](int c) { return (r < rows_valid && c < cols_valid) ? W[(size_t)(row0 + r) * ld + c] : 0.f; };
+    return pack_h2(at(k), at(k + 1));
+}
+
+// Word o of the image of one weight set (PolicyParams::set_floats words), in the order policy_act_kernel stages it:
+//   head (head_floats words): W1 fragments [NT][KS1][32 lanes][b0, b1] | b1 [H] | biases (b_ih | b_hh, or b) [NB] |
+//   W2 fragments [AT][KS][32][b0, b1] | b2 [AT * 8] (zero past n_actions);
+//   then per 8-unit column tile j of the recurrent layer a chunk [G][KS / 2][32][4]: gate matrix gi (W_ir, W_iz, W_in,
+//   W_hr, W_hz, W_hn; the Linear's W alone), k-step pair sp, lane, then (b0, b1) of k-step 2sp and of k-step 2sp + 1.
+__device__ __forceinline__ uint32_t wpack_word(const WeightSet &w, const PolicyParams &p, int H, bool rnn, int64_t o)
+{
+    const int Din = p.input_dim, A = p.n_actions, KS = H / 16;
+    if (o < p.szW1) {
+        const int js = (int)(o / 64);
+        return frag_word(w.fc1w, Din, 0, H, Din, js / p.KS1, js % p.KS1, (int)(o / 2) % 32, (int)(o & 1));
+    }
+    o -= p.szW1;
+    if (o < H) return __float_as_uint(w.fc1b[o]);
+    o -= H;
+    const int NB = rnn ? 6 * H : H;
+    if (o < NB) return __float_as_uint(o < 3 * H || !rnn ? w.bih[o] : w.bhh[o - 3 * H]);
+    o -= NB;
+    if (o < p.szW2) {
+        const int js = (int)(o / 64);
+        return frag_word(w.fc2w, H, 0, A, H, js / KS, js % KS, (int)(o / 2) % 32, (int)(o & 1));
+    }
+    o -= p.szW2;
+    if (o < 8 * p.AT) return __float_as_uint(o < A ? w.fc2b[o] : 0.f);
+    o -= 8 * p.AT;
+    const int chunk = (rnn ? 6 : 1) * KS * 64, j = (int)(o / chunk), c = (int)(o % chunk);
+    const int gi = (c / 128) / (KS / 2), sp = (c / 128) % (KS / 2), q = c % 4;
+    const float *W = rnn && gi >= 3 ? w.whh : w.wih;
+    return frag_word(W, H, rnn ? (gi % 3) * H : 0, H, H, j, 2 * sp + (q >> 1), (c / 4) % 32, q & 1);
+}
+
+// Every image a policy holds, back to back in one index space of 32-bit words: wpack, then tc2 (n_tc2 = 0 without one),
+// then w32 (n_w32 = 0 unless accurate).  Each thread writes one word, every word of every image.
+struct PackParams {
+    const float *w;                      // state_dict-order weights (device), `per_set` floats per set
+    int64_t per_set;
+    int32_t H, Din, A, rnn;
+    uint32_t *wpack, *tc2, *w32;
+    int64_t n_wpack, n_tc2, n_w32;       // words per image, all sets
+    int64_t tc2_set_words;
+    int32_t dp;
+    PolicyParams p;
+    f32::Params32 p32;
+};
+constexpr int kPackThreads = 256;
+
+__global__ void __launch_bounds__(kPackThreads) policy_pack_kernel(const PackParams k)
+{
+    int64_t i = (int64_t)blockIdx.x * kPackThreads + threadIdx.x;
+    const bool rnn = k.rnn != 0;
+    if (i < k.n_wpack) {
+        const int64_t set = i / k.p.set_floats;
+        k.wpack[i] = wpack_word(WeightSet(k.w + set * k.per_set, k.H, k.Din, k.A, rnn), k.p, k.H, rnn, i % k.p.set_floats);
+        return;
+    }
+    i -= k.n_wpack;
+    if (i < k.n_tc2) {
+        const int64_t set = i / k.tc2_set_words;
+        k.tc2[i] = tc2::image_word(WeightSet(k.w + set * k.per_set, k.H, k.Din, k.A, rnn), k.Din, k.A, k.dp, i % k.tc2_set_words);
+        return;
+    }
+    i -= k.n_tc2;
+    if (i < k.n_w32) {
+        const int64_t set = i / k.p32.set_floats;
+        k.w32[i] = __float_as_uint(f32::image_value(WeightSet(k.w + set * k.per_set, k.H, k.Din, k.A, rnn), k.p32, k.H, rnn,
+                                                    i % k.p32.set_floats));
+    }
+}
+
 }  // namespace mrb
 
 // ------------------------------------------------------------------------------------------------ host side
@@ -291,6 +372,7 @@ using namespace mrb;
 struct mrb_policy {
     mrb_policy_desc d;
     int device;
+    int64_t num_weights;        // the count mrb_policy_create took (mrb_policy_load takes the same)
     float *wpack;
     uint8_t *tc2_img;           // persistent tcgen05 path (policy_tc2.cuh), NULL when the model does not fit it
     mrb::tc2::Params2 tcp2;
@@ -300,6 +382,7 @@ struct mrb_policy {
     size_t smem_bytes;
     float *w32;                 // float32 path (policy_f32.cuh), only when desc.accurate
     mrb::f32::Params32 p32;
+    PackParams pack;            // policy_pack_kernel's arguments but the weights
     std::string err;
 };
 
@@ -312,22 +395,22 @@ static int pfail(mrb_policy *p, int code, const std::string &msg)
     return code;
 }
 
-// B fragment of W' for 8-column tile j, 16-wide k-step s (W in torch layout [out][in]; rows >= rows_valid and
-// columns >= cols_valid read as zero): lane (g, t) holds b0 = {W[r][16s+2t], W[r][16s+2t+1]} and
-// b1 = {W[r][16s+2t+8], W[r][16s+2t+9]} with r = row0 + 8j + g, each pair rounded to FP16 and packed low | high
-static uint32_t h2bits(float lo, float hi)
+// rebuilds every image of `pol` from the state_dict-order weights w (device): one launch on s
+static cudaError_t launch_pack(const mrb_policy *pol, const float *w, cudaStream_t s)
 {
-    const uint32_t a = __half_as_ushort(__float2half_rn(lo)), b = __half_as_ushort(__float2half_rn(hi));
-    return a | (b << 16);
+    PackParams k = pol->pack;
+    k.w = w;
+    const int64_t words = k.n_wpack + k.n_tc2 + k.n_w32;
+    policy_pack_kernel<<<(unsigned)((words + kPackThreads - 1) / kPackThreads), kPackThreads, 0, s>>>(k);
+    return cudaGetLastError();
 }
-static void frag(const float *W, int ld, int row0, int rows_valid, int cols_valid, int j, int s, int lane, float &b0, float &b1)
+
+static void free_images(mrb_policy *pol)
 {
-    const int g = lane >> 2, t = lane & 3, r = 8 * j + g;
-    auto at = [&](int k) { return (r < rows_valid && k < cols_valid) ? W[(size_t)(row0 + r) * ld + k] : 0.f; };
-    const int k0 = 16 * s + 2 * t;
-    const uint32_t u0 = h2bits(at(k0), at(k0 + 1)), u1 = h2bits(at(k0 + 8), at(k0 + 9));
-    std::memcpy(&b0, &u0, 4);
-    std::memcpy(&b1, &u1, 4);
+    if (pol->wpack) cudaFree(pol->wpack);
+    if (pol->tc2_img) cudaFree(pol->tc2_img);
+    if (pol->w32) cudaFree(pol->w32);
+    delete pol;
 }
 
 extern "C" const char *mrb_policy_last_error(const mrb_policy *p) { return p ? p->err.c_str() : g_policy_create_error.c_str(); }
@@ -348,7 +431,7 @@ extern "C" int mrb_policy_create(const mrb_policy_desc *desc, int device, const 
         return pfail(nullptr, MRB_E_ARG, "mrb_policy_create: input_dim must equal obs_dim (+ n_agents with obs_agent_id): "
                                          "these weights were trained on a different observation layout");
     const int sets = d.non_shared ? N : 1;
-    const int64_t per_set = (int64_t)H * Din + H + (d.use_rnn ? 2LL * 3 * H * H + 2 * 3 * H : (int64_t)H * H + H) + (int64_t)A * H + A;
+    const int64_t per_set = weight_set_floats(H, Din, A, d.use_rnn != 0);
     if (num_weights != per_set * sets)
         return pfail(nullptr, MRB_E_ARG, "mrb_policy_create: weight count does not match the descriptor");
     int ndev = 0;
@@ -359,173 +442,111 @@ extern "C" int mrb_policy_create(const mrb_policy_desc *desc, int device, const 
     if ((st = cudaGetDeviceProperties(&prop, device)) != cudaSuccess) return pfail(nullptr, MRB_E_CUDA, cudaGetErrorString(st));
     if (prop.major != 10) return pfail(nullptr, MRB_E_UNSUPPORTED, "mrb_policy_create: kernels are built for sm_100a (B200) only");
 
-    const int KS1 = (Din + 15) / 16, NT = H / 8, KS = H / 16, AT = (A + 7) / 8, G = d.use_rnn ? 6 : 1;
-    const int szW1 = NT * KS1 * 64, szW2 = AT * KS * 64, NB = d.use_rnn ? 6 * H : H;
-    const int head = szW1 + H + NB + szW2 + AT * 8;
-    const int chunk = G * KS * 64;
-    const int64_t set_floats = head + (int64_t)NT * chunk;
-    std::vector<float> img((size_t)set_floats * sets, 0.f);
-    for (int sidx = 0; sidx < sets; sidx++) {
-        const float *w = weights + per_set * sidx;
-        const float *fc1w = w, *fc1b = fc1w + (size_t)H * Din;
-        const float *rw = fc1b + H;
-        const float *wih = rw, *whh = nullptr, *bih = nullptr, *bhh = nullptr, *fc2w = nullptr;
-        if (d.use_rnn) { whh = wih + (size_t)3 * H * H; bih = whh + (size_t)3 * H * H; bhh = bih + 3 * H; fc2w = bhh + 3 * H; }
-        else { bih = wih + (size_t)H * H; fc2w = bih + H; }
-        const float *fc2b = fc2w + (size_t)A * H;
-        float *o = img.data() + (size_t)set_floats * sidx;
-        float *oW1 = o, *oB1 = oW1 + szW1, *oBias = oB1 + H, *oW2 = oBias + NB, *oB2 = oW2 + szW2, *oCh = o + head;
-        for (int j = 0; j < NT; j++)
-            for (int s = 0; s < KS1; s++)
-                for (int l = 0; l < 32; l++)
-                    frag(fc1w, Din, 0, H, Din, j, s, l, oW1[((j * KS1 + s) * 32 + l) * 2], oW1[((j * KS1 + s) * 32 + l) * 2 + 1]);
-        std::memcpy(oB1, fc1b, sizeof(float) * H);
-        if (d.use_rnn) { std::memcpy(oBias, bih, sizeof(float) * 3 * H); std::memcpy(oBias + 3 * H, bhh, sizeof(float) * 3 * H); }
-        else std::memcpy(oBias, bih, sizeof(float) * H);
-        for (int jt = 0; jt < AT; jt++)
-            for (int s = 0; s < KS; s++)
-                for (int l = 0; l < 32; l++)
-                    frag(fc2w, H, 0, A, H, jt, s, l, oW2[((jt * KS + s) * 32 + l) * 2], oW2[((jt * KS + s) * 32 + l) * 2 + 1]);
-        for (int a = 0; a < A; a++) oB2[a] = fc2b[a];
-        for (int j = 0; j < NT; j++)
-            for (int gi = 0; gi < G; gi++) {
-                const float *W = d.use_rnn ? (gi < 3 ? wih : whh) : wih;
-                const int row0 = d.use_rnn ? (gi % 3) * H : 0;
-                for (int sp = 0; sp < KS / 2; sp++)
-                    for (int l = 0; l < 32; l++) {
-                        float *q = oCh + (size_t)j * chunk + ((size_t)(gi * (KS / 2) + sp) * 32 + l) * 4;
-                        frag(W, H, row0, H, H, j, 2 * sp, l, q[0], q[1]);
-                        frag(W, H, row0, H, H, j, 2 * sp + 1, l, q[2], q[3]);
-                    }
-            }
-    }
-    // persistent tcgen05 path: head = W1 FP16 [128][dp + 8] | biases | W2 [A][128] as FP32 values rounded to FP16, then twelve
-    // 64 x 128 FP16 half slabs in the order the kernel consumes them (pass, gate r / z / n, W_ih then W_hh)
-    std::vector<uint8_t> tc2img;
-    mrb::tc2::Params2 tcp2;
-    std::memset(&tcp2, 0, sizeof(tcp2));
-    const int dp = (Din + 15) & ~15;
-    const size_t tc2_smem = mrb::tc2::smem_bytes(dp, A);
-    const bool use_tc2 = !d.accurate && H == 128 && d.use_rnn && dp <= mrb::tc::kMaxKp1 && A <= mrb::tc2::kMaxA && mrb::tc2::ring_depth(dp, A) >= 2;
-    // float32 path: transposed float32 copies of every matrix (policy_f32.cuh)
-    std::vector<float> img32;
-    mrb::f32::Params32 p32;
-    std::memset(&p32, 0, sizeof(p32));
-    if (d.accurate) {
-        const int64_t sf = mrb::f32::image_floats(H, Din, A, d.use_rnn != 0, &p32);
-        img32.assign((size_t)sf * sets, 0.f);
-        for (int sidx = 0; sidx < sets; sidx++) {
-            const float *w = weights + per_set * sidx;
-            const float *fc1w = w, *fc1b = fc1w + (size_t)H * Din, *rw = fc1b + H;
-            float *o = img32.data() + (size_t)sf * sidx;
-            for (int u = 0; u < H; u++)
-                for (int k = 0; k < Din; k++) o[(size_t)k * H + u] = fc1w[(size_t)u * Din + k];
-            std::memcpy(o + p32.off_b1, fc1b, sizeof(float) * H);
-            const float *fc2w;
-            if (d.use_rnn) {
-                const float *wih = rw, *whh = wih + (size_t)3 * H * H, *bih = whh + (size_t)3 * H * H, *bhh = bih + 3 * H;
-                for (int g = 0; g < 3; g++)
-                    for (int u = 0; u < H; u++)
-                        for (int k = 0; k < H; k++) {
-                            o[p32.off_wih + ((size_t)g * H + k) * H + u] = wih[((size_t)g * H + u) * H + k];
-                            o[p32.off_whh + ((size_t)g * H + k) * H + u] = whh[((size_t)g * H + u) * H + k];
-                        }
-                std::memcpy(o + p32.off_bias, bih, sizeof(float) * 3 * H);
-                std::memcpy(o + p32.off_bias + 3 * H, bhh, sizeof(float) * 3 * H);
-                fc2w = bhh + 3 * H;
-            } else {
-                const float *wl = rw, *bl = wl + (size_t)H * H;
-                for (int u = 0; u < H; u++)
-                    for (int k = 0; k < H; k++) o[p32.off_wih + (size_t)k * H + u] = wl[(size_t)u * H + k];
-                std::memcpy(o + p32.off_bias, bl, sizeof(float) * H);
-                fc2w = bl + H;
-            }
-            std::memcpy(o + p32.off_w2, fc2w, sizeof(float) * (size_t)A * H);
-            std::memcpy(o + p32.off_b2, fc2w + (size_t)A * H, sizeof(float) * A);
-        }
-        p32.set_floats = sf; p32.obs_dim = d.obs_dim; p32.input_dim = Din; p32.n_actions = A; p32.n_agents = N;
-        p32.obs_agent_id = d.obs_agent_id; p32.non_shared = d.non_shared;
-    }
-    if (use_tc2) {
-        const int headf = mrb::tc2::head_floats(dp, A);
-        const int64_t setb = 4LL * headf + (int64_t)mrb::tc2::kSlabsPerTile * mrb::tc2::kHalfSlabBytes;
-        tc2img.assign((size_t)setb * sets, 0);
-        auto r16 = [](float v) { return __half2float(__float2half_rn(v)); };
-        for (int sidx = 0; sidx < sets; sidx++) {
-            const float *w = weights + per_set * sidx;
-            const float *fc1w = w, *fc1b = fc1w + (size_t)H * Din, *wih = fc1b + H, *whh = wih + (size_t)3 * H * H;
-            const float *bih = whh + (size_t)3 * H * H, *bhh = bih + 3 * H, *fc2w = bhh + 3 * H, *fc2b = fc2w + (size_t)A * H;
-            uint8_t *o = tc2img.data() + (size_t)setb * sidx;
-            float *hf = reinterpret_cast<float *>(o);
-            __half *w1h = reinterpret_cast<__half *>(o);
-            for (int u = 0; u < H; u++)
-                for (int k = 0; k < Din; k++) w1h[(size_t)u * mrb::tc2::w1_stride(dp) + k] = __float2half_rn(fc1w[(size_t)u * Din + k]);
-            float *bo = hf + mrb::tc2::head_bias(dp);
-            std::memcpy(bo, fc1b, sizeof(float) * H);
-            std::memcpy(bo + H, bih, sizeof(float) * 3 * H);
-            std::memcpy(bo + 4 * H, bhh, sizeof(float) * 3 * H);
-            for (int a = 0; a < A; a++) bo[7 * H + a] = fc2b[a];
-            float *w2 = hf + mrb::tc2::head_w2(dp);
-            for (int a = 0; a < A; a++)
-                for (int k = 0; k < H; k++) w2[(size_t)a * H + k] = r16(fc2w[(size_t)a * H + k]);
-            uint8_t *slabs = o + 4 * (size_t)headf;
-            for (int pass = 0; pass < 2; pass++)
-                for (int g = 0; g < 6; g++)
-                    mrb::tc::pack_canonical(slabs + (size_t)(pass * 6 + g) * mrb::tc2::kHalfSlabBytes, (g & 1) ? whh : wih, H,
-                                            (g >> 1) * H + pass * mrb::tc2::kHalf, mrb::tc2::kHalf, H, mrb::tc2::kHalf, H);
-        }
-        tcp2.set_bytes = setb; tcp2.obs_dim = d.obs_dim; tcp2.input_dim = Din; tcp2.n_actions = A; tcp2.n_agents = N;
-        tcp2.obs_agent_id = d.obs_agent_id; tcp2.non_shared = d.non_shared; tcp2.dp = dp; tcp2.head_bytes = 4 * headf;
-        tcp2.ring_off = mrb::tc2::ring_offset(dp, A); tcp2.ring = mrb::tc2::ring_depth(dp, A);
-    }
     mrb_policy *pol = new (std::nothrow) mrb_policy();
     if (!pol) return pfail(nullptr, MRB_E_ARG, "mrb_policy_create: out of host memory");
     pol->d = d;
     pol->device = device;
+    pol->num_weights = num_weights;
     pol->wpack = nullptr;
     pol->tc2_img = nullptr;
-    pol->tcp2 = tcp2;
-    pol->tc2_smem = tc2_smem;
-    pol->num_sms = 0;
     pol->w32 = nullptr;
-    pol->p32 = p32;
-    if ((st = cudaSetDevice(device)) != cudaSuccess || (st = cudaMalloc(&pol->wpack, img.size() * sizeof(float))) != cudaSuccess ||
-        (st = cudaMemcpy(pol->wpack, img.data(), img.size() * sizeof(float), cudaMemcpyHostToDevice)) != cudaSuccess) {
-        const std::string msg = std::string("mrb_policy_create: ") + cudaGetErrorString(st);
-        if (pol->wpack) cudaFree(pol->wpack);
-        delete pol;
-        return pfail(nullptr, MRB_E_CUDA, msg);
-    }
-    if (use_tc2) {
-        if ((st = cudaMalloc(&pol->tc2_img, tc2img.size())) != cudaSuccess ||
-            (st = cudaMemcpy(pol->tc2_img, tc2img.data(), tc2img.size(), cudaMemcpyHostToDevice)) != cudaSuccess ||
-            (st = cudaDeviceGetAttribute(&pol->num_sms, cudaDevAttrMultiProcessorCount, device)) != cudaSuccess) {
-            const std::string msg = std::string("mrb_policy_create: ") + cudaGetErrorString(st);
-            if (pol->tc2_img) cudaFree(pol->tc2_img);
-            cudaFree(pol->wpack);
-            delete pol;
-            return pfail(nullptr, MRB_E_CUDA, msg);
-        }
-        pol->tcp2.img = pol->tc2_img;
-    }
-    if (d.accurate) {
-        if ((st = cudaMalloc(&pol->w32, img32.size() * sizeof(float))) != cudaSuccess ||
-            (st = cudaMemcpy(pol->w32, img32.data(), img32.size() * sizeof(float), cudaMemcpyHostToDevice)) != cudaSuccess) {
-            const std::string msg = std::string("mrb_policy_create: ") + cudaGetErrorString(st);
-            if (pol->w32) cudaFree(pol->w32);
-            cudaFree(pol->wpack);
-            delete pol;
-            return pfail(nullptr, MRB_E_CUDA, msg);
-        }
-        pol->p32.w = pol->w32;
-    }
+    pol->num_sms = 0;
+
+    // mma.sync path (policy_act_kernel, wpack_word)
+    const int KS1 = (Din + 15) / 16, NT = H / 8, KS = H / 16, AT = (A + 7) / 8, G = d.use_rnn ? 6 : 1;
+    const int szW1 = NT * KS1 * 64, szW2 = AT * KS * 64, NB = d.use_rnn ? 6 * H : H;
+    const int head = szW1 + H + NB + szW2 + AT * 8;
+    const int chunk = G * KS * 64;
     PolicyParams &p = pol->p;
-    p.wpack = pol->wpack; p.set_floats = set_floats; p.B = 0;
+    p.set_floats = head + (int64_t)NT * chunk; p.B = 0;
     p.obs_dim = d.obs_dim; p.input_dim = Din; p.n_actions = A; p.n_agents = N;
     p.obs_agent_id = d.obs_agent_id; p.non_shared = d.non_shared;
     p.KS1 = KS1; p.AT = AT; p.szW1 = szW1; p.szW2 = szW2; p.head_floats = head;
     pol->smem_bytes = sizeof(float) * ((size_t)head + 2 * (size_t)chunk);
+
+    // persistent tcgen05 path (policy_tc2.cuh image_word)
+    mrb::tc2::Params2 &tcp2 = pol->tcp2;
+    std::memset(&tcp2, 0, sizeof(tcp2));
+    const int dp = (Din + 15) & ~15;
+    pol->tc2_smem = mrb::tc2::smem_bytes(dp, A);
+    const bool use_tc2 = !d.accurate && H == 128 && d.use_rnn && dp <= mrb::tc::kMaxKp1 && A <= mrb::tc2::kMaxA && mrb::tc2::ring_depth(dp, A) >= 2;
+    if (use_tc2) {
+        const int headf = mrb::tc2::head_floats(dp, A);
+        tcp2.set_bytes = 4LL * headf + (int64_t)mrb::tc2::kSlabsPerTile * mrb::tc2::kHalfSlabBytes;
+        tcp2.obs_dim = d.obs_dim; tcp2.input_dim = Din; tcp2.n_actions = A; tcp2.n_agents = N;
+        tcp2.obs_agent_id = d.obs_agent_id; tcp2.non_shared = d.non_shared; tcp2.dp = dp; tcp2.head_bytes = 4 * headf;
+        tcp2.ring_off = mrb::tc2::ring_offset(dp, A); tcp2.ring = mrb::tc2::ring_depth(dp, A);
+    }
+
+    // float32 path (policy_f32.cuh image_value)
+    mrb::f32::Params32 &p32 = pol->p32;
+    std::memset(&p32, 0, sizeof(p32));
+    if (d.accurate) {
+        p32.set_floats = mrb::f32::image_floats(H, Din, A, d.use_rnn != 0, &p32);
+        p32.obs_dim = d.obs_dim; p32.input_dim = Din; p32.n_actions = A; p32.n_agents = N;
+        p32.obs_agent_id = d.obs_agent_id; p32.non_shared = d.non_shared;
+    }
+
+    PackParams &k = pol->pack;
+    std::memset(&k, 0, sizeof(k));
+    k.per_set = per_set; k.H = H; k.Din = Din; k.A = A; k.rnn = d.use_rnn != 0;
+    k.n_wpack = p.set_floats * sets;
+    k.n_tc2 = use_tc2 ? tcp2.set_bytes / 4 * sets : 0;
+    k.n_w32 = d.accurate ? p32.set_floats * sets : 0;
+    k.tc2_set_words = tcp2.set_bytes / 4; k.dp = dp;
+    k.p = p; k.p32 = p32;
+
+    // images, then the weights uploaded once to a temporary buffer that the pack kernel reads; synchronous
+    float *wdev = nullptr;
+    if ((st = cudaSetDevice(device)) != cudaSuccess ||
+        (st = cudaMalloc(&pol->wpack, sizeof(float) * k.n_wpack)) != cudaSuccess ||
+        (use_tc2 && (st = cudaMalloc(&pol->tc2_img, 4 * k.n_tc2)) != cudaSuccess) ||
+        (use_tc2 && (st = cudaDeviceGetAttribute(&pol->num_sms, cudaDevAttrMultiProcessorCount, device)) != cudaSuccess) ||
+        (d.accurate && (st = cudaMalloc(&pol->w32, sizeof(float) * k.n_w32)) != cudaSuccess) ||
+        (st = cudaMalloc(&wdev, sizeof(float) * num_weights)) != cudaSuccess ||
+        (st = cudaMemcpy(wdev, weights, sizeof(float) * num_weights, cudaMemcpyHostToDevice)) != cudaSuccess) {
+        const std::string msg = std::string("mrb_policy_create: ") + cudaGetErrorString(st);
+        if (wdev) cudaFree(wdev);
+        free_images(pol);
+        return pfail(nullptr, MRB_E_CUDA, msg);
+    }
+    k.wpack = reinterpret_cast<uint32_t *>(pol->wpack);
+    k.tc2 = reinterpret_cast<uint32_t *>(pol->tc2_img);
+    k.w32 = reinterpret_cast<uint32_t *>(pol->w32);
+    p.wpack = pol->wpack;
+    tcp2.img = pol->tc2_img;
+    p32.w = pol->w32;
+    if ((st = launch_pack(pol, wdev, 0)) != cudaSuccess || (st = cudaStreamSynchronize(0)) != cudaSuccess) {
+        const std::string msg = std::string("mrb_policy_create: weight packing: ") + cudaGetErrorString(st);
+        cudaFree(wdev);
+        free_images(pol);
+        return pfail(nullptr, MRB_E_CUDA, msg);
+    }
+    count_launch();
+    cudaFree(wdev);
     *out = pol;
+    return MRB_OK;
+}
+
+extern "C" int mrb_policy_load(mrb_policy *pol, const float *weights, int64_t num_weights, void *stream)
+{
+    if (!pol) return pfail(nullptr, MRB_E_ARG, "mrb_policy_load: null policy");
+    if (!weights) return pfail(pol, MRB_E_ARG, "mrb_policy_load: null weights");
+    if (num_weights != pol->num_weights)
+        return pfail(pol, MRB_E_ARG, "mrb_policy_load: " + std::to_string(num_weights) + " weights given, the policy was created with " +
+                                     std::to_string(pol->num_weights));
+    if (((uintptr_t)weights & 3) != 0) return pfail(pol, MRB_E_ARG, "mrb_policy_load: weights must be 4-byte aligned");
+    cudaPointerAttributes attr;
+    cudaError_t st = cudaPointerGetAttributes(&attr, weights);
+    if (st != cudaSuccess) {
+        cudaGetLastError();
+        return pfail(pol, MRB_E_ARG, std::string("mrb_policy_load: weights: ") + cudaGetErrorString(st));
+    }
+    if (attr.type != cudaMemoryTypeDevice || attr.device != pol->device)
+        return pfail(pol, MRB_E_ARG, "mrb_policy_load: weights must be device memory of the policy's device " + std::to_string(pol->device));
+    if ((st = cudaSetDevice(pol->device)) != cudaSuccess || (st = launch_pack(pol, weights, (cudaStream_t)stream)) != cudaSuccess)
+        return pfail(pol, MRB_E_CUDA, std::string("mrb_policy_load: ") + cudaGetErrorString(st));
+    count_launch();
     return MRB_OK;
 }
 
@@ -533,10 +554,7 @@ extern "C" int mrb_policy_destroy(mrb_policy *p)
 {
     if (!p) return MRB_E_ARG;
     cudaSetDevice(p->device);
-    if (p->wpack) cudaFree(p->wpack);
-    if (p->tc2_img) cudaFree(p->tc2_img);
-    if (p->w32) cudaFree(p->w32);
-    delete p;
+    free_images(p);
     return MRB_OK;
 }
 

@@ -46,6 +46,24 @@ inline int64_t image_floats(int H, int Din, int A, bool rnn, Params32 *p)
     return o;
 }
 
+// float o of the image of one weight set (layout above), built on the device by policy_pack_kernel (policy.cu)
+__device__ __forceinline__ float image_value(const WeightSet &w, const Params32 &p, int H, bool rnn, int64_t o)
+{
+    if (o < p.off_b1) return w.fc1w[(size_t)(o % H) * p.input_dim + o / H];
+    if (o < p.off_wih) return w.fc1b[o - p.off_b1];
+    if (o < p.off_bias) {                                           // (gate, k, unit) <- [gate * H + unit][k]
+        const bool hh = o >= p.off_whh;
+        const int64_t i = o - (hh ? p.off_whh : p.off_wih), g = i / ((int64_t)H * H), k = (i / H) % H, u = i % H;
+        return (hh ? w.whh : w.wih)[(size_t)(g * H + u) * H + k];
+    }
+    if (o < p.off_w2) {
+        const int i = (int)(o - p.off_bias);
+        return rnn && i >= 3 * H ? w.bhh[i - 3 * H] : w.bih[i];
+    }
+    if (o < p.off_b2) return w.fc2w[o - p.off_w2];
+    return w.fc2b[o - p.off_b2];
+}
+
 __device__ __forceinline__ float sigmoid_(float x) { return 1.f / (1.f + expf(-x)); }
 
 template <int H, bool RNN>

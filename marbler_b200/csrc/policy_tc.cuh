@@ -1,6 +1,6 @@
 // tcgen05 / TMEM / bulk-copy building blocks of the persistent policy kernel (policy_tc2.cuh): mbarrier and
 // cp.async.bulk wrappers, UMMA shared-memory / instruction descriptors, tcgen05.mma / commit / ld wrappers, the SFU
-// gate functions and the host-side packing of a weight matrix into the UMMA canonical layout.
+// gate functions.
 //
 // Canonical K-major layout, no swizzle (CUTLASS cute/atom/mma_traits_sm100.hpp "LayoutType::INTERLEAVE:
 // ((8,n),2):((1,SBO),LBO)" in 16-byte units): element (row r, k) of an operand with R rows lives at
@@ -87,18 +87,6 @@ __device__ __forceinline__ float ex2a(float x) { float y; asm("ex2.approx.ftz.f3
 __device__ __forceinline__ float rcpa(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ float sigm(float x) { return rcpa(1.f + ex2a(-1.4426950408889634f * x)); }
 __device__ __forceinline__ float tanh_(float x) { return fmaf(2.f, rcpa(1.f + ex2a(-2.8853900817779268f * x)), -1.f); }
-
-// ---- host: FP16 canonical images.  W is torch layout [out][in]; element (row r = output unit, k = input unit).
-inline void pack_canonical(uint8_t *dst, const float *W, int ld, int row0, int rows_valid, int cols_valid, int R, int K)
-{
-    const int lbo = R / 8 * 128;
-    for (int k = 0; k < K; k++)
-        for (int r = 0; r < R; r++) {
-            const float v = (r < rows_valid && k < cols_valid) ? W[(size_t)(row0 + r) * ld + k] : 0.f;
-            const uint16_t hbits = __half_as_ushort(__float2half_rn(v));
-            std::memcpy(dst + (size_t)(k / 8) * lbo + (r / 8) * 128 + (r % 8) * 16 + (k % 8) * 2, &hbits, 2);
-        }
-}
 
 }  // namespace tc
 }  // namespace mrb

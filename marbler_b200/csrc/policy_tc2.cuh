@@ -12,7 +12,7 @@
 //                      mma.sync.m16n8k16 (K <= 64: 1 % of the flops; a tcgen05 fc1 would need a MMA -> epilogue -> MMA
 //                      round trip per tile and TMEM columns that the two gate halves occupy); two activation buffers
 //   loader    1 thread streams the GRU weights as twelve 64 x 128 FP16 half slabs per tile (cp.async.bulk, 1-D: the
-//                      host packed them in the canonical layout) through a three-deep (two when shared memory is short) 16 KB ring
+//                      image holds them in the canonical layout, image_word) through a three-deep (two when shared memory is short) 16 KB ring
 //   mma       1 thread per tile two half passes of 64 hidden units; a pass is 6 slabs x 8 tcgen05.mma (M 128, N 64,
 //                      K 16) into one 256-column half of TMEM: r -> [0,64), z -> [64,128), W_in x -> [128,192),
 //                      W_hn h -> [192,256); tcgen05.commit releases slabs, activation buffers and TMEM halves
@@ -92,6 +92,35 @@ __host__ inline int ring_depth(int dp, int n_actions)
     return 0;
 }
 __host__ inline size_t smem_bytes(int dp, int n_actions) { return (size_t)ring_offset(dp, n_actions) + (size_t)ring_depth(dp, n_actions) * kHalfSlabBytes; }
+
+// Word o (4 bytes) of the image of one weight set, built on the device by policy_pack_kernel (policy.cu):
+//   head (head_floats words): W1 FP16 [128][dp + 8] (columns >= input_dim zero) | b1 | b_ih | b_hh | b2 [32] (zero past
+//   n_actions) | W2 [n_actions][128] as float32 values rounded to FP16;
+//   then twelve 64 x 128 FP16 half slabs in the order the kernel consumes them: pass p, gate r / z / n, W_ih then W_hh
+//   (slab 6p + g holds rows (g / 2) * 128 + 64p .. + 63 of (g odd ? W_hh : W_ih)), each in the canonical K-major layout
+//   of policy_tc.cuh with LBO = 64 / 8 * 128 = 1,024 bytes: element (r, k) at byte (k / 8) 1024 + (r / 8) 128 + (r % 8) 16 + (k % 8) 2.
+__device__ __forceinline__ uint32_t image_word(const WeightSet &w, int Din, int A, int dp, int64_t o)
+{
+    const int hb = head_bias(dp), hw = head_w2(dp), hf = head_floats(dp, A);
+    if (o < hb) {                                                   // W1 row u, columns k, k + 1 (dp + 8 is even)
+        const int ws = w1_stride(dp) / 2, u = (int)o / ws, k = 2 * ((int)o % ws);
+        const float *row = w.fc1w + (size_t)u * Din;
+        return h2(k < Din ? row[k] : 0.f, k + 1 < Din ? row[k + 1] : 0.f);
+    }
+    if (o < hw) {
+        const int i = (int)o - hb;
+        const float v = i < kH ? w.fc1b[i] : i < 4 * kH ? w.bih[i - kH] : i < 7 * kH ? w.bhh[i - 4 * kH]
+                      : (i - 7 * kH < A ? w.fc2b[i - 7 * kH] : 0.f);
+        return __float_as_uint(v);
+    }
+    if (o < hf) return __float_as_uint(__half2float(__float2half_rn(w.fc2w[o - hw])));
+    const int64_t b = 4 * (o - hf);
+    const int slab = (int)(b / kHalfSlabBytes), rem = (int)(b % kHalfSlabBytes), pass = slab / 6, g = slab % 6;
+    constexpr int lbo = kHalf / 8 * 128;
+    const int r = 8 * ((rem % lbo) / 128) + (rem % 128) / 16, k = 8 * (rem / lbo) + (rem % 16) / 2;
+    const float *W = ((g & 1) ? w.whh : w.wih) + (size_t)((g >> 1) * kH + pass * kHalf + r) * kH + k;
+    return h2(W[0], W[1]);
+}
 // D = A (16x16, row) * B (16x8, col) + D, FP16 inputs, FP32 accumulate
 __device__ __forceinline__ void mma_m16n8k16(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1)
 {

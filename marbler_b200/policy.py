@@ -27,24 +27,69 @@ def _is_ns(state_dict):
     return any(k.startswith("agents.") for k in state_dict)
 
 
+def _param_names(use_rnn):
+    """The parameters of one RNNAgent in mrb_policy_create's order (state_dict order, include/marbler_b200.h)."""
+    return ["fc1.weight", "fc1.bias"] + \
+        (["rnn.weight_ih", "rnn.weight_hh", "rnn.bias_ih", "rnn.bias_hh"] if use_rnn else ["rnn.weight", "rnn.bias"]) + \
+        ["fc2.weight", "fc2.bias"]
+
+
+def state_dict_keys(n_agents, non_shared, use_rnn):
+    """Every key of an RNNAgent (or, non_shared, RNNNSAgent) state_dict, in the order of the flat weights."""
+    prefixes = ["agents.%d." % i for i in range(n_agents)] if non_shared else [""]
+    return [p + n for p in prefixes for n in _param_names(use_rnn)]
+
+
 def flatten_state_dict(state_dict, n_agents):
     """state_dict of RNNAgent / RNNNSAgent -> (flat float32 array in mrb_policy_create's order, facts)."""
     sd = {k: np.asarray(v.detach().cpu().numpy() if hasattr(v, "detach") else v, dtype=np.float32)
           for k, v in state_dict.items()}
     ns = _is_ns(sd)
-    prefixes = ["agents.%d." % i for i in range(n_agents)] if ns else [""]
-    use_rnn = (prefixes[0] + "rnn.weight_ih") in sd
-    names = ["fc1.weight", "fc1.bias"] + \
-        (["rnn.weight_ih", "rnn.weight_hh", "rnn.bias_ih", "rnn.bias_hh"] if use_rnn else ["rnn.weight", "rnn.bias"]) + \
-        ["fc2.weight", "fc2.bias"]
-    for p in prefixes:
-        for n in names:
-            if p + n not in sd:
-                raise KeyError("state_dict has no %r (n_agents = %d)" % (p + n, n_agents))
-    flat = np.concatenate([sd[p + n].reshape(-1) for p in prefixes for n in names]).astype(np.float32)
-    hidden, input_dim = sd[prefixes[0] + "fc1.weight"].shape
+    use_rnn = ("agents.0." if ns else "") + "rnn.weight_ih" in sd
+    keys = state_dict_keys(n_agents, ns, use_rnn)
+    for k in keys:
+        if k not in sd:
+            raise KeyError("state_dict has no %r (n_agents = %d)" % (k, n_agents))
+    flat = np.concatenate([sd[k].reshape(-1) for k in keys]).astype(np.float32)
+    hidden, input_dim = sd[keys[0]].shape
     return flat, dict(non_shared=ns, use_rnn=use_rnn, hidden_dim=int(hidden), input_dim=int(input_dim),
-                      n_actions=int(sd[prefixes[0] + "fc2.weight"].shape[0]))
+                      n_actions=int(sd[keys[0].replace("fc1.weight", "fc2.weight")].shape[0]))
+
+
+def state_dict_shapes(n_agents, non_shared, use_rnn, hidden_dim, input_dim, n_actions):
+    """{key: shape} of the state_dict a policy of these facts was created from, in the order of the flat weights."""
+    H, D, A = hidden_dim, input_dim, n_actions
+    one = {"fc1.weight": (H, D), "fc1.bias": (H,), "rnn.weight_ih": (3 * H, H), "rnn.weight_hh": (3 * H, H),
+           "rnn.bias_ih": (3 * H,), "rnn.bias_hh": (3 * H,), "rnn.weight": (H, H), "rnn.bias": (H,),
+           "fc2.weight": (A, H), "fc2.bias": (A,)}
+    return {k: one[k.split(".", 2)[-1] if non_shared else k] for k in state_dict_keys(n_agents, non_shared, use_rnn)}
+
+
+def check_state_dict(state_dict, shapes):
+    """Raise ValueError, naming the first mismatching key, unless `state_dict` holds exactly the keys of `shapes`
+    (state_dict_shapes) with those shapes and a floating-point dtype.  Touches no device."""
+    for k, shape in shapes.items():
+        if k not in state_dict:
+            raise ValueError("state_dict has no %r, which this policy needs" % k)
+        v = state_dict[k]
+        if tuple(v.shape) != shape:
+            raise ValueError("state_dict[%r] has shape %s, this policy needs %s" % (k, tuple(v.shape), shape))
+        floating = v.is_floating_point() if isinstance(v, torch.Tensor) else np.issubdtype(np.asarray(v).dtype, np.floating)
+        if not floating:
+            raise ValueError("state_dict[%r] is %s, not a floating-point type" % (k, v.dtype))
+    for k in state_dict:
+        if k not in shapes:
+            raise ValueError("state_dict has %r, which this policy does not have" % k)
+
+
+def flatten_into(state_dict, keys, out):
+    """Copy the tensors (or numpy arrays) named by `keys`, flattened and converted to float32, back to back into the
+    float32 vector `out` on its device, as flatten_state_dict orders them.  Tensors already on out's device are
+    concatenated there without a synchronisation; the others are copied there first."""
+    ts = [torch.as_tensor(state_dict[k]).detach().reshape(-1) for k in keys]
+    ts = [t if t.device == out.device else t.to(out.device) for t in ts]
+    torch.cat(ts, out=out)
+    return out
 
 
 class Policy(object):
@@ -70,6 +115,9 @@ class Policy(object):
         self.handle = C.c_void_p()
         _lib.check_policy(self.lib.mrb_policy_create(C.byref(d), index, flat.ctypes.data_as(C.c_void_p), flat.size,
                                                      C.byref(self.handle)))
+        self._shapes = state_dict_shapes(n_agents, self.non_shared, self.use_rnn, self.hidden_dim, f["input_dim"],
+                                         self.n_actions)
+        self._staging = torch.empty((flat.size,), dtype=torch.float32, device=self.device)
 
     @classmethod
     def from_files(cls, weights_path, model_config_path, n_agents, obs_dim, device=None, accurate=False):
@@ -87,6 +135,23 @@ class Policy(object):
                 self.handle = None
         except Exception:
             pass
+
+    def load_state_dict(self, state_dict):
+        """Replace the weights in place: EPyMARL's mac.load_state(learner_mac) for the policy that collects.
+
+        `state_dict` is an RNNAgent / RNNNSAgent state_dict of the shape this policy was created with (hidden size, input
+        width, actions, GRU or Linear, shared or per-agent, n_agents; ValueError naming the first mismatching key
+        otherwise, before any device work).  Its tensors may be on any device, or numpy arrays, of any float dtype.
+        They are flattened into a float32 buffer the policy owns, on the current stream of its device, and
+        mrb_policy_load rebuilds the weight images from it in one launch.  Stream-ordered: with the tensors on the
+        policy's device nothing synchronises, and the call can be captured in a CUDA graph (replays read the tensors'
+        values at replay time).  A captured `Rollout` of this policy sees the new weights at its next replay."""
+        check_state_dict(state_dict, self._shapes)
+        with torch.cuda.device(self.device):
+            flatten_into(state_dict, self._shapes, self._staging)
+            _lib.check_policy(self.lib.mrb_policy_load(
+                self.handle, _ptr(self._staging), self._staging.numel(),
+                C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)), self.handle)
 
     def init_hidden(self, num_envs):
         """rnn_agent.py:17-19 init_hidden: zeros, one row per agent."""
@@ -245,7 +310,7 @@ class Rollout(object):
     def __init__(self, vec_env, policy, use_graph=True, steps_per_graph=8, explore=None, record=None):
         assert vec_env.N == policy.n_agents and vec_env.D == policy.obs_dim and vec_env.device == policy.device
         assert vec_env.n_actions == policy.n_actions, "policy and scenario disagree on the number of actions"
-        self.env, self.policy = vec_env, policy
+        self.env, self._policy = vec_env, policy
         self.hidden = policy.init_hidden(vec_env.B)
         self.actions = torch.zeros((vec_env.B, vec_env.N), dtype=torch.int32, device=vec_env.device)
         self.explore, self.q = explore, None
@@ -259,6 +324,17 @@ class Rollout(object):
         self.record = record
         self.use_graph, self.steps_per_graph = use_graph, int(steps_per_graph)
         self._graph = None
+
+    @property
+    def policy(self):
+        """The policy the rollout acts with.  A captured graph holds its weight images, so the policy cannot be
+        replaced; `rollout.policy.load_state_dict(sd)` changes its weights in place, graph included."""
+        return self._policy
+
+    @policy.setter
+    def policy(self, _):
+        raise AttributeError("Rollout.policy cannot be replaced (a captured graph keeps acting with the old policy's "
+                             "weights); load new weights with rollout.policy.load_state_dict(state_dict)")
 
     def reset(self):
         self.env.reset()
