@@ -17,7 +17,7 @@
 extern "C" {
 #endif
 
-#define MRB_ABI_VERSION 5
+#define MRB_ABI_VERSION 6
 #define MRB_MAX_ROBOTS 32
 #define MRB_MAX_PREY 32
 
@@ -300,6 +300,48 @@ int mrb_record_begin(mrb_env *env, const mrb_episode_batch *batch, void *cuda_st
 /* Records the step that mrb_step just took with `actions` (device i32 [B][N], 4-byte aligned): reads the bound obs,
  * reward and done buffers.  One launch, stream-ordered, never synchronises; checks as mrb_record_begin. */
 int mrb_record_step(mrb_env *env, const mrb_episode_batch *batch, const int32_t *actions, void *cuda_stream);
+
+/* ---- evaluation (per-episode results, utilities/misc.py:134-221 run_env; EPyMARL's runner in test mode).
+ * mrb_eval_step runs after every mrb_step and logs each env's first K finished episodes into a caller-owned table,
+ * one launch per step.  It reads only the bound reward, done, message, remaining and (when bound) dist buffers.
+ * B envs (the env handle's), N agents, all tensors contiguous, row-major, device memory:
+ *   per episode [B][K]: return_ f64 | length i32 | message u8 | timeout u8 | remaining i32 | dist f32
+ *   per env [B]: acc_return f64 | acc_length i32 | acc_dist f64 | count i32.
+ * Every step, for every env: team = the float32 sum of the N agent rewards in agent index order, starting from 0
+ * (the thread-per-env step kernels' episode return term; the team kernels of 7 or more robots sum with a warp
+ * butterfly); acc_return += (double)team; acc_length += 1; acc_dist += the float64 sum, in agent index order starting
+ * from 0, of the N floats of dist (0 when no dist buffer is bound).  Then, if done[b]:
+ * when k = count[b] < K, row k gets return_ = acc_return, length = acc_length, message = the step's message (bit 0
+ * collision, bit 1 boundary), timeout = (message == 0 && length > max_episode_steps, the MRB_STAT_TIMEOUTS test),
+ * remaining = the step's remaining, dist = (float)acc_dist, and count[b] = k + 1; whether or not a row was written, the
+ * three accumulators go back to 0.  An env with count == K logs nothing more.  Row k of env b is valid iff
+ * k < count[b]; the table is never zeroed.  Each env's accumulators and count are read and written by that env's own
+ * thread of one launch.  The lengths count steps since mrb_eval_begin, so call mrb_eval_begin together with mrb_reset
+ * of every env (or at an episode boundary of every env).
+ * Accesses are scalar and of the elements' own widths: every pointer must be aligned to its element size (8 bytes for
+ * return_, acc_return and acc_dist, 4 for length, remaining, dist, acc_length and count), MRB_E_ARG otherwise. */
+typedef struct mrb_eval_table {
+    int32_t struct_size;        /* sizeof(mrb_eval_table): ABI check */
+    int32_t episodes;           /* K: 1 .. 2^20 */
+    double *return_;
+    int32_t *length;
+    uint8_t *message;
+    uint8_t *timeout;
+    int32_t *remaining;
+    float *dist;
+    double *acc_return;
+    int32_t *acc_length;
+    double *acc_dist;
+    int32_t *count;
+} mrb_eval_table;
+/* Sets the accumulators and count of every env to 0 (the table rows are left as they are).  One launch,
+ * stream-ordered, never synchronises, capturable.  Errors through mrb_last_error(env) (mrb_last_error(NULL) when env is
+ * NULL); every argument is checked before the device is touched: NULL pointers, struct_size, episodes and alignment ->
+ * MRB_E_ARG, an env without buffers (mrb_bind) -> MRB_E_STATE. */
+int mrb_eval_begin(mrb_env *env, const mrb_eval_table *table, void *cuda_stream);
+/* Logs the step that mrb_step just took (see above).  One launch, stream-ordered, never synchronises, capturable;
+ * checks as mrb_eval_begin. */
+int mrb_eval_step(mrb_env *env, const mrb_eval_table *table, void *cuda_stream);
 
 /* FP64 roofline denominator, measured: runs a kernel of independent DFMA chains (8 per thread, one 1,024-thread
  * CTA per SM) for about `milliseconds` on `device`, timed with CUDA events, and returns the rate of the best launch

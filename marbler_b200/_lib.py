@@ -5,14 +5,15 @@ import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MARBLER_B200_LIB") or os.path.join(HERE, "libmarbler_b200.so")
-ABI_VERSION = 5
+ABI_VERSION = 6
 NUM_STATS = 16
 STAT_NAMES = ("episodes", "return_sum", "length_sum", "collisions", "boundary_exits", "scenario_metric",
               "env_steps", "qp_solves", "qp_iterations", "timeouts", "qp_stalls", "substeps", "qp_iterations_warp")
 SYMBOLS = ("mrb_version", "mrb_create", "mrb_destroy", "mrb_last_error", "mrb_state_rows", "mrb_obs_dim",
            "mrb_num_actions", "mrb_bind", "mrb_reset", "mrb_step", "mrb_step_host", "mrb_barrier_qp",
            "mrb_get_state", "mrb_set_state", "mrb_fp64_peak", "mrb_launch_count", "mrb_policy_create", "mrb_policy_destroy", "mrb_policy_last_error", "mrb_policy_act",
-           "mrb_policy_load", "mrb_select_actions", "mrb_record_begin", "mrb_record_step")
+           "mrb_policy_load", "mrb_select_actions", "mrb_record_begin", "mrb_record_step", "mrb_eval_begin",
+           "mrb_eval_step")
 
 
 class Spawn(C.Structure):
@@ -82,6 +83,12 @@ class EpisodeBatchDesc(C.Structure):
                                    "filled", "cursor")]
 
 
+class EvalTableDesc(C.Structure):
+    _fields_ = [("struct_size", C.c_int32), ("episodes", C.c_int32)] + \
+        [(n, C.c_void_p) for n in ("return_", "length", "message", "timeout", "remaining", "dist", "acc_return",
+                                   "acc_length", "acc_dist", "count")]
+
+
 _lib = None
 
 
@@ -120,6 +127,8 @@ def load():
         "mrb_select_actions": ([C.c_int, i64, i32, i32, C.POINTER(SelectDesc), vp, vp, vp, vp], C.c_int),
         "mrb_record_begin": ([vp, C.POINTER(EpisodeBatchDesc), vp], C.c_int),
         "mrb_record_step": ([vp, C.POINTER(EpisodeBatchDesc), vp, vp], C.c_int),
+        "mrb_eval_begin": ([vp, C.POINTER(EvalTableDesc), vp], C.c_int),
+        "mrb_eval_step": ([vp, C.POINTER(EvalTableDesc), vp], C.c_int),
     }
     for name, (args, res) in sig.items():
         f = getattr(L, name)

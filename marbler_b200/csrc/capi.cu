@@ -412,3 +412,41 @@ extern "C" int mrb_record_step(mrb_env *env, const mrb_episode_batch *batch, con
     if (!actions || ((uintptr_t)actions & 3)) return fail(env, MRB_E_ARG, "mrb_record_step: actions must be a 4-byte aligned device pointer");
     return record(env, batch, false, actions, stream);
 }
+
+// Everything mrb_eval_begin / mrb_eval_step check before they touch the device.
+static int check_eval_table(mrb_env *env, const mrb_eval_table *t, const char *fn)
+{
+    const std::string f(fn);
+    if (!env) return fail(nullptr, MRB_E_ARG, f + ": env is NULL");
+    if (!t) return fail(env, MRB_E_ARG, f + ": table is NULL");
+    if (t->struct_size != (int32_t)sizeof(mrb_eval_table))
+        return fail(env, MRB_E_ARG, f + ": mrb_eval_table.struct_size does not match this library (ABI mismatch)");
+    if (!t->return_ || !t->length || !t->message || !t->timeout || !t->remaining || !t->dist || !t->acc_return ||
+        !t->acc_length || !t->acc_dist || !t->count)
+        return fail(env, MRB_E_ARG, f + ": every pointer of mrb_eval_table is required");
+    if (t->episodes < 1 || t->episodes > (1 << 20)) return fail(env, MRB_E_ARG, f + ": episodes must be in [1, 2^20]");
+    // the kernel's accesses are scalar, each at its element's width
+    if ((((uintptr_t)t->return_ | (uintptr_t)t->acc_return | (uintptr_t)t->acc_dist) & 7) ||
+        (((uintptr_t)t->length | (uintptr_t)t->remaining | (uintptr_t)t->dist | (uintptr_t)t->acc_length |
+          (uintptr_t)t->count) & 3))
+        return fail(env, MRB_E_ARG, f + ": return_, acc_return and acc_dist must be 8-byte aligned, length, remaining, "
+                                        "dist, acc_length and count 4-byte aligned");
+    if (!env->bound) return fail(env, MRB_E_STATE, f + ": call mrb_bind first");
+    return MRB_OK;
+}
+
+static int eval(mrb_env *env, const mrb_eval_table *t, bool begin, void *stream)
+{
+    const int rc = check_eval_table(env, t, begin ? "mrb_eval_begin" : "mrb_eval_step");
+    if (rc != MRB_OK) return rc;
+    cudaError_t st = cudaSetDevice(env->device);
+    if (st != cudaSuccess) return cuda_fail(env, st, "cudaSetDevice");
+    if ((st = launch_eval(env->p, *t, begin, (cudaStream_t)stream)) != cudaSuccess)
+        return cuda_fail(env, st, "eval kernel launch");
+    g_launches++;
+    return MRB_OK;
+}
+
+extern "C" int mrb_eval_begin(mrb_env *env, const mrb_eval_table *table, void *stream) { return eval(env, table, true, stream); }
+
+extern "C" int mrb_eval_step(mrb_env *env, const mrb_eval_table *table, void *stream) { return eval(env, table, false, stream); }

@@ -294,6 +294,118 @@ class EpisodeBatch(object):
                        self.env.handle)
 
 
+EVAL_FIELDS = ("return", "length", "message", "timeout", "remaining", "dist")
+QUANTILES = (5, 25, 50, 75, 95)
+
+
+def _gather_rows(rows, device):
+    """Concatenate every rank's rows (float64 [n_rank, F]) in rank order (torch.distributed, when a process group of
+    more than one rank exists; the ranks may hold different numbers of rows)."""
+    import torch.distributed as dist
+    if not (dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1):
+        return rows
+    dev = device if dist.get_backend() == "nccl" else torch.device("cpu")
+    world = dist.get_world_size()
+    n = torch.tensor([rows.shape[0]], dtype=torch.int64, device=dev)
+    sizes = [torch.zeros_like(n) for _ in range(world)]
+    dist.all_gather(sizes, n)
+    sizes = [int(s.item()) for s in sizes]
+    top = max(sizes)
+    padded = torch.zeros((top, rows.shape[1]), dtype=torch.float64, device=dev)
+    padded[:rows.shape[0]] = rows.to(dev)
+    parts = [torch.empty_like(padded) for _ in range(world)]
+    dist.all_gather(parts, padded)
+    return torch.cat([p[:s] for p, s in zip(parts, sizes)])
+
+
+def summarize_episodes(data, n_agents=1, per_agent=False):
+    """Per-episode statistics of an evaluation table (`EvalLog.data`: [B,K] fields and count [B]; row k of env b is
+    an episode iff k < count[b]).  Host-side: synchronises with the table's device.  With a torch.distributed process
+    group the rows of every rank are gathered first (all_gather, rank order), so a sharded evaluation summarises the
+    same episodes as one device holding all envs.
+
+    `per_agent`: returns divided by n_agents, the reading run_env gives shared-reward scenarios (its eval-only
+    `shared_reward` config key, SURVEY.md Appendix B; the reference's misc.py is not vendored here, so this restates
+    it).  return_std is the population standard deviation (np.std, what EPyMARL logs as test_return_std); return_sem
+    uses the sample standard deviation (ddof = 1; NaN for one episode); the quantiles interpolate linearly
+    (np.quantile's default)."""
+    count = data["count"].to(torch.int64)
+    K = data["return"].shape[1]
+    valid = torch.arange(K, device=count.device)[None, :] < count[:, None]
+    rows = torch.stack([data[f][valid].to(torch.float64) for f in EVAL_FIELDS], dim=1)
+    rows = _gather_rows(rows, count.device).cpu().numpy()
+    n = rows.shape[0]
+    if n == 0:
+        raise ValueError("the evaluation table holds no finished episode")
+    ret = rows[:, 0] / (n_agents if per_agent else 1)
+    msg = rows[:, 2].astype(np.int64)
+    s = {"episodes": n, "return_mean": float(ret.mean()), "return_std": float(ret.std()),
+         "return_sem": float(ret.std(ddof=1) / np.sqrt(n)) if n > 1 else float("nan"),
+         "return_quantiles": {q: float(v) for q, v in zip(QUANTILES, np.quantile(ret, [q / 100 for q in QUANTILES]))},
+         "length_mean": float(rows[:, 1].mean()),
+         "collision_rate": float(((msg & 1) != 0).mean()), "boundary_rate": float(((msg & 2) != 0).mean()),
+         "timeout_rate": float(rows[:, 3].mean()), "remaining_mean": float(rows[:, 4].mean()),
+         "dist_mean": float(rows[:, 5].mean())}
+    s.update(test_return_mean=s["return_mean"], test_return_std=s["return_std"], test_ep_length_mean=s["length_mean"])
+    return s
+
+
+class EvalLog(object):
+    """Per-episode evaluation results of `vec_env`, filled on the device (mrb_eval_begin / mrb_eval_step,
+    csrc/eval.cu; the exact contract is in include/marbler_b200.h): what run_env (utilities/misc.py:134-221) prints
+    and logs for each of its episodes, for the first `episodes_per_env` (K) episodes of every env.
+
+    After every env step each env adds the team reward (float32 sum over agents in index order, as the thread-per-env
+    step kernels form the env's own episode return), one step and the distance its agents travelled to running accumulators; when the env finishes
+    an episode and has logged fewer than K, the next row of its table gets the episode's return, length, terminal
+    message (bit 0 collision, bit 1 boundary), timeout flag, `remaining` (prey left for PredatorCapturePrey, load left
+    for MaterialTransport, 0 elsewhere) and distance (0 without track_dist).  Lengths count from `begin()`, which is
+    meant to go with a reset of every env (as `Rollout.evaluate()` does).
+
+    `data`: return [B,K] f64, length [B,K] i32, message / timeout [B,K] u8, remaining [B,K] i32, dist [B,K] f32 and
+    count [B] i32; row k of env b is valid iff k < count[b]."""
+
+    def __init__(self, vec_env, episodes_per_env):
+        self.env, self.lib = vec_env, _lib.load()
+        B, dev = vec_env.B, vec_env.device
+        self.episodes = K = int(episodes_per_env)
+        self.return_ = torch.zeros((B, K), dtype=torch.float64, device=dev)
+        self.length = torch.zeros((B, K), dtype=torch.int32, device=dev)
+        self.message = torch.zeros((B, K), dtype=torch.uint8, device=dev)
+        self.timeout = torch.zeros((B, K), dtype=torch.uint8, device=dev)
+        self.remaining = torch.zeros((B, K), dtype=torch.int32, device=dev)
+        self.dist = torch.zeros((B, K), dtype=torch.float32, device=dev)
+        self.acc_return = torch.zeros((B,), dtype=torch.float64, device=dev)
+        self.acc_length = torch.zeros((B,), dtype=torch.int32, device=dev)
+        self.acc_dist = torch.zeros((B,), dtype=torch.float64, device=dev)
+        self.count = torch.zeros((B,), dtype=torch.int32, device=dev)
+        self.desc = _lib.EvalTableDesc(C.sizeof(_lib.EvalTableDesc), K, *[t.data_ptr() for t in (
+            self.return_, self.length, self.message, self.timeout, self.remaining, self.dist, self.acc_return,
+            self.acc_length, self.acc_dist, self.count)])
+
+    @property
+    def data(self):
+        return {"return": self.return_, "length": self.length, "message": self.message, "timeout": self.timeout,
+                "remaining": self.remaining, "dist": self.dist, "count": self.count}
+
+    def _call(self, fn):
+        with torch.cuda.device(self.env.device):
+            _lib.check(fn(self.env.handle, C.byref(self.desc),
+                          C.c_void_p(torch.cuda.current_stream(self.env.device).cuda_stream)), self.env.handle)
+
+    def begin(self):
+        """Accumulators and counts to 0 (the rows stay as they are).  One launch, stream-ordered."""
+        self._call(self.lib.mrb_eval_begin)
+
+    def record(self):
+        """Log the step the env just took.  One launch, stream-ordered, capturable."""
+        self._call(self.lib.mrb_eval_step)
+
+    def summary(self, per_agent=False):
+        """summarize_episodes over this table (synchronises; gathers the ranks of a process group)."""
+        return summarize_episodes(self.data, self.env.N, per_agent)
+
+
 class Rollout(object):
     """run_env's loop for a whole batch, on the device: act -> step -> act -> ...  (misc.py:155-187).
 
@@ -305,9 +417,12 @@ class Rollout(object):
     None it takes the env's own, so that the ranks of a sharded run draw distinct streams.
 
     `record`: an `EpisodeBatch` of the same env that records every step after it is taken (one more launch per step,
-    captured in the graph too); `collect()` then fills it with one runner batch."""
+    captured in the graph too); `collect()` then fills it with one runner batch.
 
-    def __init__(self, vec_env, policy, use_graph=True, steps_per_graph=8, explore=None, record=None):
+    `evaluate`: an `EvalLog` of the same env that logs every step after it is taken (one more launch per step, after
+    the record launch, captured in the graph too); `evaluate()` then fills it with K episodes per env."""
+
+    def __init__(self, vec_env, policy, use_graph=True, steps_per_graph=8, explore=None, record=None, evaluate=None):
         assert vec_env.N == policy.n_agents and vec_env.D == policy.obs_dim and vec_env.device == policy.device
         assert vec_env.n_actions == policy.n_actions, "policy and scenario disagree on the number of actions"
         self.env, self._policy = vec_env, policy
@@ -322,6 +437,8 @@ class Rollout(object):
                 self.q = torch.zeros((vec_env.B, vec_env.N, policy.n_actions), dtype=torch.float32, device=vec_env.device)
         assert record is None or record.env is vec_env, "the EpisodeBatch must belong to the rollout's env"
         self.record = record
+        assert evaluate is None or evaluate.env is vec_env, "the EvalLog must belong to the rollout's env"
+        self.eval_log = evaluate
         self.use_graph, self.steps_per_graph = use_graph, int(steps_per_graph)
         self._graph = None
 
@@ -346,6 +463,8 @@ class Rollout(object):
         self.env.step(self.actions)
         if self.record is not None:
             self.record.record(self.actions)
+        if self.eval_log is not None:
+            self.eval_log.record()
 
     def collect(self):
         """One EPyMARL runner batch into `record`: mrb_record_begin, `reset()`, then exactly episode_limit env steps,
@@ -358,9 +477,22 @@ class Rollout(object):
         self.run(self.record.episode_limit)
         return self.record.data
 
+    def evaluate(self):
+        """K episodes of every env into `evaluate` (its `episodes`): mrb_eval_begin, `reset()`, then
+        K * (max_episode_steps + 1) env steps.  An episode ends after at most max_episode_steps + 1 steps, so at the end
+        every env has logged exactly K episodes, whatever its episode lengths and with no host synchronisation on the
+        way; the result does not depend on the graph, the batch size or the sharding.  Envs that have logged K episodes
+        keep stepping until the end (unlogged).  Returns `evaluate.data`; `evaluate.summary()` reduces it."""
+        if self.eval_log is None:
+            raise ValueError("Rollout.evaluate needs evaluate=EvalLog(...)")
+        self.eval_log.begin()
+        self.reset()
+        self.run(self.eval_log.episodes * (self.env.c.max_episode_steps + 1))
+        return self.eval_log.data
+
     def run(self, steps):
-        """Advance every env by `steps` env steps (2 kernels per step, 4 with `explore`, one more with `record`; no
-        host synchronisation)."""
+        """Advance every env by `steps` env steps (2 kernels per step, 4 with `explore`, one more each with `record`
+        and `evaluate`; no host synchronisation)."""
         k = self.steps_per_graph
         if self.use_graph:
             if self._graph is None and steps > k:
