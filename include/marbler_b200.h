@@ -17,7 +17,7 @@
 extern "C" {
 #endif
 
-#define MRB_ABI_VERSION 6
+#define MRB_ABI_VERSION 7
 #define MRB_MAX_ROBOTS 32
 #define MRB_MAX_PREY 32
 
@@ -128,6 +128,19 @@ int mrb_reset(mrb_env *env, const uint8_t *mask, uint64_t seed, void *cuda_strea
  * (roboEnv.py:38-96) -> Controller.set_velocities (controller.py:20-25) -> rps / cvxopt.
  * actions: device i32 [B][N]. */
 int mrb_step(mrb_env *env, const int32_t *actions, void *cuda_stream);
+/* ---- masked step (EPyMARL's ParallelRunner steps only envs_not_terminated and leaves the others alone until the batch
+ * ends).  active: device u8 [B] on the env's device; an env b with active[b] != 0 is stepped exactly as mrb_step steps
+ * it - its state and every output row (obs, reward, done, message, remaining, dist, obs_f64, reward_f64) bit for bit,
+ * auto-reset included.  Of an env with active[b] == 0 nothing is read or written: no state row, no output row, no
+ * auto-reset, no contribution to stats.  The integer stats counters (env steps, QP solves and iterations, sub-steps,
+ * episodes, collisions, boundary exits, timeouts) count exactly the active env-steps; the float sums (return, length)
+ * are those of the same episodes up to the order of the atomic additions.  active == NULL is mrb_step.
+ * Two launches whatever the mask holds: a compaction of `active` into a list of active env ids (library-internal
+ * scratch allocated by mrb_create), then the step kernel over that list with its grid sized for B, so a captured CUDA
+ * graph keeps its shape.  Stream-ordered, never synchronises, capturable; the caller keeps `active` unchanged until
+ * the launches have run.  Every argument is checked before the device is touched: as mrb_step, plus an `active` that is
+ * not device memory of the env's device (cudaPointerGetAttributes) -> MRB_E_ARG.  mrb_step_host has no mask. */
+int mrb_step_masked(mrb_env *env, const int32_t *actions, const uint8_t *active, void *cuda_stream);
 /* same step with HOST buffers (pinned for full speed; pageable works): H2D actions, step, D2H
  * obs/reward/done/message, then synchronises.  Batches of >= 16,384 envs are cut into up to 8 chunks,
  * each on its own library-internal stream (ordered after the caller's stream), so that the PCIe copies

@@ -5,12 +5,12 @@ import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MARBLER_B200_LIB") or os.path.join(HERE, "libmarbler_b200.so")
-ABI_VERSION = 6
+ABI_VERSION = 7
 NUM_STATS = 16
 STAT_NAMES = ("episodes", "return_sum", "length_sum", "collisions", "boundary_exits", "scenario_metric",
               "env_steps", "qp_solves", "qp_iterations", "timeouts", "qp_stalls", "substeps", "qp_iterations_warp")
 SYMBOLS = ("mrb_version", "mrb_create", "mrb_destroy", "mrb_last_error", "mrb_state_rows", "mrb_obs_dim",
-           "mrb_num_actions", "mrb_bind", "mrb_reset", "mrb_step", "mrb_step_host", "mrb_barrier_qp",
+           "mrb_num_actions", "mrb_bind", "mrb_reset", "mrb_step", "mrb_step_masked", "mrb_step_host", "mrb_barrier_qp",
            "mrb_get_state", "mrb_set_state", "mrb_fp64_peak", "mrb_launch_count", "mrb_policy_create", "mrb_policy_destroy", "mrb_policy_last_error", "mrb_policy_act",
            "mrb_policy_load", "mrb_select_actions", "mrb_record_begin", "mrb_record_step", "mrb_eval_begin",
            "mrb_eval_step")
@@ -113,6 +113,7 @@ def load():
         "mrb_bind": ([vp, C.POINTER(Buffers)], C.c_int),
         "mrb_reset": ([vp, vp, u64, vp], C.c_int),
         "mrb_step": ([vp, vp, vp], C.c_int),
+        "mrb_step_masked": ([vp, vp, vp, vp], C.c_int),
         "mrb_step_host": ([vp, vp, vp, vp, vp, vp, vp], C.c_int),
         "mrb_barrier_qp": ([C.c_int, i32, i32, i64, vp, vp, vp, vp, vp], C.c_int),
         "mrb_get_state": ([vp, i64, i64, C.POINTER(StateFields), vp], C.c_int),

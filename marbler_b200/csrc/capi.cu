@@ -71,7 +71,7 @@ extern "C" int mrb_create(const mrb_config *cfg, int device, int64_t num_envs, i
     if (c.num_robots < 2 || c.num_robots > MRB_MAX_ROBOTS) return fail(nullptr, MRB_E_ARG, "mrb_create: num_robots must be in [2, 32]");
     if (!(c.collision_diameter > 0.0) || !(c.collision_offset >= 0.0) || !std::isfinite(c.collision_diameter + c.collision_offset))
         return fail(nullptr, MRB_E_ARG, "mrb_create: collision_diameter must be > 0 and collision_offset >= 0 (rps: 0.135 and 0 or 0.025)");
-    if (num_envs < 1) return fail(nullptr, MRB_E_ARG, "mrb_create: num_envs must be >= 1");
+    if (num_envs < 1 || num_envs > INT32_MAX) return fail(nullptr, MRB_E_ARG, "mrb_create: num_envs must be in [1, 2^31)");
     if (c.update_frequency < 1 || c.ctrl_period < 1) return fail(nullptr, MRB_E_ARG, "mrb_create: update_frequency / ctrl_period must be >= 1");
     if (c.scenario == MRB_PCP && (c.num_prey < 1 || c.num_prey > MRB_MAX_PREY || c.num_predators < 0 || c.num_predators > c.num_robots))
         return fail(nullptr, MRB_E_ARG, "mrb_create: PredatorCapturePrey needs 1..32 prey and predators <= robots");
@@ -104,6 +104,19 @@ extern "C" int mrb_create(const mrb_config *cfg, int device, int64_t num_envs, i
 
     mrb_env *e = new (std::nothrow) mrb_env();
     if (!e) return fail(nullptr, MRB_E_ARG, "mrb_create: out of host memory");
+    // the scratch of mrb_step_masked, here so that no step allocates (a captured graph could not); the caller's
+    // current device is left as it was
+    int prev = device;
+    cudaGetDevice(&prev);
+    e->step_list = nullptr;
+    if ((st = cudaSetDevice(device)) == cudaSuccess && (st = cudaMalloc(&e->step_list, sizeof(int32_t) * (num_envs + 3))) == cudaSuccess)
+        st = cudaMemset(e->step_list + num_envs, 0, 3 * sizeof(int32_t));
+    cudaSetDevice(prev);
+    if (st != cudaSuccess) {
+        if (e->step_list) cudaFree(e->step_list);
+        delete e;
+        return cuda_fail(nullptr, st, "mrb_create: step list");
+    }
     std::memset(&e->p, 0, sizeof(Params));
     e->p.cfg = c;
     e->p.B = num_envs;
@@ -132,6 +145,7 @@ extern "C" int mrb_destroy(mrb_env *env)
     if (!env) return MRB_E_ARG;
     cudaSetDevice(env->device);
     if (env->actions_dev) cudaFree(env->actions_dev);
+    if (env->step_list) cudaFree(env->step_list);
     if (env->pipe_ready) {
         for (int k = 0; k < kPipeStreams; k++) { cudaStreamDestroy(env->pipe[k]); cudaEventDestroy(env->ev_out[k]); }
         cudaEventDestroy(env->ev_in);
@@ -182,13 +196,15 @@ extern "C" int mrb_reset(mrb_env *env, const uint8_t *mask, uint64_t seed, void 
     return MRB_OK;
 }
 
-// launch the step kernel for envs [lo, hi) on stream s
-static int step_range(mrb_env *env, const int32_t *actions, int64_t lo, int64_t hi, cudaStream_t s, const HostOut *hout = nullptr)
+// launch the step kernel for envs [lo, hi) on stream s, or (list: env->step_list after the compaction) for the listed envs
+static int step_range(mrb_env *env, const int32_t *actions, int64_t lo, int64_t hi, cudaStream_t s, const HostOut *hout = nullptr,
+                      const int32_t *list = nullptr)
 {
     Params p = env->p;
     p.env_lo = lo;
     p.env_hi = hi;
     if (hout) p.hout = *hout;
+    if (list) { p.envs = list; p.count = list + p.B; }
     cudaError_t st;
     switch (p.cfg.scenario) {
     case MRB_PCP: st = launch_step<MRB_PCP>(p, actions, s); break;
@@ -211,6 +227,32 @@ extern "C" int mrb_step(mrb_env *env, const int32_t *actions, void *stream)
     cudaError_t st = cudaSetDevice(env->device);
     if (st != cudaSuccess) return cuda_fail(env, st, "cudaSetDevice");
     return step_range(env, actions, 0, env->p.B, (cudaStream_t)stream);
+}
+
+// Two launches whatever `active` holds: the compaction into env->step_list, then the step kernel over the list, its grid
+// sized for all B envs so that a captured graph does not depend on the mask.
+extern "C" int mrb_step_masked(mrb_env *env, const int32_t *actions, const uint8_t *active, void *stream)
+{
+    if (!active) return mrb_step(env, actions, stream);
+    if (!env) return MRB_E_ARG;
+    if (!actions) return fail(env, MRB_E_ARG, "mrb_step_masked: actions is NULL");
+    if (!env->bound) return fail(env, MRB_E_STATE, "mrb_step_masked: call mrb_bind first");
+    if ((uintptr_t)actions & 15) return fail(env, MRB_E_ARG, "mrb_step_masked: actions must be 16-byte aligned");
+    cudaPointerAttributes at;
+    cudaError_t st = cudaPointerGetAttributes(&at, active);
+    if (st != cudaSuccess) {
+        cudaGetLastError();
+        return fail(env, MRB_E_ARG, std::string("mrb_step_masked: active: ") + cudaGetErrorString(st));
+    }
+    if (at.type != cudaMemoryTypeDevice || at.device != env->device)
+        return fail(env, MRB_E_ARG, "mrb_step_masked: active must be device memory of the env's device " + std::to_string(env->device));
+    if ((st = cudaSetDevice(env->device)) != cudaSuccess) return cuda_fail(env, st, "cudaSetDevice");
+    const cudaStream_t s = (cudaStream_t)stream;
+    const int64_t B = env->p.B;
+    if ((st = launch_compact(active, B, env->step_list, env->step_list + B, s)) != cudaSuccess)
+        return cuda_fail(env, st, "compaction kernel launch");
+    g_launches++;
+    return step_range(env, actions, 0, B, s, nullptr, env->step_list);
 }
 
 // Host-buffer step.  Large batches are cut into up to 8 chunks, each on its own internal stream: all the

@@ -43,6 +43,9 @@ struct Params {
     int32_t rows_f64, rows_i32;
     // exact squared thresholds: sqrt(d2) <= r  <=>  d2 <= thr2(r)   (computed on the host)
     double collision_thr2, sense_thr2, capture_thr2, zone1_thr2;
+    // mrb_step_masked: the compacted ids of the active envs and their number (written by the compaction kernel on the
+    // stream); item i of the step launch steps env envs[i] and items >= *count none.  NULL on every other path.
+    const int32_t *envs, *count;
 };
 
 // ---- state rows (env index fastest).  f64 rows:

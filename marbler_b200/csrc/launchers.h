@@ -30,6 +30,9 @@ cudaError_t launch_select_actions(int64_t num_envs, int32_t n_agents, int32_t n_
 // record.cu: mrb_record_begin (begin, actions unused) and mrb_record_step, one launch each
 cudaError_t launch_record(const Params &p, int n_actions, const mrb_episode_batch &batch, bool begin,
                           const int32_t *actions, cudaStream_t s);
+// compact.cu: mrb_step_masked's list of active envs.  work i32 [3]: count (out), then two words that must be 0 on entry
+// and are 0 again on exit
+cudaError_t launch_compact(const uint8_t *active, int64_t B, int32_t *envs, int32_t *work, cudaStream_t s);
 // eval.cu: mrb_eval_begin (begin) and mrb_eval_step, one launch each
 cudaError_t launch_eval(const Params &p, const mrb_eval_table &table, bool begin, cudaStream_t s);
 }  // namespace mrb

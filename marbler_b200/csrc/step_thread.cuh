@@ -231,13 +231,20 @@ __global__ void reset_kernel(const __grid_constant__ Params p, const uint8_t *ma
 }
 
 // ---- the step
-template <int SCN, int N>
+// LIST = {true} (mrb_step_masked): item i steps env p.envs[i]; the live items are a prefix of the launch, so the warps
+// are full but for the last one.  LIST empty: item i steps env env_lo + i.  A compile-time switch, because read at run
+// time the env index could no longer be recomputed from blockIdx where registers are short (the N = 4 kernel would
+// spill); an empty pack, so that the range kernels keep their names and their code.
+template <int SCN, int N, bool... LIST>
 __global__ void __launch_bounds__(ThreadShape<N>::kThreads, ThreadShape<N>::kMinBlocks)
 step_thread_kernel(const __grid_constant__ Params p, const int32_t *__restrict__ actions)
 {
-    const int64_t env = p.env_lo + (int64_t)blockIdx.x * ThreadShape<N>::kThreads + threadIdx.x;
-    const unsigned warp_envs = __ballot_sync(0xffffffffu, env < p.env_hi);      // lanes of this warp that own an env
-    if (env >= p.env_hi) return;
+    constexpr bool kList = (false || ... || LIST);
+    const int64_t item = (int64_t)blockIdx.x * ThreadShape<N>::kThreads + threadIdx.x;
+    const int64_t env = kList ? (item < *p.count ? (int64_t)p.envs[item] : -1) : p.env_lo + item;
+    const bool live = kList ? env >= 0 : env < p.env_hi;
+    const unsigned warp_envs = __ballot_sync(0xffffffffu, live);      // lanes of this warp that own an env
+    if (!live) return;
     const mrb_config &c = p.cfg;
     const int64_t S = p.B;
     double *sf = p.buf.state_f64 + env;
@@ -716,7 +723,8 @@ step_thread_kernel(const __grid_constant__ Params p, const int32_t *__restrict__
     p.buf.remaining[env] = remaining;
     if (p.hout.obs || p.hout.reward || p.hout.done || p.hout.message) {
         // host mirrors.  The observations of a warp's envs are one contiguous block of obs[B][N][D]: re-read it
-        // warp-wide so that every store instruction sends 512 contiguous bytes over PCIe
+        // warp-wide so that every store instruction sends 512 contiguous bytes over PCIe.  Only mrb_step_host sets
+        // hout, and it launches ranges (never a LIST, whose warps' envs are not contiguous)
         const unsigned act = warp_envs;      // not __activemask(): lanes that diverged above must reconverge here
         __syncwarp(act);
         if (p.hout.obs) {
@@ -778,11 +786,12 @@ inline cudaError_t launch_thread(const Params &p, const int32_t *actions, cudaSt
     constexpr int tpb = ThreadShape<N>::kThreads;
     const unsigned grid = (unsigned)((p.env_hi - p.env_lo + tpb - 1) / tpb);
     constexpr size_t smem = QpStore<N>::kBytes;
+    const auto kernel = p.envs ? step_thread_kernel<SCN, N, true> : step_thread_kernel<SCN, N>;
     if (smem > 48 * 1024) {
-        const cudaError_t attr = cudaFuncSetAttribute(step_thread_kernel<SCN, N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        const cudaError_t attr = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (attr != cudaSuccess) return attr;
     }
-    step_thread_kernel<SCN, N><<<grid, tpb, smem, s>>>(p, actions);
+    kernel<<<grid, tpb, smem, s>>>(p, actions);
     return cudaGetLastError();
 }
 

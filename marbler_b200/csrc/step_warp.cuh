@@ -661,14 +661,17 @@ struct QpWarp {
 // WPB: warps (= envs) per CTA.  The 20-robot instantiation runs its 12 resident warps as ONE CTA: they then execute the
 // 14 k-instruction body roughly in step and share the instruction fetches (21.8 vs 22.5 ms per 32,768 envs); the generic
 // path keeps 4-warp CTAs because the workspace of a 32-robot team would not fit twelve times.
-template <int SCN, int PPL, int NC = 0, int WPB = kWarpsPerBlock, bool EXACT = true>
+// LIST = {true} (mrb_step_masked): warp i steps env p.envs[i] if i < *p.count, as in step_thread_kernel.
+template <int SCN, int PPL, int NC = 0, int WPB = kWarpsPerBlock, bool EXACT = true, bool... LIST>
 __global__ void __launch_bounds__(WPB * 32, NC == 0 ? kWarpMinBlocks : 1)
 step_warp_kernel(const __grid_constant__ Params p, const int32_t *__restrict__ actions)
 {
+    constexpr bool kList = (false || ... || LIST);
     extern __shared__ __align__(16) double smem[];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-    const int64_t env = p.env_lo + (int64_t)blockIdx.x * WPB + wib;
-    if (env >= p.env_hi) return;
+    const int64_t item = (int64_t)blockIdx.x * WPB + wib;
+    const int64_t env = kList ? (item < *p.count ? (int64_t)p.envs[item] : -1) : p.env_lo + item;
+    if (kList ? env < 0 : env >= p.env_hi) return;
     const mrb_config &c = p.cfg;
     const int N = (NC && EXACT) ? NC : c.num_robots;
     const int64_t S = p.B;
@@ -1007,10 +1010,11 @@ inline cudaError_t launch_step_warp_ppl(const Params &p, const int32_t *actions,
 {
     constexpr int WPB = NC != 0 ? team_warps(NC) : kWarpsPerBlock;
     const size_t smem = warp_workspace_doubles(NC ? NC : p.cfg.num_robots) * sizeof(double) * WPB;
-    cudaError_t st = cudaFuncSetAttribute(step_warp_kernel<SCN, PPL, NC, WPB, EXACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const auto kernel = p.envs ? step_warp_kernel<SCN, PPL, NC, WPB, EXACT, true> : step_warp_kernel<SCN, PPL, NC, WPB, EXACT>;
+    cudaError_t st = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (st != cudaSuccess) return st;
     const unsigned grid = (unsigned)((p.env_hi - p.env_lo + WPB - 1) / WPB);
-    step_warp_kernel<SCN, PPL, NC, WPB, EXACT><<<grid, WPB * 32, smem, s>>>(p, actions);
+    kernel<<<grid, WPB * 32, smem, s>>>(p, actions);
     return cudaSuccess;
 }
 

@@ -420,9 +420,22 @@ class Rollout(object):
     captured in the graph too); `collect()` then fills it with one runner batch.
 
     `evaluate`: an `EvalLog` of the same env that logs every step after it is taken (one more launch per step, after
-    the record launch, captured in the graph too); `evaluate()` then fills it with K episodes per env."""
+    the record launch, captured in the graph too); `evaluate()` then fills it with K episodes per env.
 
-    def __init__(self, vec_env, policy, use_graph=True, steps_per_graph=8, explore=None, record=None, evaluate=None):
+    `skip_finished`: step only the envs that `record` or `evaluate` still needs (mrb_step_masked), as EPyMARL's
+    ParallelRunner steps only envs_not_terminated: with `record`, the envs whose recorded episode has not terminated
+    (cursor >= 0); with `evaluate`, the envs that have logged fewer than K episodes; with both, either.  The mask is
+    computed on the device before every step, inside the captured graph.  A `collect()` or `evaluate()` that starts
+    from the same env state fills `record.data` / `evaluate.data` bit for bit as without it, with the same exploration
+    draws; what differs is `env.stats` (it counts only the steps taken) and the state the skipped envs are left in: they
+    stop where their last needed step left them instead of running on into episodes nobody reads, so their episode
+    counters, which key the reset streams, do not advance, and the next call's `reset()` starts them in other episodes.
+    Off by default; needs `record` or `evaluate`."""
+
+    def __init__(self, vec_env, policy, use_graph=True, steps_per_graph=8, explore=None, record=None, evaluate=None,
+                 skip_finished=False):
+        if skip_finished and record is None and evaluate is None:
+            raise ValueError("Rollout(skip_finished=True) needs record= or evaluate=: they decide which envs are finished")
         assert vec_env.N == policy.n_agents and vec_env.D == policy.obs_dim and vec_env.device == policy.device
         assert vec_env.n_actions == policy.n_actions, "policy and scenario disagree on the number of actions"
         self.env, self._policy = vec_env, policy
@@ -439,6 +452,12 @@ class Rollout(object):
         self.record = record
         assert evaluate is None or evaluate.env is vec_env, "the EvalLog must belong to the rollout's env"
         self.eval_log = evaluate
+        self.skip_finished = bool(skip_finished)
+        # u8 [B] mask of the envs the next step takes, written through a bool view; with both record and evaluate the
+        # second buffer holds evaluate's part
+        self.active = torch.ones((vec_env.B,), dtype=torch.uint8, device=vec_env.device) if skip_finished else None
+        self._eval_needs = torch.ones((vec_env.B,), dtype=torch.bool, device=vec_env.device) \
+            if skip_finished and record is not None and evaluate is not None else None
         self.use_graph, self.steps_per_graph = use_graph, int(steps_per_graph)
         self._graph = None
 
@@ -458,9 +477,21 @@ class Rollout(object):
         self.env.done.fill_(1)          # every env starts an episode: first act() sees fresh = 1 everywhere
         self.hidden.zero_()
 
+    def _update_active(self):
+        """self.active = the envs `record` or `evaluate` still needs, from their cursors and counts (on the stream)."""
+        a = self.active.view(torch.bool)
+        if self.record is not None:
+            torch.ge(self.record.cursor, 0, out=a)
+            if self.eval_log is not None:
+                torch.lt(self.eval_log.count, self.eval_log.episodes, out=self._eval_needs)
+                a.logical_or_(self._eval_needs)
+        else:
+            torch.lt(self.eval_log.count, self.eval_log.episodes, out=a)
+        return self.active
+
     def _one(self):
         self.policy.act(self.env.obs, self.hidden, actions=self.actions, q=self.q, fresh=self.env.done, explore=self.explore)
-        self.env.step(self.actions)
+        self.env.step(self.actions, active=self._update_active() if self.skip_finished else None)
         if self.record is not None:
             self.record.record(self.actions)
         if self.eval_log is not None:
@@ -482,7 +513,8 @@ class Rollout(object):
         K * (max_episode_steps + 1) env steps.  An episode ends after at most max_episode_steps + 1 steps, so at the end
         every env has logged exactly K episodes, whatever its episode lengths and with no host synchronisation on the
         way; the result does not depend on the graph, the batch size or the sharding.  Envs that have logged K episodes
-        keep stepping until the end (unlogged).  Returns `evaluate.data`; `evaluate.summary()` reduces it."""
+        keep stepping until the end (unlogged), unless `skip_finished`.  Returns `evaluate.data`; `evaluate.summary()`
+        reduces it."""
         if self.eval_log is None:
             raise ValueError("Rollout.evaluate needs evaluate=EvalLog(...)")
         self.eval_log.begin()
@@ -492,7 +524,7 @@ class Rollout(object):
 
     def run(self, steps):
         """Advance every env by `steps` env steps (2 kernels per step, 4 with `explore`, one more each with `record`
-        and `evaluate`; no host synchronisation)."""
+        and `evaluate`, one more and the mask's torch kernels with `skip_finished`; no host synchronisation)."""
         k = self.steps_per_graph
         if self.use_graph:
             if self._graph is None and steps > k:

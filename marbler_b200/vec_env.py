@@ -84,14 +84,33 @@ class VecEnv(object):
             _lib.check(self.lib.mrb_reset(self.handle, _ptr(m), self.seed, self._stream()), self.handle)
         return self.obs
 
-    def step(self, actions):
+    def active_mask(self, active):
+        """The u8 [B] view mrb_step_masked reads of `active`, a bool or uint8 tensor [B] on the env's device (no copy
+        when it is contiguous).  TypeError / ValueError otherwise, before any device work."""
+        if not isinstance(active, torch.Tensor) or active.dtype not in (torch.bool, torch.uint8):
+            raise TypeError("active must be a bool or uint8 tensor, not %r" % (getattr(active, "dtype", type(active)),))
+        if tuple(active.shape) != (self.B,):
+            raise ValueError("active must have shape (%d,), not %s" % (self.B, tuple(active.shape)))
+        if active.device != self.device:
+            raise ValueError("active must be on the env's device %s, not %s" % (self.device, active.device))
+        return active.contiguous().view(torch.uint8)
+
+    def step(self, actions, active=None):
         """actions: int32 CUDA tensor [B, N].  Stream-ordered, no synchronisation.  Returns the
-        output buffers (obs [B,N,D] f32, reward [B,N] f32, done [B] u8, message [B] u8)."""
+        output buffers (obs [B,N,D] f32, reward [B,N] f32, done [B] u8, message [B] u8).
+
+        `active`: a bool or uint8 tensor [B] on the env's device (mrb_step_masked).  Only the envs it flags are stepped;
+        the state, output rows and stats of the others are left exactly as they are.  Stream-ordered and capturable
+        too: the mask is read on the device when the step runs."""
+        m = None if active is None else self.active_mask(active)
         if actions.device != self.device or actions.dtype != torch.int32 or not actions.is_contiguous() \
                 or tuple(actions.shape) != (self.B, self.N):
             actions = actions.to(device=self.device, dtype=torch.int32).reshape(self.B, self.N).contiguous()
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.mrb_step(self.handle, _ptr(actions), self._stream()), self.handle)
+            if m is None:
+                _lib.check(self.lib.mrb_step(self.handle, _ptr(actions), self._stream()), self.handle)
+            else:
+                _lib.check(self.lib.mrb_step_masked(self.handle, _ptr(actions), _ptr(m), self._stream()), self.handle)
         return self.obs, self.reward, self.done, self.message
 
     def host_buffers(self):
